@@ -6,7 +6,7 @@ batch of synthetic frames.  Per-GPU batch is fixed (weak scaling); frames shard 
 across ranks with no data-path collective.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload detect|dense|dense4k|rig] [--batch B]
+                    [--workload detect|dense|dense4k|rig] [--batch B] [--dump-outputs DIR]
 
 Workloads (BASELINE.json configs):
   detect   configs[2]: rendered 6x6 T36H11 boards, 1280x1024 L8, 1024 frames per GPU per step (default)
@@ -20,6 +20,10 @@ ag_detect_batch with HOST buffers (H2D + D2H inside the timed region).  The defa
 carries short runs of dense4k, the f32 blur operator alone (benches/bench_blur.rs) and rig under "extras".
 `--impl reference` times the reference's CPU algorithm (the oracle port, all host threads) on
 the first frames of the same device-rendered batch.
+
+`--dump-outputs DIR` (detect and dense4k workloads) writes, after the timed steps, the detections
+of rank 0's last timed step as DIR/<name>.npy (see dump_detections).  The frames are rendered
+from a fixed seed, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import glob
@@ -172,6 +176,32 @@ def render_frames(det, torch, n, w, h, cols, rows, seed, stream):
     return frames
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_detections(out_dir, tag_dtype, d_tags, d_cnt, d_status, cap, limit=DUMP_LIMIT_BYTES):
+    """Write the results of one detect_batch_device call (its three output tensors) as .npy files:
+    frame_index (frames,), tag_counts (frames,), frame_status (frames,) and tag_ids (frames, cap)
+    in float64, tag_corners (frames, cap, 4, 2) in float32.  Slots past a frame's count hold id -1
+    and corners 0.  Above `limit` bytes in all, a fixed seeded sample of the frames is written;
+    frame_index says which frames of the batch the rows are."""
+    n = d_cnt.shape[0]
+    per_frame = 3 * 8 + cap * 8 + cap * 8 * 4
+    keep = min(n, limit // per_frame)
+    idx = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    rec = d_tags.cpu().numpy().view(tag_dtype).reshape(n, cap)[idx]
+    cnt = d_cnt.cpu().numpy()[idx]
+    valid = np.arange(cap)[None, :] < cnt[:, None]
+    arrays = {"frame_index": idx.astype(np.float64),
+              "tag_counts": cnt.astype(np.float64),
+              "frame_status": d_status.cpu().numpy().view(np.uint32)[idx].astype(np.float64),
+              "tag_ids": np.where(valid, rec["id"].astype(np.float64), -1.0),
+              "tag_corners": np.where(valid[..., None], rec["xy"], np.float32(0)).reshape(keep, cap, 4, 2)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def gather_list(value, world, device):
     """This rank's python float from every rank, as a list (rank order)."""
     if world == 1:
@@ -303,9 +333,10 @@ def run_rig(pkg, det, torch, n_frames, warmup, stream, seed):
 # -------------------------------------------------------------------------------------------
 # configs[3]: 4K RGB dense board
 # -------------------------------------------------------------------------------------------
-def run_dense4k(pkg, det, torch, n, steps, warmup, stream, seed):
+def run_dense4k(pkg, det, torch, n, steps, warmup, stream, seed, dump_dir=None):
     """Streaming calls like the detect workload: device_async, two sets of result buffers, one wait
-    after the last step (the board searches of step k overlap the front end of step k + 1)."""
+    after the last step (the board searches of step k overlap the front end of step k + 1).
+    With `dump_dir`, the last timed step's detections are written there (dump_detections)."""
     w, h, cap = 3840, 2160, 512
     gray = render_frames(det, torch, n, w, h, 24, 13, seed, stream.cuda_stream)
     rgb = gray[..., None].expand(n, h, w, 3).contiguous()
@@ -338,6 +369,9 @@ def run_dense4k(pkg, det, torch, n, steps, warmup, stream, seed):
         det.set_option("device_async", 0)
     ms = e0.elapsed_time(e1)
     assert steps < 2 or bool((cnt[0] == cnt[1]).all()), "steps disagree on the same frames"
+    if dump_dir:
+        last = (k[0] - 1) & 1
+        dump_detections(dump_dir, pkg.TAG_DTYPE, tags[last], cnt[last], st[last], cap)
     return {"image": [w, h], "format": "RGB8", "board": "24x13 T36H11", "frames_per_step": n, "steps": steps,
             "frames_per_s": float(n * steps / (ms * 1e-3)), "ms_per_step": ms / steps,
             "calls": "streaming (device_async, two result sets, one wait after the last step)",
@@ -392,7 +426,14 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the short dense4k / rig runs of the default line")
     ap.add_argument("--opt", action="append", default=[], metavar="KEY=VALUE",
                     help="extra ag_set_option settings (experiments), e.g. --opt k1_chunk_rows=124")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write rank 0's detections of the last timed step as "
+                         "DIR/<name>.npy (detect and dense4k workloads)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload not in ("detect", "dense4k")):
+        ap.error("--dump-outputs: only the detect and dense4k workloads return detections to the caller")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -497,7 +538,8 @@ def main():
             sampler.start()
             time.sleep(0.5)
             sampler.t_begin = time.perf_counter()
-        r = run_dense4k(pkg, det, torch, B, args.steps, max(args.warmup, 3), stream, SEED + 7919 * rank)
+        r = run_dense4k(pkg, det, torch, B, args.steps, max(args.warmup, 3), stream, SEED + 7919 * rank,
+                        dump_dir=args.dump_outputs if rank == 0 else None)
         if sampler:
             sampler.t_end = time.perf_counter()
         clocks = sampler.finish() if sampler else None
@@ -586,6 +628,9 @@ def main():
     if cnt_host is not None:
         assert np.array_equal(cnt_host, d_cnt[1].cpu().numpy()), "steps disagree on the same frames"
         assert not d_status[0].any().item(), "a frame of the benchmark batch was flagged"
+    if args.dump_outputs and rank == 0:
+        last = (step_no[0] - 1) & 1  # result buffers of the last timed step
+        dump_detections(args.dump_outputs, pkg.TAG_DTYPE, d_tags[last], d_cnt[last], d_status[last], cap)
     if streaming:
         det.set_option("device_async", 0)
 
