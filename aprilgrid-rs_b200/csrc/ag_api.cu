@@ -234,6 +234,9 @@ int make_geom(ag_detector* det, int w, int h, size_t row_stride, size_t frame_st
   if (frame_stride == 0) frame_stride = row_stride * h;
   if (frame_stride < row_stride * (size_t)(h - 1) + min_row)
     return fail(det, AG_ERR_INVALID, "frame_stride smaller than a frame");
+  // every other frame of an odd stride would start at an odd address: K1 and K6 read 16-bit pixels
+  // with 2-byte loads (the host path keeps the caller's frame stride in its device staging too)
+  if (format == AG_L16 && (frame_stride & 1)) return fail(det, AG_ERR_INVALID, "L16 frame_stride must be even");
   g->w = w;
   g->h = h;
   g->wpr = (w + 31) / 32;
@@ -1018,6 +1021,8 @@ int ag_detect_batch_device(ag_detector* det, const void* d_frames, size_t frame_
   FrameGeom g;
   int rc = make_geom(det, width, height, row_stride, frame_stride, format, &g);
   if (rc) return rc;
+  if (format == AG_L16 && ((uintptr_t)d_frames & 1))
+    return fail(det, AG_ERR_INVALID, "L16 frames must start at an even device address");
   // chunks of host-buffer calls still in flight share the dense buffers and the board slots:
   // hand their results out first (streaming host calls and device calls do not overlap)
   if ((rc = collect_host(det, det->host_seq))) return rc;
@@ -1103,6 +1108,8 @@ int ag_dense_batch_device(ag_detector* det, const void* d_frames, size_t frame_s
   FrameGeom g;
   int rc = make_geom(det, width, height, row_stride, frame_stride, format, &g);
   if (rc) return rc;
+  if (format == AG_L16 && ((uintptr_t)d_frames & 1))
+    return fail(det, AG_ERR_INVALID, "L16 frames must start at an even device address");
   Slot& S = det->slot[0];
   set_caps(det, g);
   const int chunk = chunk_limit(det, g, std::min<long>(det->chunk_frames, std::max(n_frames, 1)));
@@ -1904,9 +1911,10 @@ int ag_multi_detect_batch(ag_multi* m, const void* frames, size_t frame_stride, 
   auto work = [&](int g) {
     const long long lo = bound[g], hi = bound[g + 1];
     if (hi <= lo) return;
-    rcs[g] = ag_detect_batch(m->dets[g], (const uint8_t*)frames + (size_t)lo * fs, fs, (int)(hi - lo), width, height,
-                             rs, format, out + (size_t)lo * cap_per_frame, cap_per_frame, n_per_frame + lo,
-                             frame_status ? frame_status + lo : nullptr);
+    // synchronous whatever a device's "host_async" says (ag_multi has no wait entry point), as ag_detect
+    rcs[g] = detect_batch_host(m->dets[g], (const uint8_t*)frames + (size_t)lo * fs, fs, (int)(hi - lo), width,
+                               height, rs, format, out + (size_t)lo * cap_per_frame, cap_per_frame, n_per_frame + lo,
+                               frame_status ? frame_status + lo : nullptr, /*async_call=*/false);
   };
   std::vector<std::thread> th;
   for (int g = 1; g < G; ++g) th.emplace_back(work, g);

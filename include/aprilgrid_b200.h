@@ -141,7 +141,8 @@ AG_API int ag_detect_planes(ag_detector* det, const float* luma32f, size_t f32_r
                             ag_tag* out, int cap, int* n);
 
 /* detect_batch: n_frames host images of one shape at frames + i*frame_stride.
- * out[i*cap_per_frame ..], n_per_frame[i]; frame_status may be NULL.                     */
+ * out[i*cap_per_frame ..], n_per_frame[i]; frame_status may be NULL.
+ * Strides in bytes (0 = packed); for AG_L16 both must be even (else AG_ERR_INVALID).      */
 AG_API int ag_detect_batch(ag_detector* det, const void* frames, size_t frame_stride,
                            int n_frames, int width, int height, size_t row_stride, int format,
                            ag_tag* out, int cap_per_frame, int* n_per_frame,
@@ -150,7 +151,8 @@ AG_API int ag_detect_batch(ag_detector* det, const void* frames, size_t frame_st
 /* Same, frames already resident in device memory; outputs are DEVICE pointers
  * (d_out: n_frames*cap_per_frame ag_tag, d_n_per_frame: n_frames int32,
  *  d_frame_status: n_frames uint32 or NULL).  Work is enqueued on `stream`
- * (a cudaStream_t, NULL = the detector's own stream) and is asynchronous.               */
+ * (a cudaStream_t, NULL = the detector's own stream) and is asynchronous.
+ * AG_L16 frames must start at an even device address (else AG_ERR_INVALID; nothing runs). */
 AG_API int ag_detect_batch_device(ag_detector* det, const void* d_frames, size_t frame_stride,
                                   int n_frames, int width, int height, size_t row_stride,
                                   int format, ag_tag* d_out, int cap_per_frame,
@@ -196,7 +198,7 @@ AG_API int ag_gaussian_blur_f32_device(ag_detector* det, const float* d_in, int 
 
 /* Dense front end only (gray -> blur -> Hessian -> min -> threshold mask), device-resident
  * frames, results stay in the detector's workspace.  This is the unit bench.py times for
- * the "blur / threshold kernels alone" configuration.                                   */
+ * the "blur / threshold kernels alone" configuration.  AG_L16: even address and strides. */
 AG_API int ag_dense_batch_device(ag_detector* det, const void* d_frames, size_t frame_stride,
                                  int n_frames, int width, int height, size_t row_stride,
                                  int format, void* stream);
@@ -252,7 +254,8 @@ AG_API void ag_host_free(void* p);
  * unless the devices' host-to-device rates (measured at creation, all devices copying at once)
  * differ by more than 5 %: then they are proportional to those rates.  devices = NULL or
  * n_devices = 0: every visible device.  Same arguments, results and error behaviour as
- * ag_detect_batch (always synchronous); byte-identical to one device processing the batch.   */
+ * ag_detect_batch, but always synchronous, whatever the devices' "host_async" option says;
+ * byte-identical to one device processing the batch.                                          */
 typedef struct ag_multi ag_multi;
 AG_API int ag_multi_create(int family, const ag_params* params, const int* devices, int n_devices,
                            ag_multi** out);

@@ -114,6 +114,30 @@ def render_board_numpy(w=640, h=480, cols=6, rows=6, seed=0, tag_px=None, family
     return img
 
 
+def composite_boards(tiles, tile_w, tile_h, grid_cols, canvas=None):
+    """Boards of different layouts, one per tile of a grid (row-major), in one L8 frame.
+    tiles: (cols, rows, seed, tag_px) each.  Every board numbers its tags from 0, so the id ranges
+    overlap and a board found in a later round of the board search overwrites earlier ids.
+    canvas: (height, width) of a larger paper-white frame the grid is placed in at (0, 0)."""
+    grid_rows = (len(tiles) + grid_cols - 1) // grid_cols
+    h, w = canvas or (grid_rows * tile_h, grid_cols * tile_w)
+    img = np.full((h, w), 200, np.uint8)
+    for k, (cols, rows, seed, tag_px) in enumerate(tiles):
+        r, c = divmod(k, grid_cols)
+        img[r * tile_h:(r + 1) * tile_h, c * tile_w:(c + 1) * tile_w] = render_board_numpy(
+            tile_w, tile_h, cols=cols, rows=rows, seed=seed, tag_px=tag_px)
+    return img
+
+
+# 1280 x 960: 456 refined saddles (512-saddle tier of the board kernel); the oracle finds the 3 x 3
+# board with one round, the 6 x 6 board (overwriting all 9 ids) with two, and with three rounds 12 ids
+# carry the 4 x 3 board's corners
+FOUR_BOARDS = ([(6, 6, 3, 44.0), (4, 3, 5, 60.0), (5, 4, 8, 52.0), (3, 3, 11, 70.0)], 640, 480, 2)
+# four small boards in the same 1280 x 960 frame, <= 320 refined saddles (the small tier); every
+# round up to the fourth changes the result
+SMALL_BOARDS = ([(3, 3, 11, 60.0), (4, 3, 5, 52.0), (3, 2, 7, 60.0), (2, 2, 2, 70.0)], 320, 320, 2)
+
+
 def fixture_like_frames(n, w, h, seed=0, **kw):
     return np.stack([render_board_numpy(w, h, seed=seed + i, **kw) for i in range(n)])
 
