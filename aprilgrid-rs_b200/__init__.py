@@ -127,6 +127,7 @@ def lib():
         L.ag_test_unorm_tables.argtypes = [vp, vp, vp, vp, vp]
         L.ag_test_board_times.argtypes = [vp, ci, vp, ci]
         L.ag_test_board_layout.argtypes = [ci, ci, ci, ci, ci, ci, vp]
+        L.ag_test_board_decode_room.argtypes = [ci, ci, ci, vp]
         L.ag_test_render_pose.argtypes = [vp, vp, ci, ci, ci, ci, vp, ci, C.c_uint64]
         L.ag_test_boards_from_saddles.argtypes = [vp, vp, ci, vp, ci, ci, sz, ci, vp, ci, vp, vp, ci, vp]
         _lib = L

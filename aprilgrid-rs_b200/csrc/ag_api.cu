@@ -1670,6 +1670,17 @@ AG_API int ag_test_board_layout(int max_saddles, int lattice, int warps, int sme
   return AG_OK;
 }
 
+// Test hook (not in the public header; needs no GPU): the decode scratch of the board kernel for a
+// configuration.  The bit patterns of the listed quads (8 bytes each) go to warp 0's seed-best values;
+// out = {bytes of that region up to the next array of the warp, most quads a board can list}.
+AG_API int ag_test_board_decode_room(int max_saddles, int lattice, int warps, long long out[2]) {
+  if (!out || max_saddles < 1 || lattice < 1) return AG_ERR_INVALID;
+  const BoardWsLayout L = make_board_layout(max_saddles, lattice, warps, max_saddles);
+  out[0] = (long long)(L.woff_stack - L.woff_sb_vals);
+  out[1] = std::min(L.max_quads, lattice * lattice);
+  return AG_OK;
+}
+
 // Test hook (not in the public header): ONE frame of the renderer under a GIVEN pose -- hinv maps
 // image (x, y, 1) to page coordinates in tag sides (row-major 3x3, host pointer) -- with or without
 // the noise, so that tests can pin the renderer's geometry (id <-> lattice position, corner

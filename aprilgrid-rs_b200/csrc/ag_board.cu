@@ -62,7 +62,9 @@ BoardWsLayout make_board_layout(int max_saddles, int lattice, int warps, int sme
   L.woff_touched = wtake(sizeof(int16_t) * cells);
   L.woff_sb_quads = wtake(sizeof(int16_t) * 4 * Q);
   L.woff_sb_touched = wtake(sizeof(int16_t) * cells);
-  L.woff_sb_vals = wtake(sizeof(int16_t) * cells);
+  // warp 0's seed-best values double as the decode's bit patterns: 8 bytes for each quad the board
+  // lists, and a board lists at most min(Q, lattice^2) quads
+  L.woff_sb_vals = wtake(std::max(sizeof(int16_t) * cells, sizeof(unsigned long long) * std::min(Q, cells)));
   L.woff_stack = wtake(sizeof(int16_t) * 2 * (Q + 1));
   L.bytes_per_warp = align_up(w, 64);
   L.bytes_per_frame = align_up(L.off_warp0 + L.bytes_per_warp * kBoardWarps, 256);

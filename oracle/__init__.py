@@ -283,6 +283,21 @@ def detect(img, family="t36h11", min_angle=30.0, max_angle=60.0, max_boards=2, c
     return {int(t["id"]): t["xy"].reshape(4, 2).copy() for t in out[:n]}
 
 
+def detect_from_saddles(img, saddles, family="t36h11", max_boards=2, cap=1024):
+    """The board rounds of detect (board search + decoding, detector.rs:511-536) on a given refined
+    saddle list (N x 5 float32: x, y, k, theta, phi) over img -> {id: 4x2 float32 corners}."""
+    img = np.ascontiguousarray(img)
+    fmt, w, h, st = image_format(img)
+    s = np.ascontiguousarray(saddles, np.float32).reshape(-1, 5)
+    out = np.zeros(cap, TAG_DTYPE)
+    L = lib()
+    L.orc_detect_from_saddles.argtypes = [C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int,
+                                          C.c_size_t, C.c_int, C.c_void_p, C.c_int]
+    n = L.orc_detect_from_saddles(FAMILY[family], max_boards, _p(s), len(s), _p(img), w, h, st, fmt, _p(out), cap)
+    assert 0 <= n <= cap, n
+    return {int(t["id"]): t["xy"].reshape(4, 2).copy() for t in out[:n]}
+
+
 def detect_planes(luma32f, luma8, family="t36h11", min_angle=30.0, max_angle=60.0, max_boards=2, cap=1024):
     """detect on a frame given as its two gray planes (to_luma32f / to_luma8 of the DynamicImage)."""
     f = np.ascontiguousarray(luma32f, np.float32)

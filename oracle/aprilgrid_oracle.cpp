@@ -983,26 +983,15 @@ bool try_decode_quad(const Family& fam, const uint8_t* grey, uint32_t w, uint32_
   return true;
 }
 
-// a-14  detect -- src/detector.rs:505-540.  The result map is returned in ascending id order.
-//       Quads of one board are visited in Board::all_tag_indexes order (see Board); a repeated
-//       id overwrites, as HashMap::insert does.
-// grey_plane: null = to_luma8 of `pixels` (detector.rs:507); else the Luma<u8> plane itself, `pixels`
-// then being the Luma<f32> plane (fmt 3): the frame as its two derived gray images (detect_planes).
-int detect(const Family& fam, const Params& prm, const void* pixels, int w, int h, size_t stride,
-           int fmt, TagOut* out, int cap, const uint8_t* grey_plane = nullptr, size_t grey_stride = 0) {
-  std::vector<uint8_t> grey((size_t)w * h);
-  {
-    StageTimer tm(0);
-    if (grey_plane) to_luma_u8(grey_plane, w, h, grey_stride ? grey_stride : (size_t)w, 0, grey.data());
-    else to_luma_u8(pixels, w, h, stride, fmt, grey.data());
-  }
-  ++g_stage_frames;
-  FrontEnd fe;
-  refined_saddle_points(pixels, w, h, stride, fmt, prm, &fe, false);
-  std::vector<Saddle> refined = fe.refined;
+// a-14  board rounds of detect -- src/detector.rs:511-536: `max_num_of_boards` rounds of board
+//       search + decoding on the refined saddle list and the Luma<u8> plane `grey` (w x h, packed).
+//       The result map is returned in ascending id order.  Quads of one board are visited in
+//       Board::all_tag_indexes order (see Board); a repeated id overwrites, as HashMap::insert does.
+int detect_from_saddles(const Family& fam, int max_boards, std::vector<Saddle> refined, const uint8_t* grey,
+                        int w, int h, TagOut* out, int cap) {
   std::map<uint32_t, TagOut> detected;
   std::vector<Quad> quads;
-  for (int b = 0; b < prm.max_num_of_boards; ++b) {
+  for (int b = 0; b < max_boards; ++b) {
     {
       StageTimer tm(2);
       if (!try_find_best_board(refined, &quads)) continue;
@@ -1016,7 +1005,7 @@ int detect(const Family& fam, const Params& prm, const void* pixels, int w, int 
         qy[j] = refined[q[j]].y;
       }
       TagOut t;
-      if (try_decode_quad(fam, grey.data(), (uint32_t)w, (uint32_t)h, qx, qy, &t)) {
+      if (try_decode_quad(fam, grey, (uint32_t)w, (uint32_t)h, qx, qy, &t)) {
         detected[t.id] = t;
         for (int j = 0; j < 4; ++j) remove[q[j]] = 1;
       }
@@ -1032,6 +1021,23 @@ int detect(const Family& fam, const Params& prm, const void* pixels, int w, int 
     ++n;
   }
   return n;
+}
+
+// a-14  detect -- src/detector.rs:505-540: the gray planes, refined_saddle_points, then the rounds.
+// grey_plane: null = to_luma8 of `pixels` (detector.rs:507); else the Luma<u8> plane itself, `pixels`
+// then being the Luma<f32> plane (fmt 3): the frame as its two derived gray images (detect_planes).
+int detect(const Family& fam, const Params& prm, const void* pixels, int w, int h, size_t stride,
+           int fmt, TagOut* out, int cap, const uint8_t* grey_plane = nullptr, size_t grey_stride = 0) {
+  std::vector<uint8_t> grey((size_t)w * h);
+  {
+    StageTimer tm(0);
+    if (grey_plane) to_luma_u8(grey_plane, w, h, grey_stride ? grey_stride : (size_t)w, 0, grey.data());
+    else to_luma_u8(pixels, w, h, stride, fmt, grey.data());
+  }
+  ++g_stage_frames;
+  FrontEnd fe;
+  refined_saddle_points(pixels, w, h, stride, fmt, prm, &fe, false);
+  return detect_from_saddles(fam, prm.max_num_of_boards, fe.refined, grey.data(), w, h, out, cap);
 }
 
 }  // namespace
@@ -1291,6 +1297,19 @@ int orc_detect(int family, float min_angle, float max_angle, int max_boards, con
   prm.max_saddle_angle = max_angle;
   prm.max_num_of_boards = max_boards;
   return detect(f, prm, px, w, h, stride, fmt, (TagOut*)tags_out, cap);
+}
+
+// The board rounds of detect on a caller-supplied refined saddle list (n x {x, y, k, theta, phi})
+// over the frame `pixels` (L8 / L16 / RGB8, converted with to_luma8).  Returns the number of tags.
+int orc_detect_from_saddles(int family, int max_boards, const float* saddles, int n, const void* px, int w,
+                            int h, size_t stride, int fmt, void* tags_out, int cap) {
+  Family f;
+  if (!family_by_id(family, &f) || n < 0 || fmt < 0 || fmt > 2) return -1;
+  std::vector<Saddle> s(n);
+  if (n) memcpy(s.data(), saddles, (size_t)n * 20);
+  std::vector<uint8_t> grey((size_t)w * h);
+  to_luma_u8(px, w, h, stride, fmt, grey.data());
+  return detect_from_saddles(f, max_boards, s, grey.data(), w, h, (TagOut*)tags_out, cap);
 }
 
 // detect on a frame given as its two gray planes: luma32f = to_luma32f(img), luma8 = to_luma8(img).

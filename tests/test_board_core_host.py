@@ -23,7 +23,7 @@ def hb():
 
 def host_detect(hb, pkg, oracle, img, saddles=None, family=None, max_boards=2, max_saddles=2048,
                 use_grid=1, lattice=64):
-    family = family or pkg.TagFamily.T36H11
+    family = pkg.TagFamily.T36H11 if family is None else family  # T16H5 is 0
     fam = pkg.family_info(family)
     if saddles is None:
         saddles = oracle.front_end(img, want_labels=False)["refined"]
