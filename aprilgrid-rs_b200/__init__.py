@@ -23,6 +23,10 @@ if os.environ.get("AG_LIB"):  # profiling tools only: another build of the same 
 
 AG_OK, AG_ERR_INVALID, AG_ERR_NO_DEVICE, AG_ERR_CUDA, AG_ERR_CAPACITY, AG_ERR_UNSUPPORTED = range(6)
 FMT_L8, FMT_L16, FMT_RGB8 = 0, 1, 2
+FMT_LA8, FMT_RGBA8, FMT_LA16, FMT_RGB16, FMT_RGBA16 = 4, 5, 6, 7, 8  # 3 is reserved
+# (channels, dtype) -> pixel format of an H x W x channels image (DynamicImage LumaA / Rgb / Rgba)
+_CHANNEL_FORMATS = {(2, np.uint8): FMT_LA8, (3, np.uint8): FMT_RGB8, (4, np.uint8): FMT_RGBA8,
+                    (2, np.uint16): FMT_LA16, (3, np.uint16): FMT_RGB16, (4, np.uint16): FMT_RGBA16}
 
 TAG_DTYPE = np.dtype([("id", np.uint32), ("xy", np.float32, (8,))])
 SADDLE_DTYPE = np.dtype([("x", np.float32), ("y", np.float32), ("k", np.float32),
@@ -139,14 +143,15 @@ def _p(a):
 
 
 def image_format(img):
-    """(fmt, width, height, row_stride_bytes) for HxW u8 (Luma8), HxW u16 (Luma16), HxWx3 u8 (Rgb8)."""
+    """(fmt, width, height, row_stride_bytes) for HxW u8 (Luma8) / u16 (Luma16), and HxWxN u8 / u16
+    with N = 2 (LumaA8 / LumaA16), 3 (Rgb8 / Rgb16) or 4 (Rgba8 / Rgba16), channels interleaved."""
     if img.ndim == 2 and img.dtype == np.uint8:
         return FMT_L8, img.shape[1], img.shape[0], img.strides[0]
     if img.ndim == 2 and img.dtype == np.uint16:
         return FMT_L16, img.shape[1], img.shape[0], img.strides[0]
-    if img.ndim == 3 and img.shape[2] == 3 and img.dtype == np.uint8:
-        return FMT_RGB8, img.shape[1], img.shape[0], img.strides[0]
-    raise ValueError("unsupported image: shape %s dtype %s (want HxW u8/u16 or HxWx3 u8)"
+    if img.ndim == 3 and (img.shape[2], img.dtype.type) in _CHANNEL_FORMATS:
+        return _CHANNEL_FORMATS[(img.shape[2], img.dtype.type)], img.shape[1], img.shape[0], img.strides[0]
+    raise ValueError("unsupported image: shape %s dtype %s (want HxW or HxWxN, N in 2..4, u8/u16)"
                      % (img.shape, img.dtype))
 
 
@@ -218,7 +223,7 @@ class TagDetector:
         """TagDetector::detect(&DynamicImage) -> HashMap<u32, [(f32, f32); 4]> (detector.rs:505)."""
         img = np.asarray(img)
         fmt, w, h, st = image_format(img)
-        if img.strides[-1] != img.itemsize or (img.ndim == 3 and img.strides[1] != 3):
+        if img.strides[-1] != img.itemsize or (img.ndim == 3 and img.strides[1] != img.shape[2] * img.itemsize):
             img = np.ascontiguousarray(img)
             fmt, w, h, st = image_format(img)
         out = np.zeros(cap, TAG_DTYPE)
@@ -248,7 +253,7 @@ class TagDetector:
         return self.detect(np.ascontiguousarray(img))
 
     def detect_batch(self, frames, cap_per_frame=128, return_status=False):
-        """New batched entry point: frames is N x H x W (u8/u16) or N x H x W x 3 (u8)."""
+        """New batched entry point: frames is N x H x W or N x H x W x C (C in 2..4), u8 or u16."""
         frames = np.asarray(frames)
         if not frames.flags.c_contiguous:
             frames = np.ascontiguousarray(frames)

@@ -219,24 +219,23 @@ int fail(ag_detector* det, int code, const char* msg) {
   return code;
 }
 
-int bytes_per_px(int format) { return format == AG_L8 ? 1 : (format == AG_L16 ? 2 : 3); }
-
 int make_geom(ag_detector* det, int w, int h, size_t row_stride, size_t frame_stride, int format,
               FrameGeom* g) {
   if (w <= 0 || h <= 0) return fail(det, AG_ERR_INVALID, "width/height must be positive");
-  if (format != AG_L8 && format != AG_L16 && format != AG_RGB8)
-    return fail(det, AG_ERR_INVALID, "unknown pixel format");
+  if (format == kFmtF32 || bytes_per_px(format) == 0) return fail(det, AG_ERR_INVALID, "unknown pixel format");
   if ((long long)w * h > (1ll << 30)) return fail(det, AG_ERR_INVALID, "image too large");
   size_t min_row = (size_t)w * bytes_per_px(format);
   if (row_stride == 0) row_stride = min_row;
   if (row_stride < min_row) return fail(det, AG_ERR_INVALID, "row_stride smaller than a row");
-  if (format == AG_L16 && (row_stride & 1)) return fail(det, AG_ERR_INVALID, "L16 row_stride must be even");
+  if (is_16bit_format(format) && (row_stride & 1))
+    return fail(det, AG_ERR_INVALID, "row_stride of a 16-bit format must be even");
   if (frame_stride == 0) frame_stride = row_stride * h;
   if (frame_stride < row_stride * (size_t)(h - 1) + min_row)
     return fail(det, AG_ERR_INVALID, "frame_stride smaller than a frame");
   // every other frame of an odd stride would start at an odd address: K1 and K6 read 16-bit pixels
   // with 2-byte loads (the host path keeps the caller's frame stride in its device staging too)
-  if (format == AG_L16 && (frame_stride & 1)) return fail(det, AG_ERR_INVALID, "L16 frame_stride must be even");
+  if (is_16bit_format(format) && (frame_stride & 1))
+    return fail(det, AG_ERR_INVALID, "frame_stride of a 16-bit format must be even");
   g->w = w;
   g->h = h;
   g->wpr = (w + 31) / 32;
@@ -1021,8 +1020,8 @@ int ag_detect_batch_device(ag_detector* det, const void* d_frames, size_t frame_
   FrameGeom g;
   int rc = make_geom(det, width, height, row_stride, frame_stride, format, &g);
   if (rc) return rc;
-  if (format == AG_L16 && ((uintptr_t)d_frames & 1))
-    return fail(det, AG_ERR_INVALID, "L16 frames must start at an even device address");
+  if (is_16bit_format(format) && ((uintptr_t)d_frames & 1))
+    return fail(det, AG_ERR_INVALID, "frames of a 16-bit format must start at an even device address");
   // chunks of host-buffer calls still in flight share the dense buffers and the board slots:
   // hand their results out first (streaming host calls and device calls do not overlap)
   if ((rc = collect_host(det, det->host_seq))) return rc;
@@ -1108,8 +1107,8 @@ int ag_dense_batch_device(ag_detector* det, const void* d_frames, size_t frame_s
   FrameGeom g;
   int rc = make_geom(det, width, height, row_stride, frame_stride, format, &g);
   if (rc) return rc;
-  if (format == AG_L16 && ((uintptr_t)d_frames & 1))
-    return fail(det, AG_ERR_INVALID, "L16 frames must start at an even device address");
+  if (is_16bit_format(format) && ((uintptr_t)d_frames & 1))
+    return fail(det, AG_ERR_INVALID, "frames of a 16-bit format must start at an even device address");
   Slot& S = det->slot[0];
   set_caps(det, g);
   const int chunk = chunk_limit(det, g, std::min<long>(det->chunk_frames, std::max(n_frames, 1)));
@@ -1900,8 +1899,7 @@ int ag_multi_detect_batch(ag_multi* m, const void* frames, size_t frame_stride, 
     return AG_ERR_INVALID;
   }
   // the strides every shard's offsets are computed with (0 = tightly packed, as in ag_detect_batch)
-  const size_t bpp = format == AG_L8 ? 1 : (format == AG_L16 ? 2 : 3);
-  const size_t rs = row_stride ? row_stride : (size_t)(width > 0 ? width : 0) * bpp;
+  const size_t rs = row_stride ? row_stride : (size_t)(width > 0 ? width : 0) * bytes_per_px(format);
   const size_t fs = frame_stride ? frame_stride : rs * (size_t)(height > 0 ? height : 0);
   const int G = (int)m->dets.size();
   std::vector<int> rcs(G, AG_OK);

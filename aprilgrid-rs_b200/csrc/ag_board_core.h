@@ -1211,10 +1211,27 @@ AGB_NOINLINE int find_best_board(Frame& F) {
 }
 
 // ---- decoding (detector.rs:42-169, :448-476) ---------------------------------------------------
-AGB_FN int luma8_at(const Frame& F, uint32_t x, uint32_t y) {  // image 0.25 to_luma8
+// to_luma8 of pixel x of a row of LA8 (4), RGBA8 (5), LA16 (6), RGB16 (7) or RGBA16 (8): alpha is
+// dropped, colour is the integer sRGB luma in the source width, u16 luma is scaled to u8.  Out of
+// line, so that the frame formats of the benchmark keep the board kernel's code as it was.
+AGB_NOINLINE int luma8_wide(const uint8_t* row, uint32_t x, int format) {
+  const uint16_t* r16 = (const uint16_t*)row;
+  if (format == 4) return row[2 * (size_t)x];
+  if (format == 5) {
+    const uint8_t* p = row + 4 * (size_t)x;
+    return (int)((2126u * p[0] + 7152u * p[1] + 722u * p[2]) / 10000u);
+  }
+  if (format == 6) return (int)((((uint32_t)r16[2 * (size_t)x]) + 128u) / 257u);
+  const uint16_t* p = r16 + (format == 7 ? 3 : 4) * (size_t)x;
+  return (int)(((2126u * p[0] + 7152u * p[1] + 722u * p[2]) / 10000u + 128u) / 257u);
+}
+
+// image 0.25 to_luma8 of pixel (x, y) in the public pixel format F.format (include/aprilgrid_b200.h)
+AGB_FN int luma8_at(const Frame& F, uint32_t x, uint32_t y) {
   const uint8_t* row = F.img + (size_t)y * F.row_stride;
   if (F.format == 0) return row[x];
   if (F.format == 1) return (int)((((uint32_t)((const uint16_t*)row)[x]) + 128u) / 257u);
+  if (F.format != 2) return luma8_wide(row, x, F.format);
   const uint8_t* p = row + 3 * (size_t)x;
   return (int)((2126u * p[0] + 7152u * p[1] + 722u * p[2]) / 10000u);
 }

@@ -24,6 +24,16 @@ namespace ag {
 // to_luma32f itself); not a value of the public format enum.
 constexpr int kFmtF32 = 3;
 
+// Bytes of one pixel of format `fmt` (a public AG_* format or kFmtF32); 0 for any other value.
+AG_HD constexpr int bytes_per_px(int fmt) {
+  return fmt == AG_L8 ? 1 : fmt == AG_L16 ? 2 : fmt == AG_RGB8 ? 3 : fmt == kFmtF32 ? 4 : fmt == AG_LA8 ? 2
+       : fmt == AG_RGBA8 ? 4 : fmt == AG_LA16 ? 4 : fmt == AG_RGB16 ? 6 : fmt == AG_RGBA16 ? 8 : 0;
+}
+// The public formats whose pixels are 16-bit words: rows, frames and device frames must be 2-byte aligned.
+AG_HD constexpr bool is_16bit_format(int fmt) {
+  return fmt == AG_L16 || fmt == AG_LA16 || fmt == AG_RGB16 || fmt == AG_RGBA16;
+}
+
 constexpr int kBlurRadius = 3;  // ceil(2 * 1.5), src/image_util.rs:111
 constexpr int kBlurTaps = 7;
 
@@ -35,7 +45,7 @@ struct FrameGeom {
   int n_px;             // w * h
   size_t frame_stride;  // bytes between input frames
   size_t row_stride;    // bytes between input rows
-  int format;           // AG_L8 / AG_L16 / AG_RGB8
+  int format;           // a public AG_* pixel format, or kFmtF32
 };
 
 // Monotone float <-> uint key so that atomicMin on the key is a float min.

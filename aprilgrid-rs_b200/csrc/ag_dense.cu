@@ -36,16 +36,31 @@ AG_D float unorm16_to_f32(float v) {
 AG_D uint32_t rgb_luma_u8(uint32_t r, uint32_t g, uint32_t b) {
   return (2126u * r + 7152u * g + 722u * b) / 10000u;
 }
+// The same on u16 (Y16); the largest sum, 655 350 000, fits 32 bits.
+AG_D uint32_t rgb_luma_u16(uint32_t r, uint32_t g, uint32_t b) {
+  return (2126u * r + 7152u * g + 722u * b) / 10000u;
+}
 
 template <int FMT>
 AG_D float load_luma(const uint8_t* __restrict__ frame, size_t row_stride, int x, int y) {
   const uint8_t* row = frame + (size_t)y * row_stride;
+  const uint16_t* row16 = reinterpret_cast<const uint16_t*>(row);
   if (FMT == AG_L8) {
     return unorm8_to_f32((float)row[x]);
   } else if (FMT == AG_L16) {
-    return unorm16_to_f32((float)reinterpret_cast<const uint16_t*>(row)[x]);
+    return unorm16_to_f32((float)row16[x]);
   } else if (FMT == kFmtF32) {
     return reinterpret_cast<const float*>(row)[x];
+  } else if (FMT == AG_LA8) {  // alpha never contributes
+    return unorm8_to_f32((float)row[2 * x]);
+  } else if (FMT == AG_RGBA8) {
+    const uint8_t* p = row + 4 * x;
+    return unorm8_to_f32((float)rgb_luma_u8(p[0], p[1], p[2]));
+  } else if (FMT == AG_LA16) {
+    return unorm16_to_f32((float)row16[2 * x]);
+  } else if (FMT == AG_RGB16 || FMT == AG_RGBA16) {
+    const uint16_t* p = row16 + (FMT == AG_RGB16 ? 3 : 4) * x;
+    return unorm16_to_f32((float)rgb_luma_u16(p[0], p[1], p[2]));
   } else {
     const uint8_t* p = row + 3 * x;
     return unorm8_to_f32((float)rgb_luma_u8(p[0], p[1], p[2]));
@@ -157,7 +172,8 @@ k_blur_hessian_tile(const uint8_t* __restrict__ frames, FrameGeom g, float* __re
 //   * Hessian: the last three blurred rows of the 4 columns plus one halo column per side.
 // No shared memory, no block barrier.  Clamp-to-edge is obtained by clamping the loaded row /
 // replicating the edge pixel.  Requires width % 4 == 0 and rows aligned to the lane's load
-// (4 bytes for L8 and RGB8 -- a lane's 4 RGB pixels are three words --, 8 bytes for L16).
+// (4 bytes for L8 and RGB8 -- a lane's 4 RGB pixels are three words --, 8 bytes for L16, LA8 and
+// RGB16, 16 bytes for the other formats; see launch_blur_hessian).
 // -----------------------------------------------------------------------------------------
 constexpr int S_COLS = 120;  // output columns per warp
 // Output rows per warp (chunk): the launcher picks one of these.  chunk + 8 row steps (7 rows of
@@ -171,30 +187,85 @@ AG_D float u8_lane(uint32_t word, int k) {  // byte k of a packed pixel word -> 
   return unorm8_to_f32((float)((word >> (8 * k)) & 0xffu));
 }
 
-// A lane's 4 raw pixels of one row: 1 (L8), 2 (L16) or 3 (RGB8) 32-bit words.
+// A lane's 4 raw pixels of one row: 1 (L8), 2 (L16), 3 (RGB8) or 4 (f32) 32-bit words.
 template <int FMT>
 struct RawPx {
-  static constexpr int NW = FMT == AG_L8 ? 1 : (FMT == AG_L16 ? 2 : (FMT == kFmtF32 ? 4 : 3));
+  static constexpr int NW = bytes_per_px(FMT);
   uint32_t w[NW];
 };
+// What a lane keeps of a row of format FMT until its use.  The formats with alpha or 16-bit colour
+// are reduced to gray one row step after the load, to one L8 word (LA8, RGBA8: the luma bytes) or
+// two L16 words (LA16, RGB16, RGBA16: the luma words), so that only the newest row in flight costs
+// its raw registers and the rest of the row step is the L8 / L16 code.
+template <int FMT>
+constexpr int kLaneFmt = (FMT == AG_LA8 || FMT == AG_RGBA8) ? AG_L8
+                       : (FMT == AG_LA16 || FMT == AG_RGB16 || FMT == AG_RGBA16) ? AG_L16 : FMT;
+AG_D uint32_t lo16(uint32_t v) { return v & 0xffffu; }
+AG_D uint32_t hi16(uint32_t v) { return v >> 16; }
+AG_D uint32_t rgba8_luma(uint32_t px) {  // one R G B A pixel word -> Y8
+  return rgb_luma_u8(px & 0xffu, (px >> 8) & 0xffu, (px >> 16) & 0xffu);
+}
+// A lane's raw words of one row (vector loads as wide as the lane's alignment allows).
 template <int FMT>
 AG_D RawPx<FMT> load_raw(const uint8_t* p) {
   RawPx<FMT> r;
-  if (FMT == AG_L16) {
+  constexpr int NW = RawPx<FMT>::NW;
+  if (NW == 2) {  // L16, LA8: one 8-byte load
     const uint2 v = __ldg(reinterpret_cast<const uint2*>(p));
     r.w[0] = v.x;
-    r.w[RawPx<FMT>::NW - 1] = v.y;
-  } else if (FMT == kFmtF32) {
-    const uint4 v = __ldg(reinterpret_cast<const uint4*>(p));
-    r.w[0] = v.x;
-    r.w[1 % RawPx<FMT>::NW] = v.y;
-    r.w[2 % RawPx<FMT>::NW] = v.z;
-    r.w[3 % RawPx<FMT>::NW] = v.w;
-  } else {
+    r.w[NW - 1] = v.y;
+  } else if (NW == 4 || NW == 8) {  // f32, RGBA8, LA16: one 16-byte load; RGBA16: two
 #pragma unroll
-    for (int i = 0; i < RawPx<FMT>::NW; ++i) r.w[i] = __ldg(reinterpret_cast<const uint32_t*>(p) + i);
+    for (int i = 0; i < NW; i += 4) {
+      const uint4 v = __ldg(reinterpret_cast<const uint4*>(p) + i / 4);
+      r.w[i] = v.x;
+      r.w[(i + 1) % NW] = v.y;
+      r.w[(i + 2) % NW] = v.z;
+      r.w[(i + 3) % NW] = v.w;
+    }
+  } else if (NW == 6) {  // RGB16: three 8-byte loads
+#pragma unroll
+    for (int i = 0; i < NW; i += 2) {
+      const uint2 v = __ldg(reinterpret_cast<const uint2*>(p) + i / 2);
+      r.w[i] = v.x;
+      r.w[(i + 1) % NW] = v.y;
+    }
+  } else {  // L8, RGB8: 32-bit words
+#pragma unroll
+    for (int i = 0; i < NW; ++i) r.w[i] = __ldg(reinterpret_cast<const uint32_t*>(p) + i);
   }
   return r;
+}
+// A lane's raw words -> what it keeps of the row (kLaneFmt); the identity for L8, L16, RGB8 and f32.
+template <int FMT>
+AG_D RawPx<kLaneFmt<FMT>> pack_raw(const RawPx<FMT>& v) {
+  if constexpr (kLaneFmt<FMT> == FMT) {
+    return v;
+  } else {
+    RawPx<kLaneFmt<FMT>> r;
+    constexpr int NW = RawPx<kLaneFmt<FMT>>::NW, NI = RawPx<FMT>::NW;
+    const uint32_t* x = v.w;
+    if (FMT == AG_LA8) {  // L A L A | L A L A -> L L L L
+      r.w[0] = __byte_perm(x[0], x[1 % NI], 0x6420);
+    } else if (FMT == AG_RGBA8) {  // a pixel per word
+      r.w[0] = rgba8_luma(x[0]) | (rgba8_luma(x[1 % NI]) << 8) | (rgba8_luma(x[2 % NI]) << 16) |
+               (rgba8_luma(x[3 % NI]) << 24);
+    } else if (FMT == AG_LA16) {  // L A per word
+      r.w[0] = __byte_perm(x[0], x[1 % NI], 0x5410);
+      r.w[1 % NW] = __byte_perm(x[2 % NI], x[3 % NI], 0x5410);
+    } else if (FMT == AG_RGB16) {  // R0 G0 | B0 R1 | G1 B1 | R2 G2 | B2 R3 | G3 B3
+      r.w[0] = rgb_luma_u16(lo16(x[0]), hi16(x[0]), lo16(x[1 % NI])) |
+               (rgb_luma_u16(hi16(x[1 % NI]), lo16(x[2 % NI]), hi16(x[2 % NI])) << 16);
+      r.w[1 % NW] = rgb_luma_u16(lo16(x[3 % NI]), hi16(x[3 % NI]), lo16(x[4 % NI])) |
+                    (rgb_luma_u16(hi16(x[4 % NI]), lo16(x[5 % NI]), hi16(x[5 % NI])) << 16);
+    } else {  // RGBA16: R G | B A per pixel
+      r.w[0] = rgb_luma_u16(lo16(x[0]), hi16(x[0]), lo16(x[1 % NI])) |
+               (rgb_luma_u16(lo16(x[2 % NI]), hi16(x[2 % NI]), lo16(x[3 % NI])) << 16);
+      r.w[1 % NW] = rgb_luma_u16(lo16(x[4 % NI]), hi16(x[4 % NI]), lo16(x[5 % NI])) |
+                    (rgb_luma_u16(lo16(x[6 % NI]), hi16(x[6 % NI]), lo16(x[7 % NI])) << 16);
+    }
+    return r;
+  }
 }
 // luma f32 of pixel k (0..3) of the lane's raw pixels (image 0.25 to_luma32f, see load_luma)
 template <int FMT>
@@ -230,7 +301,8 @@ k_blur_hessian_stream(const uint8_t* __restrict__ frames, FrameGeom g, int chunk
   const int Y0 = blockIdx.y * chunk_rows, Y1 = min(Y0 + chunk_rows, g.h);
   const int c0 = X0 - 4 + 4 * lane;  // first of this lane's 4 columns (may lie outside the image)
   const int cw = min(max(c0, 0), g.w - 4);  // column of the word actually loaded
-  constexpr int kBpp = FMT == AG_L8 ? 1 : (FMT == AG_L16 ? 2 : (FMT == kFmtF32 ? 4 : 3));
+  constexpr int kBpp = bytes_per_px(FMT);
+  constexpr int LF = kLaneFmt<FMT>;  // the format of what load_raw returns
   // frame bases are block-uniform; what varies per lane and row are 32-bit offsets (the launcher
   // checks that a frame's bytes fit them)
   // The lane's pointers into the frame are held in registers (opaque, or the compiler re-derives
@@ -272,24 +344,27 @@ k_blur_hessian_stream(const uint8_t* __restrict__ frames, FrameGeom g, int chunk
   const uint32_t out_row_bytes = (uint32_t)g.w * 4u;
 
   const int r_begin = Y0 - 4, r_end = Y1 + 3;  // temp rows r_begin..r_end inclusive
-  RawPx<FMT> w_cur = load_row(r_begin), w_n1 = load_row(r_begin + 1), w_n2 = load_row(r_begin + 2);
+  // rows r + 1 and r + 2 as kept (kLaneFmt), row r + 3 as loaded: a row is reduced one step after its
+  // load, when the load has had a row step to arrive
+  RawPx<LF> w_cur = pack_raw<FMT>(load_row(r_begin)), w_n1 = pack_raw<FMT>(load_row(r_begin + 1));
+  RawPx<FMT> w_n2 = load_row(r_begin + 2);
 
   // One row step: consumes raw row r, completes blurred row r-3 into N, emits Hessian row r-4
   // from M (row r-5), C (row r-4), N (row r-3).
   auto step = [&](int r, const BlurRow& M, const BlurRow& C, BlurRow& N) {
-    RawPx<FMT> wd = w_cur;
+    RawPx<LF> wd = w_cur;
     w_cur = w_n1;
-    w_n1 = w_n2;
+    w_n1 = pack_raw<FMT>(w_n2);
     w_n2 = load_row(r + 3);  // three rows ahead
-    if (FMT == AG_L8 && edge_strip) {
+    if (LF == AG_L8 && edge_strip) {
       if (left_out) wd.w[0] = (wd.w[0] & 0xffu) * 0x01010101u;  // replicate pixel 0
       if (right_out) wd.w[0] = (wd.w[0] >> 24) * 0x01010101u;   // replicate pixel w-1
     }
     // ---- gray conversion + halo exchange: p[0..9] = pixels c0-3 .. c0+6
     float p[10];
-    p[3] = raw_luma<FMT>(wd, 0); p[4] = raw_luma<FMT>(wd, 1); p[5] = raw_luma<FMT>(wd, 2);
-    p[6] = raw_luma<FMT>(wd, 3);
-    if (FMT != AG_L8 && edge_strip) {  // strips hanging over the image edge replicate the edge pixel
+    p[3] = raw_luma<LF>(wd, 0); p[4] = raw_luma<LF>(wd, 1); p[5] = raw_luma<LF>(wd, 2);
+    p[6] = raw_luma<LF>(wd, 3);
+    if (LF != AG_L8 && edge_strip) {  // strips hanging over the image edge replicate the edge pixel
       if (left_out) p[4] = p[5] = p[6] = p[3];
       if (right_out) p[3] = p[4] = p[5] = p[6];
     }
@@ -619,7 +694,10 @@ int launch_blur_hessian(const uint8_t* frames, const FrameGeom& g, int n_frames,
   int launches = 0;
   k_fill_u32<<<(n_frames + 255) / 256, 256, 0, s>>>(frame_min, n_frames, kOrderedFltMax);
   ++launches;
-  const size_t al = g.format == AG_L16 ? 8 : (g.format == kFmtF32 ? 16 : 4);  // alignment of a lane's load
+  // alignment of a lane's loads: L8 and RGB8 load 32-bit words, L16, LA8 and RGB16 8-byte words,
+  // the others 16-byte words
+  const int bpp = bytes_per_px(g.format);
+  const size_t al = bpp == 1 || bpp == 3 ? 4 : (bpp == 2 || bpp == 6 ? 8 : 16);
   const bool can_stream = (g.w % 4) == 0 && g.w >= 8 && (g.row_stride % al) == 0 && (g.frame_stride % al) == 0 &&
                           ((uintptr_t)frames % al) == 0 && variant != 1 &&
                           (uint64_t)g.row_stride * (uint64_t)g.h < (1ull << 32);  // 32-bit offsets within a frame
@@ -645,6 +723,11 @@ int launch_blur_hessian(const uint8_t* frames, const FrameGeom& g, int n_frames,
       case AG_L8: AG_STREAM(AG_L8); break;
       case AG_L16: AG_STREAM(AG_L16); break;
       case kFmtF32: AG_STREAM(kFmtF32); break;
+      case AG_LA8: AG_STREAM(AG_LA8); break;
+      case AG_RGBA8: AG_STREAM(AG_RGBA8); break;
+      case AG_LA16: AG_STREAM(AG_LA16); break;
+      case AG_RGB16: AG_STREAM(AG_RGB16); break;
+      case AG_RGBA16: AG_STREAM(AG_RGBA16); break;
       default: AG_STREAM(AG_RGB8); break;
     }
 #undef AG_STREAM
@@ -654,6 +737,11 @@ int launch_blur_hessian(const uint8_t* frames, const FrameGeom& g, int n_frames,
     case AG_L8: launch_tile<AG_L8>(frames, g, n_frames, blur, resp, frame_min, write_blur, s); break;
     case AG_L16: launch_tile<AG_L16>(frames, g, n_frames, blur, resp, frame_min, write_blur, s); break;
     case kFmtF32: launch_tile<kFmtF32>(frames, g, n_frames, blur, resp, frame_min, write_blur, s); break;
+    case AG_LA8: launch_tile<AG_LA8>(frames, g, n_frames, blur, resp, frame_min, write_blur, s); break;
+    case AG_RGBA8: launch_tile<AG_RGBA8>(frames, g, n_frames, blur, resp, frame_min, write_blur, s); break;
+    case AG_LA16: launch_tile<AG_LA16>(frames, g, n_frames, blur, resp, frame_min, write_blur, s); break;
+    case AG_RGB16: launch_tile<AG_RGB16>(frames, g, n_frames, blur, resp, frame_min, write_blur, s); break;
+    case AG_RGBA16: launch_tile<AG_RGBA16>(frames, g, n_frames, blur, resp, frame_min, write_blur, s); break;
     default: launch_tile<AG_RGB8>(frames, g, n_frames, blur, resp, frame_min, write_blur, s); break;
   }
   return launches + 1;

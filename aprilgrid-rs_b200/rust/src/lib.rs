@@ -133,6 +133,11 @@ mod ffi {
 const AG_L8: c_int = 0;
 const AG_L16: c_int = 1;
 const AG_RGB8: c_int = 2;
+const AG_LA8: c_int = 4;
+const AG_RGBA8: c_int = 5;
+const AG_LA16: c_int = 6;
+const AG_RGB16: c_int = 7;
+const AG_RGBA16: c_int = 8;
 const AG_ERR_CAPACITY: c_int = 4;
 const TAG_CAP: usize = 1024; // >= the largest family (587 codes)
 
@@ -184,14 +189,12 @@ fn last_error(h: *const ffi::AgDetector) -> String {
     unsafe { std::ffi::CStr::from_ptr(ffi::ag_last_error(h)).to_string_lossy().into_owned() }
 }
 
-/// Raw pixel view of the DynamicImage variants the detect path is used with (Luma8, Luma16,
-/// Rgb8: passed through untouched, converted on the GPU exactly as `image` 0.25 does).
-/// `detect` handles every OTHER variant exactly as the reference does:
-/// they compute `img.to_luma32f()` and `img.to_luma8()` with the `image` crate itself
-/// (src/detector.rs:409, :507) and hand both planes to `ag_detect_planes`.  Only `detect_batch`
-/// (frames packed into one buffer of one format) converts such variants first -- with `image`'s own
-/// `to_luma16()` (16-bit and float sources) or `to_rgb8()` (8-bit sources with alpha) -- where for
-/// e.g. Rgb16 the last bits of the float gray image can differ from the reference's.
+/// Raw pixel view of a DynamicImage.  The eight integer variants (Luma8, LumaA8, Rgb8, Rgba8 and
+/// their 16-bit forms) are passed through untouched and converted on the GPU as `image` 0.25 does.
+/// The float variants (Rgb32F, Rgba32F) have no pixel format of the library: `detect` hands the
+/// reference's own planes, `img.to_luma32f()` and `img.to_luma8()` (src/detector.rs:409, :507), to
+/// `ag_detect_planes`; `detect_batch` and `refined_saddle_points` convert them first with `image`'s
+/// own `to_luma16()`, where the last bits of the float gray image can differ from the reference's.
 enum Pixels<'a> {
     Borrowed(&'a [u8], c_int, usize),
     Owned(Vec<u8>, c_int, usize),
@@ -215,10 +218,12 @@ fn pixels_of(img: &DynamicImage) -> (Pixels<'_>, u32, u32) {
         DynamicImage::ImageLuma8(b) => (Pixels::Borrowed(b.as_raw(), AG_L8, w as usize), w, h),
         DynamicImage::ImageRgb8(b) => (Pixels::Borrowed(b.as_raw(), AG_RGB8, 3 * w as usize), w, h),
         DynamicImage::ImageLuma16(b) => (Pixels::Borrowed(u16_bytes(b.as_raw()), AG_L16, 2 * w as usize), w, h),
-        DynamicImage::ImageLumaA8(_) | DynamicImage::ImageRgba8(_) => {
-            (Pixels::Owned(img.to_rgb8().into_raw(), AG_RGB8, 3 * w as usize), w, h)
-        }
-        other => {
+        DynamicImage::ImageLumaA8(b) => (Pixels::Borrowed(b.as_raw(), AG_LA8, 2 * w as usize), w, h),
+        DynamicImage::ImageRgba8(b) => (Pixels::Borrowed(b.as_raw(), AG_RGBA8, 4 * w as usize), w, h),
+        DynamicImage::ImageLumaA16(b) => (Pixels::Borrowed(u16_bytes(b.as_raw()), AG_LA16, 4 * w as usize), w, h),
+        DynamicImage::ImageRgb16(b) => (Pixels::Borrowed(u16_bytes(b.as_raw()), AG_RGB16, 6 * w as usize), w, h),
+        DynamicImage::ImageRgba16(b) => (Pixels::Borrowed(u16_bytes(b.as_raw()), AG_RGBA16, 8 * w as usize), w, h),
+        other => {  // Rgb32F, Rgba32F
             let l16 = other.to_luma16();
             (Pixels::Owned(u16_bytes(l16.as_raw()).to_vec(), AG_L16, 2 * w as usize), w, h)
         }
@@ -277,16 +282,16 @@ impl TagDetector {
 
     pub fn detect(&self, img: &DynamicImage) -> HashMap<u32, [(f32, f32); 4]> {
         match img {
-            DynamicImage::ImageLuma8(_) | DynamicImage::ImageLuma16(_) | DynamicImage::ImageRgb8(_) => {
+            DynamicImage::ImageRgb32F(_) | DynamicImage::ImageRgba32F(_) => self.detect_planes(img),
+            _ => {
                 let (px, w, h) = pixels_of(img);
                 let (bytes, fmt, stride) = px.parts();
                 self.detect_raw(bytes.as_ptr(), w, h, stride, fmt)
             }
-            other => self.detect_planes(other),
         }
     }
 
-    /// Any other variant: the reference's own conversions (`to_luma32f`, `to_luma8`), both planes to the GPU.
+    /// The float variants: the reference's own conversions (`to_luma32f`, `to_luma8`), both planes to the GPU.
     fn detect_planes(&self, img: &DynamicImage) -> HashMap<u32, [(f32, f32); 4]> {
         let luma32f = img.to_luma32f();
         let luma8 = img.to_luma8();

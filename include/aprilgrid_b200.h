@@ -51,11 +51,23 @@ enum {
   AG_T36H11B1 = 4 /* 1-bit border */
 };
 
-/* ---- pixel formats: the DynamicImage variants the detect path is used with -------- */
+/* ---- pixel formats: the integer DynamicImage variants, channels interleaved ----------
+ * Gray conversion as `image` 0.25 does it (to_luma32f for the stencils, to_luma8 for bit
+ * sampling): alpha is dropped; colour is the integer sRGB luma (2126 R + 7152 G + 722 B) / 10000,
+ * computed and truncated in the source type's width (u8 -> Y8, u16 -> Y16, 32-bit arithmetic);
+ * then to_luma32f = Y8 / 255 or Y16 / 65535 (correctly rounded) and to_luma8 = Y8 or
+ * (Y16 + 128) / 257.  16-bit words are native endian.  Value 3 is reserved (an internal f32 plane).
+ * The 16-bit formats need even row and frame strides everywhere and an even device address
+ * on the device entry points (else AG_ERR_INVALID; nothing runs).                          */
 enum {
-  AG_L8 = 0,   /* ImageLuma8  : 1 byte / px                                   */
-  AG_L16 = 1,  /* ImageLuma16 : 2 bytes / px, native endian                   */
-  AG_RGB8 = 2  /* ImageRgb8   : 3 bytes / px, interleaved (detect_kornia N=3) */
+  AG_L8 = 0,     /* ImageLuma8   : 1 byte / px                                   */
+  AG_L16 = 1,    /* ImageLuma16  : 2 bytes / px                                  */
+  AG_RGB8 = 2,   /* ImageRgb8    : 3 bytes / px, R G B (detect_kornia N=3)       */
+  AG_LA8 = 4,    /* ImageLumaA8  : 2 bytes / px, L A                             */
+  AG_RGBA8 = 5,  /* ImageRgba8   : 4 bytes / px, R G B A                         */
+  AG_LA16 = 6,   /* ImageLumaA16 : 4 bytes / px, L A (u16 each)                  */
+  AG_RGB16 = 7,  /* ImageRgb16   : 6 bytes / px, R G B (u16 each)                */
+  AG_RGBA16 = 8  /* ImageRgba16  : 8 bytes / px, R G B A (u16 each)              */
 };
 
 /* ---- DetectorParams (src/detector.rs:25-41) -------------------------------------- */
@@ -132,9 +144,9 @@ AG_API int ag_detect(ag_detector* det, const void* pixels, int width, int height
 
 /* TagDetector::detect on a frame given as the TWO gray planes the reference derives from its
  * DynamicImage itself: luma32f = img.to_luma32f() (the stencil chain, src/detector.rs:409) and
- * luma8 = img.to_luma8() (bit sampling, :507).  For DynamicImage variants other than Luma8 / Luma16 /
- * Rgb8 (Rgb16, Rgba8, Rgb32F ...) a shim computes both planes with the `image` crate and calls
- * this: the conversion is then the reference's own, whatever the variant.  Row strides in bytes
+ * luma8 = img.to_luma8() (bit sampling, :507).  For the float DynamicImage variants (Rgb32F,
+ * Rgba32F), which have no pixel format above, a shim computes both planes with the `image` crate
+ * and calls this: the conversion is then the reference's own.  Row strides in bytes
  * (0 = packed).  Synchronous; same result and error conventions as ag_detect.              */
 AG_API int ag_detect_planes(ag_detector* det, const float* luma32f, size_t f32_row_stride,
                             const uint8_t* luma8, size_t u8_row_stride, int width, int height,
@@ -142,7 +154,7 @@ AG_API int ag_detect_planes(ag_detector* det, const float* luma32f, size_t f32_r
 
 /* detect_batch: n_frames host images of one shape at frames + i*frame_stride.
  * out[i*cap_per_frame ..], n_per_frame[i]; frame_status may be NULL.
- * Strides in bytes (0 = packed); for AG_L16 both must be even (else AG_ERR_INVALID).      */
+ * Strides in bytes (0 = packed); for 16-bit formats both must be even (else AG_ERR_INVALID). */
 AG_API int ag_detect_batch(ag_detector* det, const void* frames, size_t frame_stride,
                            int n_frames, int width, int height, size_t row_stride, int format,
                            ag_tag* out, int cap_per_frame, int* n_per_frame,
@@ -152,7 +164,7 @@ AG_API int ag_detect_batch(ag_detector* det, const void* frames, size_t frame_st
  * (d_out: n_frames*cap_per_frame ag_tag, d_n_per_frame: n_frames int32,
  *  d_frame_status: n_frames uint32 or NULL).  Work is enqueued on `stream`
  * (a cudaStream_t, NULL = the detector's own stream) and is asynchronous.
- * AG_L16 frames must start at an even device address (else AG_ERR_INVALID; nothing runs). */
+ * 16-bit formats must start at an even device address (else AG_ERR_INVALID; nothing runs). */
 AG_API int ag_detect_batch_device(ag_detector* det, const void* d_frames, size_t frame_stride,
                                   int n_frames, int width, int height, size_t row_stride,
                                   int format, ag_tag* d_out, int cap_per_frame,
@@ -198,7 +210,7 @@ AG_API int ag_gaussian_blur_f32_device(ag_detector* det, const float* d_in, int 
 
 /* Dense front end only (gray -> blur -> Hessian -> min -> threshold mask), device-resident
  * frames, results stay in the detector's workspace.  This is the unit bench.py times for
- * the "blur / threshold kernels alone" configuration.  AG_L16: even address and strides. */
+ * the "blur / threshold kernels alone" configuration.  16-bit formats: even address and strides. */
 AG_API int ag_dense_batch_device(ag_detector* det, const void* d_frames, size_t frame_stride,
                                  int n_frames, int width, int height, size_t row_stride,
                                  int format, void* stream);
