@@ -24,9 +24,11 @@ if os.environ.get("AG_LIB"):  # profiling tools only: another build of the same 
 AG_OK, AG_ERR_INVALID, AG_ERR_NO_DEVICE, AG_ERR_CUDA, AG_ERR_CAPACITY, AG_ERR_UNSUPPORTED = range(6)
 FMT_L8, FMT_L16, FMT_RGB8 = 0, 1, 2
 FMT_LA8, FMT_RGBA8, FMT_LA16, FMT_RGB16, FMT_RGBA16 = 4, 5, 6, 7, 8  # 3 is reserved
+FMT_RGB32F, FMT_RGBA32F = 9, 10
 # (channels, dtype) -> pixel format of an H x W x channels image (DynamicImage LumaA / Rgb / Rgba)
 _CHANNEL_FORMATS = {(2, np.uint8): FMT_LA8, (3, np.uint8): FMT_RGB8, (4, np.uint8): FMT_RGBA8,
-                    (2, np.uint16): FMT_LA16, (3, np.uint16): FMT_RGB16, (4, np.uint16): FMT_RGBA16}
+                    (2, np.uint16): FMT_LA16, (3, np.uint16): FMT_RGB16, (4, np.uint16): FMT_RGBA16,
+                    (3, np.float32): FMT_RGB32F, (4, np.float32): FMT_RGBA32F}
 
 TAG_DTYPE = np.dtype([("id", np.uint32), ("xy", np.float32, (8,))])
 SADDLE_DTYPE = np.dtype([("x", np.float32), ("y", np.float32), ("k", np.float32),
@@ -134,6 +136,8 @@ def lib():
         L.ag_test_board_decode_room.argtypes = [ci, ci, ci, vp]
         L.ag_test_render_pose.argtypes = [vp, vp, ci, ci, ci, ci, vp, ci, C.c_uint64]
         L.ag_test_boards_from_saddles.argtypes = [vp, vp, ci, vp, ci, ci, sz, ci, vp, ci, vp, vp, ci, vp]
+        L.ag_test_float_luma.argtypes = [vp, vp, C.c_longlong, ci, vp, vp]
+        L.ag_test_host_chunk.argtypes = [C.c_longlong, ci, vp]
         _lib = L
     return _lib
 
@@ -143,15 +147,18 @@ def _p(a):
 
 
 def image_format(img):
-    """(fmt, width, height, row_stride_bytes) for HxW u8 (Luma8) / u16 (Luma16), and HxWxN u8 / u16
-    with N = 2 (LumaA8 / LumaA16), 3 (Rgb8 / Rgb16) or 4 (Rgba8 / Rgba16), channels interleaved."""
+    """(fmt, width, height, row_stride_bytes) for HxW u8 (Luma8) / u16 (Luma16), HxWxN u8 / u16
+    with N = 2 (LumaA8 / LumaA16), 3 (Rgb8 / Rgb16) or 4 (Rgba8 / Rgba16), and HxWxN float32 with
+    N = 3 (Rgb32F) or 4 (Rgba32F); channels interleaved.  HxW float32 is no DynamicImage variant:
+    see TagDetector.detect_planes."""
     if img.ndim == 2 and img.dtype == np.uint8:
         return FMT_L8, img.shape[1], img.shape[0], img.strides[0]
     if img.ndim == 2 and img.dtype == np.uint16:
         return FMT_L16, img.shape[1], img.shape[0], img.strides[0]
     if img.ndim == 3 and (img.shape[2], img.dtype.type) in _CHANNEL_FORMATS:
         return _CHANNEL_FORMATS[(img.shape[2], img.dtype.type)], img.shape[1], img.shape[0], img.strides[0]
-    raise ValueError("unsupported image: shape %s dtype %s (want HxW or HxWxN, N in 2..4, u8/u16)"
+    raise ValueError("unsupported image: shape %s dtype %s (want HxW or HxWxN u8/u16 with N in 2..4, "
+                     "or HxWxN float32 with N in 3..4)"
                      % (img.shape, img.dtype))
 
 
@@ -253,7 +260,8 @@ class TagDetector:
         return self.detect(np.ascontiguousarray(img))
 
     def detect_batch(self, frames, cap_per_frame=128, return_status=False):
-        """New batched entry point: frames is N x H x W or N x H x W x C (C in 2..4), u8 or u16."""
+        """New batched entry point: frames is N x H x W or N x H x W x C (C in 2..4), u8 or u16, or
+        N x H x W x C (C in 3..4) float32."""
         frames = np.asarray(frames)
         if not frames.flags.c_contiguous:
             frames = np.ascontiguousarray(frames)
@@ -397,11 +405,29 @@ class TagDetector:
         self._check(lib().ag_test_board_times(self._h, slot, _p(out), n_frames))
         return out
 
+    def _float_luma(self, pixels):
+        """Test hook: the device's to_luma32f / to_luma8 of float pixels (M x 3 or M x 4 float32)."""
+        px = np.ascontiguousarray(pixels, np.float32)
+        if px.ndim != 2 or px.shape[1] not in (3, 4):
+            raise ValueError("want M x 3 or M x 4 float32 pixels")
+        l32, l8 = np.zeros(len(px), np.float32), np.zeros(len(px), np.uint8)
+        self._check(lib().ag_test_float_luma(self._h, _p(px), len(px), px.shape[1], _p(l32), _p(l8)))
+        return l32, l8
+
     def _unorm_tables(self):
         o8, o16 = np.zeros(256, np.float32), np.zeros(65536, np.float32)
         r8, r16 = np.zeros(256, np.float32), np.zeros(65536, np.float32)
         self._check(lib().ag_test_unorm_tables(self._h, _p(o8), _p(o16), _p(r8), _p(r16)))
         return o8, o16, r8, r16
+
+
+def host_chunk_frames(host_chunk, fmt):
+    """Test hook (no GPU): frames per chunk of the host-buffer path for option host_chunk_frames and a
+    pixel format, before the bound on the dense buffers."""
+    out = C.c_longlong(0)
+    if lib().ag_test_host_chunk(int(host_chunk), int(fmt), C.byref(out)) != AG_OK:
+        raise ValueError("bad host_chunk_frames or format")
+    return out.value
 
 
 def pinned_empty(shape, dtype=np.uint8):

@@ -39,12 +39,12 @@ struct Saddle {  // src/saddle.rs:3-9
   float k, theta, phi;
 };
 
-// A borrowed image in one of the integer DynamicImage variants (the AG_* pixel formats).
+// A borrowed image in one of the DynamicImage variants (the AG_* pixel formats).
 struct ImageView {
   const void* pixels;
   int width, height;
   size_t row_stride;  // bytes; 0 = tightly packed
-  int format;         // AG_L8 .. AG_RGBA16 (include/aprilgrid_b200.h)
+  int format;         // AG_L8 .. AG_RGBA32F (include/aprilgrid_b200.h)
 };
 
 using TagMap = std::unordered_map<uint32_t, std::array<std::pair<float, float>, 4>>;

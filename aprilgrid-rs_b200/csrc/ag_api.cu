@@ -227,15 +227,15 @@ int make_geom(ag_detector* det, int w, int h, size_t row_stride, size_t frame_st
   size_t min_row = (size_t)w * bytes_per_px(format);
   if (row_stride == 0) row_stride = min_row;
   if (row_stride < min_row) return fail(det, AG_ERR_INVALID, "row_stride smaller than a row");
-  if (is_16bit_format(format) && (row_stride & 1))
-    return fail(det, AG_ERR_INVALID, "row_stride of a 16-bit format must be even");
+  const size_t al = (size_t)channel_align(format);
+  if (row_stride % al) return fail(det, AG_ERR_INVALID, "row_stride must be a multiple of the format's channel word");
   if (frame_stride == 0) frame_stride = row_stride * h;
   if (frame_stride < row_stride * (size_t)(h - 1) + min_row)
     return fail(det, AG_ERR_INVALID, "frame_stride smaller than a frame");
-  // every other frame of an odd stride would start at an odd address: K1 and K6 read 16-bit pixels
-  // with 2-byte loads (the host path keeps the caller's frame stride in its device staging too)
-  if (is_16bit_format(format) && (frame_stride & 1))
-    return fail(det, AG_ERR_INVALID, "frame_stride of a 16-bit format must be even");
+  // other frames of a misaligned stride would start misaligned: K1 and K6 read 16-bit and f32 channels
+  // with loads of their size (the host path keeps the caller's frame stride in its device staging too)
+  if (frame_stride % al)
+    return fail(det, AG_ERR_INVALID, "frame_stride must be a multiple of the format's channel word");
   g->w = w;
   g->h = h;
   g->wpr = (w + 31) / 32;
@@ -256,6 +256,13 @@ void set_caps(ag_detector* det, const FrameGeom& g) {
   if (nsd <= 0) nsd = std::min<long>(std::max<long>(((g.n_px / 640 + 255) / 256) * 256, 2048), 16384);
   det->cur_clusters = (int)ncl;
   det->cur_saddles = (int)nsd;
+}
+// Frames per chunk of the host-buffer path, before chunk_limit: the option host_chunk_frames, scaled
+// down for formats above 8 bytes per pixel so that a board slot's staging (device, and pinned for
+// pageable input) never holds more bytes per chunk than for RGBA16 frames of the same size.
+long host_chunk_for(long host_chunk_frames, int format) {
+  const int bpp = bytes_per_px(format);
+  return bpp > 8 ? std::max<long>(1, host_chunk_frames * 8 / bpp) : host_chunk_frames;
 }
 // Frames per pipeline chunk: the option, bounded so that the dense buffers of a chunk (blur +
 // response, 8 bytes per pixel) stay below 24 GB whatever the image size.
@@ -1020,8 +1027,8 @@ int ag_detect_batch_device(ag_detector* det, const void* d_frames, size_t frame_
   FrameGeom g;
   int rc = make_geom(det, width, height, row_stride, frame_stride, format, &g);
   if (rc) return rc;
-  if (is_16bit_format(format) && ((uintptr_t)d_frames & 1))
-    return fail(det, AG_ERR_INVALID, "frames of a 16-bit format must start at an even device address");
+  if ((uintptr_t)d_frames % channel_align(format))
+    return fail(det, AG_ERR_INVALID, "device frames must start at a multiple of the format's channel word");
   // chunks of host-buffer calls still in flight share the dense buffers and the board slots:
   // hand their results out first (streaming host calls and device calls do not overlap)
   if ((rc = collect_host(det, det->host_seq))) return rc;
@@ -1107,8 +1114,8 @@ int ag_dense_batch_device(ag_detector* det, const void* d_frames, size_t frame_s
   FrameGeom g;
   int rc = make_geom(det, width, height, row_stride, frame_stride, format, &g);
   if (rc) return rc;
-  if (is_16bit_format(format) && ((uintptr_t)d_frames & 1))
-    return fail(det, AG_ERR_INVALID, "frames of a 16-bit format must start at an even device address");
+  if ((uintptr_t)d_frames % channel_align(format))
+    return fail(det, AG_ERR_INVALID, "device frames must start at a multiple of the format's channel word");
   Slot& S = det->slot[0];
   set_caps(det, g);
   const int chunk = chunk_limit(det, g, std::min<long>(det->chunk_frames, std::max(n_frames, 1)));
@@ -1149,7 +1156,8 @@ static int detect_batch_host(ag_detector* det, const void* frames, size_t frame_
   // run on the dense stream, K6 and the download of the results on the board slot's stream, so
   // uploads, front end, board searches and downloads of up to eight chunks overlap.  The staged
   // input of a chunk stays in its board slot until K6 (which samples the tag bits) is done.
-  const int chunk = chunk_limit(det, g, std::min<long>(std::min<long>(det->chunk_frames, det->host_chunk_frames), n_frames));
+  const int chunk = chunk_limit(
+      det, g, std::min<long>(std::min<long>(det->chunk_frames, host_chunk_for(det->host_chunk_frames, format)), n_frames));
   Slot& D = det->slot[0];
   if ((rc = ensure_slot(det, D, g, chunk, 1, false, false))) return rc;
   if (!det->up_stream) AG_CUDA(det, cudaStreamCreateWithFlags(&det->up_stream, cudaStreamNonBlocking));
@@ -1680,6 +1688,14 @@ AG_API int ag_test_board_decode_room(int max_saddles, int lattice, int warps, lo
   return AG_OK;
 }
 
+// Test hook (not in the public header; needs no GPU): the frames per chunk of the host-buffer path
+// for a host_chunk_frames option and a pixel format, before the dense-buffer bound of chunk_limit.
+AG_API int ag_test_host_chunk(long long host_chunk_frames, int format, long long* out) {
+  if (!out || host_chunk_frames < 1 || format == kFmtF32 || bytes_per_px(format) == 0) return AG_ERR_INVALID;
+  *out = host_chunk_for((long)host_chunk_frames, format);
+  return AG_OK;
+}
+
 // Test hook (not in the public header): ONE frame of the renderer under a GIVEN pose -- hinv maps
 // image (x, y, 1) to page coordinates in tag sides (row-major 3x3, host pointer) -- with or without
 // the noise, so that tests can pin the renderer's geometry (id <-> lattice position, corner
@@ -1765,6 +1781,32 @@ AG_API int ag_test_unorm_tables(ag_detector* det, float* out8, float* out16, flo
   AG_CUDA(det, cudaMemcpy(ref8, r8, 256 * 4, cudaMemcpyDeviceToHost));
   AG_CUDA(det, cudaMemcpy(ref16, r16, 65536 * 4, cudaMemcpyDeviceToHost));
   cudaFree(d);
+  return AG_OK;
+}
+
+// Test hook (not in the public header): the device's gray conversion of n float pixels (channels 3:
+// R G B, 4: R G B A, host array) -> to_luma32f and to_luma8 of each (host arrays of n).
+AG_API int ag_test_float_luma(ag_detector* det, const float* rgb, long long n, int channels, float* out_luma32f,
+                              uint8_t* out_luma8) {
+  if (!det || !rgb || !out_luma32f || !out_luma8 || n < 0 || (channels != 3 && channels != 4)) return AG_ERR_INVALID;
+  if (n == 0) return AG_OK;
+  std::lock_guard<std::mutex> lk(det->mu);
+  AG_CUDA(det, cudaSetDevice(det->device));
+  const size_t in_bytes = sizeof(float) * channels * (size_t)n, out_bytes = 5 * (size_t)n;
+  uint8_t* d = nullptr;
+  AG_CUDA(det, cudaMalloc((void**)&d, in_bytes + out_bytes));
+  float* d_in = (float*)d;
+  float* d_l32 = (float*)(d + in_bytes);
+  uint8_t* d_l8 = d + in_bytes + 4 * (size_t)n;
+  cudaError_t e = cudaMemcpy(d_in, rgb, in_bytes, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) {
+    det->launches += launch_float_luma(d_in, n, channels, d_l32, d_l8, 0);
+    e = cudaDeviceSynchronize();
+  }
+  if (e == cudaSuccess) e = cudaMemcpy(out_luma32f, d_l32, 4 * (size_t)n, cudaMemcpyDeviceToHost);
+  if (e == cudaSuccess) e = cudaMemcpy(out_luma8, d_l8, (size_t)n, cudaMemcpyDeviceToHost);
+  cudaFree(d);
+  AG_CUDA(det, e);
   return AG_OK;
 }
 

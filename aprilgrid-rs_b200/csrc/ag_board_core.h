@@ -21,6 +21,7 @@
 #include <math.h>
 #include <stdint.h>
 
+#include "ag_float_luma.h"
 #include "ag_libm.h"
 
 #if defined(__CUDA_ARCH__)
@@ -1211,11 +1212,16 @@ AGB_NOINLINE int find_best_board(Frame& F) {
 }
 
 // ---- decoding (detector.rs:42-169, :448-476) ---------------------------------------------------
-// to_luma8 of pixel x of a row of LA8 (4), RGBA8 (5), LA16 (6), RGB16 (7) or RGBA16 (8): alpha is
-// dropped, colour is the integer sRGB luma in the source width, u16 luma is scaled to u8.  Out of
-// line, so that the frame formats of the benchmark keep the board kernel's code as it was.
+// to_luma8 of pixel x of a row of LA8 (4), RGBA8 (5), LA16 (6), RGB16 (7), RGBA16 (8), RGB32F (9) or
+// RGBA32F (10): alpha is dropped, colour is the integer sRGB luma in the source width (u16 luma is
+// scaled to u8) or, for f32, the f64 luma of ag_float_luma.h.  Out of line, so that the frame formats
+// of the benchmark keep the board kernel's code as it was.
 AGB_NOINLINE int luma8_wide(const uint8_t* row, uint32_t x, int format) {
   const uint16_t* r16 = (const uint16_t*)row;
+  if (format >= 9) {
+    const float* p = (const float*)row + (format == 9 ? 3 : 4) * (size_t)x;
+    return (int)ag::luma32f_to_u8(ag::rgb32f_luma(p[0], p[1], p[2]));
+  }
   if (format == 4) return row[2 * (size_t)x];
   if (format == 5) {
     const uint8_t* p = row + 4 * (size_t)x;

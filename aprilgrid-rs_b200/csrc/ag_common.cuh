@@ -9,6 +9,7 @@
 #include <stdint.h>
 
 #include "../../include/aprilgrid_b200.h"
+#include "ag_float_luma.h"
 
 #if defined(__CUDACC__)
 #define AG_HD __host__ __device__ __forceinline__
@@ -27,11 +28,14 @@ constexpr int kFmtF32 = 3;
 // Bytes of one pixel of format `fmt` (a public AG_* format or kFmtF32); 0 for any other value.
 AG_HD constexpr int bytes_per_px(int fmt) {
   return fmt == AG_L8 ? 1 : fmt == AG_L16 ? 2 : fmt == AG_RGB8 ? 3 : fmt == kFmtF32 ? 4 : fmt == AG_LA8 ? 2
-       : fmt == AG_RGBA8 ? 4 : fmt == AG_LA16 ? 4 : fmt == AG_RGB16 ? 6 : fmt == AG_RGBA16 ? 8 : 0;
+       : fmt == AG_RGBA8 ? 4 : fmt == AG_LA16 ? 4 : fmt == AG_RGB16 ? 6 : fmt == AG_RGBA16 ? 8
+       : fmt == AG_RGB32F ? 12 : fmt == AG_RGBA32F ? 16 : 0;
 }
-// The public formats whose pixels are 16-bit words: rows, frames and device frames must be 2-byte aligned.
-AG_HD constexpr bool is_16bit_format(int fmt) {
-  return fmt == AG_L16 || fmt == AG_LA16 || fmt == AG_RGB16 || fmt == AG_RGBA16;
+// Alignment in bytes of a pixel's channel words (1, 2 or 4): row strides, frame strides and the
+// address of device frames must be multiples of it (K1 and K6 read the words with loads of that size).
+AG_HD constexpr int channel_align(int fmt) {
+  return fmt == AG_L16 || fmt == AG_LA16 || fmt == AG_RGB16 || fmt == AG_RGBA16 ? 2
+       : fmt == AG_RGB32F || fmt == AG_RGBA32F ? 4 : 1;
 }
 
 constexpr int kBlurRadius = 3;  // ceil(2 * 1.5), src/image_util.rs:111

@@ -61,6 +61,9 @@ AG_D float load_luma(const uint8_t* __restrict__ frame, size_t row_stride, int x
   } else if (FMT == AG_RGB16 || FMT == AG_RGBA16) {
     const uint16_t* p = row16 + (FMT == AG_RGB16 ? 3 : 4) * x;
     return unorm16_to_f32((float)rgb_luma_u16(p[0], p[1], p[2]));
+  } else if (FMT == AG_RGB32F || FMT == AG_RGBA32F) {
+    const float* p = reinterpret_cast<const float*>(row) + (FMT == AG_RGB32F ? 3 : 4) * x;
+    return rgb32f_luma(p[0], p[1], p[2]);
   } else {
     const uint8_t* p = row + 3 * x;
     return unorm8_to_f32((float)rgb_luma_u8(p[0], p[1], p[2]));
@@ -187,19 +190,21 @@ AG_D float u8_lane(uint32_t word, int k) {  // byte k of a packed pixel word -> 
   return unorm8_to_f32((float)((word >> (8 * k)) & 0xffu));
 }
 
-// A lane's 4 raw pixels of one row: 1 (L8), 2 (L16), 3 (RGB8) or 4 (f32) 32-bit words.
+// A lane's 4 raw pixels of one row: as many 32-bit words as a pixel has bytes (1 for L8 ... 16 for RGBA32F).
 template <int FMT>
 struct RawPx {
   static constexpr int NW = bytes_per_px(FMT);
   uint32_t w[NW];
 };
-// What a lane keeps of a row of format FMT until its use.  The formats with alpha or 16-bit colour
-// are reduced to gray one row step after the load, to one L8 word (LA8, RGBA8: the luma bytes) or
-// two L16 words (LA16, RGB16, RGBA16: the luma words), so that only the newest row in flight costs
-// its raw registers and the rest of the row step is the L8 / L16 code.
+// What a lane keeps of a row of format FMT until its use.  The formats with alpha, 16-bit colour or
+// float colour are reduced to gray one row step after the load, to one L8 word (LA8, RGBA8: the luma
+// bytes), two L16 words (LA16, RGB16, RGBA16: the luma words) or four f32 words (RGB32F, RGBA32F:
+// to_luma32f), so that only the newest row in flight costs its raw registers and the rest of the row
+// step is the L8 / L16 / f32 code.
 template <int FMT>
 constexpr int kLaneFmt = (FMT == AG_LA8 || FMT == AG_RGBA8) ? AG_L8
-                       : (FMT == AG_LA16 || FMT == AG_RGB16 || FMT == AG_RGBA16) ? AG_L16 : FMT;
+                       : (FMT == AG_LA16 || FMT == AG_RGB16 || FMT == AG_RGBA16) ? AG_L16
+                       : (FMT == AG_RGB32F || FMT == AG_RGBA32F) ? kFmtF32 : FMT;
 AG_D uint32_t lo16(uint32_t v) { return v & 0xffffu; }
 AG_D uint32_t hi16(uint32_t v) { return v >> 16; }
 AG_D uint32_t rgba8_luma(uint32_t px) {  // one R G B A pixel word -> Y8
@@ -214,7 +219,7 @@ AG_D RawPx<FMT> load_raw(const uint8_t* p) {
     const uint2 v = __ldg(reinterpret_cast<const uint2*>(p));
     r.w[0] = v.x;
     r.w[NW - 1] = v.y;
-  } else if (NW == 4 || NW == 8) {  // f32, RGBA8, LA16: one 16-byte load; RGBA16: two
+  } else if (NW % 4 == 0) {  // f32, RGBA8, LA16: one 16-byte load; RGBA16: two; RGB32F: three; RGBA32F: four
 #pragma unroll
     for (int i = 0; i < NW; i += 4) {
       const uint4 v = __ldg(reinterpret_cast<const uint4*>(p) + i / 4);
@@ -253,6 +258,12 @@ AG_D RawPx<kLaneFmt<FMT>> pack_raw(const RawPx<FMT>& v) {
     } else if (FMT == AG_LA16) {  // L A per word
       r.w[0] = __byte_perm(x[0], x[1 % NI], 0x5410);
       r.w[1 % NW] = __byte_perm(x[2 % NI], x[3 % NI], 0x5410);
+    } else if (FMT == AG_RGB32F || FMT == AG_RGBA32F) {  // R G B (A) per pixel, one f32 per word
+      constexpr int C = FMT == AG_RGB32F ? 3 : 4;
+#pragma unroll
+      for (int k = 0; k < 4; ++k)
+        r.w[k % NW] = __float_as_uint(rgb32f_luma(__uint_as_float(x[(C * k) % NI]), __uint_as_float(x[(C * k + 1) % NI]),
+                                                  __uint_as_float(x[(C * k + 2) % NI])));
     } else if (FMT == AG_RGB16) {  // R0 G0 | B0 R1 | G1 B1 | R2 G2 | B2 R3 | G3 B3
       r.w[0] = rgb_luma_u16(lo16(x[0]), hi16(x[0]), lo16(x[1 % NI])) |
                (rgb_luma_u16(hi16(x[1 % NI]), lo16(x[2 % NI]), hi16(x[2 % NI])) << 16);
@@ -290,7 +301,10 @@ template <int FMT, bool WRITE_BLUR>
 #ifndef AG_K1_MIN_BLOCKS
 #define AG_K1_MIN_BLOCKS 7
 #endif
-__global__ void __launch_bounds__(S_WARPS * 32, FMT == AG_L8 ? AG_K1_MIN_BLOCKS : 6)
+// The float formats keep a row of 12 or 16 raw words in flight and convert it in f64: they need 114-120
+// registers, four blocks per SM (at 80 or 96 registers they spill).
+__global__ void __launch_bounds__(S_WARPS * 32, FMT == AG_L8 ? AG_K1_MIN_BLOCKS
+                                                : (FMT == AG_RGB32F || FMT == AG_RGBA32F) ? 4 : 6)
 k_blur_hessian_stream(const uint8_t* __restrict__ frames, FrameGeom g, int chunk_rows, float* __restrict__ blur,
                       float* __restrict__ resp, uint32_t* __restrict__ frame_min) {
   const int lane = threadIdx.x & 31;
@@ -377,10 +391,10 @@ k_blur_hessian_stream(const uint8_t* __restrict__ frames, FrameGeom g, int chunk
 #pragma unroll
     for (int c = 0; c < 4; ++c) {
       // ---- horizontal pass (image_util.rs:138-185): val = 0; val += px * k[i], i = 0..6
-      //      (0.0 + x*k0 == x*k0 for x >= 0; an f32 plane may hold negative values or -0.0, where
-      //      0.0 + (-0.0) = +0.0, so that instantiation keeps the addition)
+      //      (0.0 + x*k0 == x*k0 for x >= 0; an f32 plane or float pixels may give negative values or
+      //      -0.0, where 0.0 + (-0.0) = +0.0, so those instantiations keep the addition)
       float t = __fmul_rn(p[c], k0);
-      if (FMT == kFmtF32) t = __fadd_rn(0.0f, t);
+      if (LF == kFmtF32) t = __fadd_rn(0.0f, t);
       t = __fadd_rn(t, __fmul_rn(p[c + 1], k1));
       t = __fadd_rn(t, __fmul_rn(p[c + 2], k2));
       t = __fadd_rn(t, __fmul_rn(p[c + 3], k3));
@@ -396,7 +410,7 @@ k_blur_hessian_stream(const uint8_t* __restrict__ frames, FrameGeom g, int chunk
       a4[c] = __fadd_rn(a3[c], q3);       // tap 3 of row r
       a3[c] = __fadd_rn(a2[c], q2);       // tap 2 of row r + 1
       a2[c] = __fadd_rn(a1[c], q1);       // tap 1 of row r + 2
-      a1[c] = FMT == kFmtF32 ? __fadd_rn(0.0f, q0) : q0;  // tap 0 of row r + 3 (0.0 + q0)
+      a1[c] = LF == kFmtF32 ? __fadd_rn(0.0f, q0) : q0;  // tap 0 of row r + 3 (0.0 + q0)
     }
     N.v[0] = __shfl_up_sync(0xffffffffu, N.v[4], 1);
     N.v[5] = __shfl_down_sync(0xffffffffu, N.v[1], 1);
@@ -675,6 +689,17 @@ __global__ void k_unorm_table(float* out8, float* out16, float* ref8, float* ref
   }
 }
 
+// The float formats' gray conversion of n pixels (test only): what K1 and the board kernel compute.
+__global__ void k_float_luma(const float* __restrict__ rgb, long long n, int channels, float* __restrict__ luma32f,
+                             uint8_t* __restrict__ luma8) {
+  const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const float* p = rgb + (size_t)channels * i;
+  const float l = rgb32f_luma(p[0], p[1], p[2]);
+  luma32f[i] = l;
+  luma8[i] = (uint8_t)luma32f_to_u8(l);
+}
+
 // ---------------------------------------------------------------------------------------
 // launchers
 // ---------------------------------------------------------------------------------------
@@ -728,6 +753,8 @@ int launch_blur_hessian(const uint8_t* frames, const FrameGeom& g, int n_frames,
       case AG_LA16: AG_STREAM(AG_LA16); break;
       case AG_RGB16: AG_STREAM(AG_RGB16); break;
       case AG_RGBA16: AG_STREAM(AG_RGBA16); break;
+      case AG_RGB32F: AG_STREAM(AG_RGB32F); break;
+      case AG_RGBA32F: AG_STREAM(AG_RGBA32F); break;
       default: AG_STREAM(AG_RGB8); break;
     }
 #undef AG_STREAM
@@ -742,6 +769,8 @@ int launch_blur_hessian(const uint8_t* frames, const FrameGeom& g, int n_frames,
     case AG_LA16: launch_tile<AG_LA16>(frames, g, n_frames, blur, resp, frame_min, write_blur, s); break;
     case AG_RGB16: launch_tile<AG_RGB16>(frames, g, n_frames, blur, resp, frame_min, write_blur, s); break;
     case AG_RGBA16: launch_tile<AG_RGBA16>(frames, g, n_frames, blur, resp, frame_min, write_blur, s); break;
+    case AG_RGB32F: launch_tile<AG_RGB32F>(frames, g, n_frames, blur, resp, frame_min, write_blur, s); break;
+    case AG_RGBA32F: launch_tile<AG_RGBA32F>(frames, g, n_frames, blur, resp, frame_min, write_blur, s); break;
     default: launch_tile<AG_RGB8>(frames, g, n_frames, blur, resp, frame_min, write_blur, s); break;
   }
   return launches + 1;
@@ -796,6 +825,10 @@ int launch_hessian_f32(const float* in, float* out, int w, int h, cudaStream_t s
 }
 int launch_unorm_table(float* out8, float* out16, float* ref8, float* ref16, cudaStream_t s) {
   k_unorm_table<<<256, 256, 0, s>>>(out8, out16, ref8, ref16);
+  return 1;
+}
+int launch_float_luma(const float* rgb, long long n, int channels, float* luma32f, uint8_t* luma8, cudaStream_t s) {
+  k_float_luma<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(rgb, n, channels, luma32f, luma8);
   return 1;
 }
 

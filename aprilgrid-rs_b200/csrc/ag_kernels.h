@@ -41,6 +41,7 @@ int launch_blur_f32(const float* in, float* tmp, float* out, int w, int h, int n
                     const float* d_taps, int radius, cudaStream_t s);
 int launch_hessian_f32(const float* in, float* out, int w, int h, cudaStream_t s);
 int launch_unorm_table(float* out8, float* out16, float* ref8, float* ref16, cudaStream_t s);
+int launch_float_luma(const float* rgb, long long n, int channels, float* luma32f, uint8_t* luma8, cudaStream_t s);
 
 // ag_sparse.cu
 int upload_rochade_tables(const float* cone25, const float* pinv150);

@@ -138,6 +138,8 @@ const AG_RGBA8: c_int = 5;
 const AG_LA16: c_int = 6;
 const AG_RGB16: c_int = 7;
 const AG_RGBA16: c_int = 8;
+const AG_RGB32F: c_int = 9;
+const AG_RGBA32F: c_int = 10;
 const AG_ERR_CAPACITY: c_int = 4;
 const TAG_CAP: usize = 1024; // >= the largest family (587 codes)
 
@@ -189,45 +191,31 @@ fn last_error(h: *const ffi::AgDetector) -> String {
     unsafe { std::ffi::CStr::from_ptr(ffi::ag_last_error(h)).to_string_lossy().into_owned() }
 }
 
-/// Raw pixel view of a DynamicImage.  The eight integer variants (Luma8, LumaA8, Rgb8, Rgba8 and
-/// their 16-bit forms) are passed through untouched and converted on the GPU as `image` 0.25 does.
-/// The float variants (Rgb32F, Rgba32F) have no pixel format of the library: `detect` hands the
-/// reference's own planes, `img.to_luma32f()` and `img.to_luma8()` (src/detector.rs:409, :507), to
-/// `ag_detect_planes`; `detect_batch` and `refined_saddle_points` convert them first with `image`'s
-/// own `to_luma16()`, where the last bits of the float gray image can differ from the reference's.
-enum Pixels<'a> {
-    Borrowed(&'a [u8], c_int, usize),
-    Owned(Vec<u8>, c_int, usize),
-}
-impl<'a> Pixels<'a> {
-    fn parts(&self) -> (&[u8], c_int, usize) {
-        match self {
-            Pixels::Borrowed(b, f, s) => (b, *f, *s),
-            Pixels::Owned(b, f, s) => (b.as_slice(), *f, *s),
-        }
-    }
-}
-
 fn u16_bytes(raw: &[u16]) -> &[u8] {
     unsafe { std::slice::from_raw_parts(raw.as_ptr() as *const u8, raw.len() * 2) }
 }
+fn f32_bytes(raw: &[f32]) -> &[u8] {
+    unsafe { std::slice::from_raw_parts(raw.as_ptr() as *const u8, raw.len() * 4) }
+}
 
-fn pixels_of(img: &DynamicImage) -> (Pixels<'_>, u32, u32) {
+/// Raw pixel view of a DynamicImage: (bytes, pixel format, row stride in bytes, width, height).  All ten
+/// variants are passed through untouched and converted to gray on the GPU as `image` 0.25 does it.
+fn pixels_of(img: &DynamicImage) -> (&[u8], c_int, usize, u32, u32) {
     let (w, h) = (img.width(), img.height());
-    match img {
-        DynamicImage::ImageLuma8(b) => (Pixels::Borrowed(b.as_raw(), AG_L8, w as usize), w, h),
-        DynamicImage::ImageRgb8(b) => (Pixels::Borrowed(b.as_raw(), AG_RGB8, 3 * w as usize), w, h),
-        DynamicImage::ImageLuma16(b) => (Pixels::Borrowed(u16_bytes(b.as_raw()), AG_L16, 2 * w as usize), w, h),
-        DynamicImage::ImageLumaA8(b) => (Pixels::Borrowed(b.as_raw(), AG_LA8, 2 * w as usize), w, h),
-        DynamicImage::ImageRgba8(b) => (Pixels::Borrowed(b.as_raw(), AG_RGBA8, 4 * w as usize), w, h),
-        DynamicImage::ImageLumaA16(b) => (Pixels::Borrowed(u16_bytes(b.as_raw()), AG_LA16, 4 * w as usize), w, h),
-        DynamicImage::ImageRgb16(b) => (Pixels::Borrowed(u16_bytes(b.as_raw()), AG_RGB16, 6 * w as usize), w, h),
-        DynamicImage::ImageRgba16(b) => (Pixels::Borrowed(u16_bytes(b.as_raw()), AG_RGBA16, 8 * w as usize), w, h),
-        other => {  // Rgb32F, Rgba32F
-            let l16 = other.to_luma16();
-            (Pixels::Owned(u16_bytes(l16.as_raw()).to_vec(), AG_L16, 2 * w as usize), w, h)
-        }
-    }
+    let (bytes, fmt, bpp) = match img {
+        DynamicImage::ImageLuma8(b) => (b.as_raw().as_slice(), AG_L8, 1),
+        DynamicImage::ImageRgb8(b) => (b.as_raw().as_slice(), AG_RGB8, 3),
+        DynamicImage::ImageLuma16(b) => (u16_bytes(b.as_raw()), AG_L16, 2),
+        DynamicImage::ImageLumaA8(b) => (b.as_raw().as_slice(), AG_LA8, 2),
+        DynamicImage::ImageRgba8(b) => (b.as_raw().as_slice(), AG_RGBA8, 4),
+        DynamicImage::ImageLumaA16(b) => (u16_bytes(b.as_raw()), AG_LA16, 4),
+        DynamicImage::ImageRgb16(b) => (u16_bytes(b.as_raw()), AG_RGB16, 6),
+        DynamicImage::ImageRgba16(b) => (u16_bytes(b.as_raw()), AG_RGBA16, 8),
+        DynamicImage::ImageRgb32F(b) => (f32_bytes(b.as_raw()), AG_RGB32F, 12),
+        DynamicImage::ImageRgba32F(b) => (f32_bytes(b.as_raw()), AG_RGBA32F, 16),
+        _ => panic!("aprilgrid_b200: unsupported DynamicImage variant"),
+    };
+    (bytes, fmt, bpp * w as usize, w, h)
 }
 
 fn corners(t: &AgTag) -> [(f32, f32); 4] {
@@ -242,13 +230,11 @@ fn maps_of(out: &[AgTag], counts: &[c_int], cap: usize) -> Vec<HashMap<u32, [(f3
 
 /// Pack equally sized images of one pixel format into one pinned buffer.
 fn pack(imgs: &[DynamicImage]) -> (Pinned, u32, u32, c_int, usize) {
-    let (first, w, h) = pixels_of(&imgs[0]);
-    let (_, fmt, stride) = first.parts();
+    let (_, fmt, stride, w, h) = pixels_of(&imgs[0]);
     let frame_bytes = stride * h as usize;
     let mut packed = Pinned::new(frame_bytes * imgs.len());
     for (i, im) in imgs.iter().enumerate() {
-        let (p, ww, hh) = pixels_of(im);
-        let (bytes, f, _) = p.parts();
+        let (bytes, f, _, ww, hh) = pixels_of(im);
         assert!(ww == w && hh == h && f == fmt, "detect_batch: all frames must have the same size and pixel format");
         packed.as_mut_slice()[i * frame_bytes..(i + 1) * frame_bytes].copy_from_slice(&bytes[..frame_bytes]);
     }
@@ -282,10 +268,10 @@ impl TagDetector {
 
     pub fn detect(&self, img: &DynamicImage) -> HashMap<u32, [(f32, f32); 4]> {
         match img {
+            // exact by construction: the reference's own conversions
             DynamicImage::ImageRgb32F(_) | DynamicImage::ImageRgba32F(_) => self.detect_planes(img),
             _ => {
-                let (px, w, h) = pixels_of(img);
-                let (bytes, fmt, stride) = px.parts();
+                let (bytes, fmt, stride, w, h) = pixels_of(img);
                 self.detect_raw(bytes.as_ptr(), w, h, stride, fmt)
             }
         }
@@ -365,8 +351,7 @@ impl TagDetector {
     }
 
     pub fn refined_saddle_points(&self, img: &DynamicImage) -> Vec<Saddle> {
-        let (px, w, h) = pixels_of(img);
-        let (bytes, fmt, stride) = px.parts();
+        let (bytes, fmt, stride, w, h) = pixels_of(img);
         let mut out = vec![AgSaddle::default(); 16384];
         let mut n: c_int = 0;
         let det = self.checkout();

@@ -51,23 +51,34 @@ enum {
   AG_T36H11B1 = 4 /* 1-bit border */
 };
 
-/* ---- pixel formats: the integer DynamicImage variants, channels interleaved ----------
+/* ---- pixel formats: the DynamicImage variants, channels interleaved -------------------
  * Gray conversion as `image` 0.25 does it (to_luma32f for the stencils, to_luma8 for bit
- * sampling): alpha is dropped; colour is the integer sRGB luma (2126 R + 7152 G + 722 B) / 10000,
- * computed and truncated in the source type's width (u8 -> Y8, u16 -> Y16, 32-bit arithmetic);
- * then to_luma32f = Y8 / 255 or Y16 / 65535 (correctly rounded) and to_luma8 = Y8 or
- * (Y16 + 128) / 257.  16-bit words are native endian.  Value 3 is reserved (an internal f32 plane).
- * The 16-bit formats need even row and frame strides everywhere and an even device address
- * on the device entry points (else AG_ERR_INVALID; nothing runs).                          */
+ * sampling); alpha is dropped.
+ * Integer formats: colour is the integer sRGB luma (2126 R + 7152 G + 722 B) / 10000, computed
+ * and truncated in the source type's width (u8 -> Y8, u16 -> Y16, 32-bit arithmetic); then
+ * to_luma32f = Y8 / 255 or Y16 / 65535 (correctly rounded) and to_luma8 = Y8 or (Y16 + 128) / 257.
+ * Float formats: rgb_to_luma runs in f32::Larger = f64.  With r, g, b widened to f64 (the
+ * products are exact) and RN the round-to-nearest-even of each operation, left to right:
+ *   S = RN64(RN64(2126 r + 7152 g) + 722 b),  L = (f32) clamp(RN64(S / 10000), -f32::MAX, f32::MAX)
+ *   to_luma32f = L,  to_luma8 = round_half_away(RN32(clamp(L, 0, 1) * 255))
+ * The clamp is Enlargeable::clamp_from with Bounded::min_value / max_value as its bounds; it
+ * never acts on finite pixels.  Channel values outside [0, 1] are converted like any other;
+ * NaN and infinities are outside this contract (their result is unspecified).
+ * 16-bit words and f32 values are native endian.  Value 3 is reserved (an internal f32 plane).
+ * Row and frame strides must be multiples of a channel word (2 bytes for the 16-bit formats,
+ * 4 for the float ones) everywhere, and so must the address of device frames on the device
+ * entry points (else AG_ERR_INVALID; nothing runs).  Host frames may start at any address.  */
 enum {
-  AG_L8 = 0,     /* ImageLuma8   : 1 byte / px                                   */
-  AG_L16 = 1,    /* ImageLuma16  : 2 bytes / px                                  */
-  AG_RGB8 = 2,   /* ImageRgb8    : 3 bytes / px, R G B (detect_kornia N=3)       */
-  AG_LA8 = 4,    /* ImageLumaA8  : 2 bytes / px, L A                             */
-  AG_RGBA8 = 5,  /* ImageRgba8   : 4 bytes / px, R G B A                         */
-  AG_LA16 = 6,   /* ImageLumaA16 : 4 bytes / px, L A (u16 each)                  */
-  AG_RGB16 = 7,  /* ImageRgb16   : 6 bytes / px, R G B (u16 each)                */
-  AG_RGBA16 = 8  /* ImageRgba16  : 8 bytes / px, R G B A (u16 each)              */
+  AG_L8 = 0,       /* ImageLuma8   : 1 byte / px                                   */
+  AG_L16 = 1,      /* ImageLuma16  : 2 bytes / px                                  */
+  AG_RGB8 = 2,     /* ImageRgb8    : 3 bytes / px, R G B (detect_kornia N=3)       */
+  AG_LA8 = 4,      /* ImageLumaA8  : 2 bytes / px, L A                             */
+  AG_RGBA8 = 5,    /* ImageRgba8   : 4 bytes / px, R G B A                         */
+  AG_LA16 = 6,     /* ImageLumaA16 : 4 bytes / px, L A (u16 each)                  */
+  AG_RGB16 = 7,    /* ImageRgb16   : 6 bytes / px, R G B (u16 each)                */
+  AG_RGBA16 = 8,   /* ImageRgba16  : 8 bytes / px, R G B A (u16 each)              */
+  AG_RGB32F = 9,   /* ImageRgb32F  : 12 bytes / px, R G B (f32 each)               */
+  AG_RGBA32F = 10  /* ImageRgba32F : 16 bytes / px, R G B A (f32 each)             */
 };
 
 /* ---- DetectorParams (src/detector.rs:25-41) -------------------------------------- */
@@ -144,17 +155,16 @@ AG_API int ag_detect(ag_detector* det, const void* pixels, int width, int height
 
 /* TagDetector::detect on a frame given as the TWO gray planes the reference derives from its
  * DynamicImage itself: luma32f = img.to_luma32f() (the stencil chain, src/detector.rs:409) and
- * luma8 = img.to_luma8() (bit sampling, :507).  For the float DynamicImage variants (Rgb32F,
- * Rgba32F), which have no pixel format above, a shim computes both planes with the `image` crate
- * and calls this: the conversion is then the reference's own.  Row strides in bytes
- * (0 = packed).  Synchronous; same result and error conventions as ag_detect.              */
+ * luma8 = img.to_luma8() (bit sampling, :507).  A shim that computes both planes with the `image`
+ * crate and calls this gets the reference's own conversion, whatever the DynamicImage variant.
+ * Row strides in bytes (0 = packed).  Synchronous; same result and error conventions as ag_detect. */
 AG_API int ag_detect_planes(ag_detector* det, const float* luma32f, size_t f32_row_stride,
                             const uint8_t* luma8, size_t u8_row_stride, int width, int height,
                             ag_tag* out, int cap, int* n);
 
 /* detect_batch: n_frames host images of one shape at frames + i*frame_stride.
  * out[i*cap_per_frame ..], n_per_frame[i]; frame_status may be NULL.
- * Strides in bytes (0 = packed); for 16-bit formats both must be even (else AG_ERR_INVALID). */
+ * Strides in bytes (0 = packed), multiples of the format's channel word (else AG_ERR_INVALID). */
 AG_API int ag_detect_batch(ag_detector* det, const void* frames, size_t frame_stride,
                            int n_frames, int width, int height, size_t row_stride, int format,
                            ag_tag* out, int cap_per_frame, int* n_per_frame,
@@ -164,7 +174,7 @@ AG_API int ag_detect_batch(ag_detector* det, const void* frames, size_t frame_st
  * (d_out: n_frames*cap_per_frame ag_tag, d_n_per_frame: n_frames int32,
  *  d_frame_status: n_frames uint32 or NULL).  Work is enqueued on `stream`
  * (a cudaStream_t, NULL = the detector's own stream) and is asynchronous.
- * 16-bit formats must start at an even device address (else AG_ERR_INVALID; nothing runs). */
+ * Frames must start at a multiple of the channel word (else AG_ERR_INVALID; nothing runs). */
 AG_API int ag_detect_batch_device(ag_detector* det, const void* d_frames, size_t frame_stride,
                                   int n_frames, int width, int height, size_t row_stride,
                                   int format, ag_tag* d_out, int cap_per_frame,
@@ -210,7 +220,7 @@ AG_API int ag_gaussian_blur_f32_device(ag_detector* det, const float* d_in, int 
 
 /* Dense front end only (gray -> blur -> Hessian -> min -> threshold mask), device-resident
  * frames, results stay in the detector's workspace.  This is the unit bench.py times for
- * the "blur / threshold kernels alone" configuration.  16-bit formats: even address and strides. */
+ * the "blur / threshold kernels alone" configuration.  Address and strides aligned as above. */
 AG_API int ag_dense_batch_device(ag_detector* det, const void* d_frames, size_t frame_stride,
                                  int n_frames, int width, int height, size_t row_stride,
                                  int format, void* stream);

@@ -7,7 +7,8 @@ limit first: the numbers belong to that card at that limit.
 K1's algorithmic bytes are its input (B/px) plus its two f32 outputs, blur and response (8 B/px); its
 time is the CUDA-event time of stage 0 (K1 and the per-frame min reset) with option "profile" on.
 The copy peak is a device-to-device copy of 4 GB (read + write), larger than L2.  Board frames are
-rendered on the device and widened there: R = G = B = gray, 16-bit words = gray * 257, random alpha."""
+rendered on the device and widened there: R = G = B = gray, 16-bit words = gray * 257, f32 values =
+gray / 255, random alpha.  Every format must find the L8 frames' tags."""
 import argparse
 import os
 import subprocess
@@ -23,12 +24,21 @@ import __graft_entry__ as entry  # noqa: E402
 pkg = entry.load_package()
 FORMATS = [("L8", pkg.FMT_L8, 1, 1), ("L16", pkg.FMT_L16, 1, 2), ("RGB8", pkg.FMT_RGB8, 3, 1),
            ("LA8", pkg.FMT_LA8, 2, 1), ("RGBA8", pkg.FMT_RGBA8, 4, 1), ("LA16", pkg.FMT_LA16, 2, 2),
-           ("RGB16", pkg.FMT_RGB16, 3, 2), ("RGBA16", pkg.FMT_RGBA16, 4, 2)]  # name, code, channels, bytes/channel
+           ("RGB16", pkg.FMT_RGB16, 3, 2), ("RGBA16", pkg.FMT_RGBA16, 4, 2),
+           ("RGB32F", pkg.FMT_RGB32F, 3, 4), ("RGBA32F", pkg.FMT_RGBA32F, 4, 4)]  # name, code, channels, bytes/channel
 CAP = 128
 
 
 def widen(gray, channels, width):
     """N x H x W u8 gray -> N x H x (W * channels * width) bytes of the interleaved format."""
+    if width == 4:  # f32: gray / 255, alpha random in [0, 1]
+        g = gray.to(torch.float32) / 255.0
+        chans = [g] * 3
+        if channels == 4:
+            chans.append(torch.rand(gray.shape, device=gray.device,
+                                    generator=torch.Generator(device=gray.device).manual_seed(1)))
+        px = torch.stack(chans, dim=-1).contiguous()
+        return px.view(torch.uint8).reshape(gray.shape[0], gray.shape[1], -1).contiguous()
     g = gray.to(torch.int32) * (257 if width == 2 else 1)
     n_col = 1 if channels <= 2 else 3
     chans = [g] * n_col
