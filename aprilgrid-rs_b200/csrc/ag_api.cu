@@ -41,14 +41,12 @@ bool family_info(int family, FamilyInfo* f) {  // src/detector.rs:369-405
 // creation errors have no handle to live in: one message per calling thread
 thread_local std::string g_create_error;
 
-// Pipeline slots.  The device-batch path keeps up to kSlots chunks in flight: the dense + sparse
-// front end of chunk i+1 runs on the caller's stream while the latency-bound board searches of
-// chunks i, i-1, ... run on their slots' own streams, side by side.
-constexpr int kSlots = 2;
-// Device-batch path: the dense buffers of ONE slot are reused chunk after chunk (K1-K4 of
-// consecutive chunks are serial on the caller's stream anyway); only the light board-search side
-// is multi-buffered, so the board searches of up to kBoardSlots chunks overlap each other and
-// the front end of later chunks, which hides the long tail of the slowest frames of a chunk.
+// Pipeline.  The dense + sparse front end (K1-K4) of chunk i+1 runs on one stream while the
+// latency-bound board searches of chunks i, i-1, ... run on their board slots' own streams, side
+// by side.  The dense buffers of ONE slot are reused chunk after chunk (K1-K4 of consecutive
+// chunks are serial on that stream anyway); only the light board-search side is multi-buffered,
+// so the board searches of up to kBoardSlots chunks overlap each other and the front end of later
+// chunks, which hides the long tail of the slowest frames of a chunk.
 constexpr int kBoardSlots = 8;
 #ifndef AG_BIG_TIER_WARPS
 #define AG_BIG_TIER_WARPS 2
@@ -79,8 +77,9 @@ struct BoardSlot {
   BoardWsLayout layout[4]{};        // sized for the largest warps-per-frame (allocation)
   BoardWsLayout layout_batch[4]{};  // layout used when many frames are in flight
   BoardWsLayout layout_split0{};    // ... by the first launch of a split batch: frames of at most 320 saddles only
-  // host-frame path (ag_detect_batch): staged input of the chunk (K6 samples the tag bits from it,
-  // so it lives as long as the slot's board search), device results and pinned result staging
+  // host-frame path (ag_detect_batch) and the one-frame slot: staged input of the chunk (K6
+  // samples the tag bits from it, so it lives as long as the slot's board search), device results
+  // and pinned result staging
   uint8_t* d_in = nullptr;
   size_t cap_in_bytes = 0;
   uint8_t* h_in = nullptr;  // pinned staging for frames that arrive in pageable host memory
@@ -94,26 +93,20 @@ struct BoardSlot {
   cudaEvent_t ev_up = nullptr, ev_done = nullptr;  // upload done / results on the host
 };
 
-// Device buffers of one pipeline slot (one chunk in flight).
+// Dense and sparse buffers of one chunk (K1-K4).
 struct Slot {
   cudaStream_t stream = nullptr;
   cudaEvent_t done = nullptr;
-  BoardSlot bb;  // the slot's own board-search side (host path, taps)
+  BoardSlot bb;  // the slot's own board-search side and host staging (one-frame slot only)
   int cap_frames = 0;
-  size_t cap_px = 0, cap_words = 0, cap_in_bytes = 0;
-  int cap_clusters = 0, cap_saddles = 0, cap_tags = 0;
-  uint8_t* d_in = nullptr;
+  size_t cap_px = 0, cap_words = 0;
+  int cap_clusters = 0, cap_saddles = 0;
   float *d_blur = nullptr, *d_resp = nullptr;
-  uint32_t *d_min = nullptr, *d_mask = nullptr, *d_status = nullptr;
-  int *d_parent = nullptr, *d_acc = nullptr, *d_ncl = nullptr, *d_ntags = nullptr;
+  uint32_t *d_min = nullptr, *d_mask = nullptr;
+  int *d_parent = nullptr, *d_acc = nullptr, *d_ncl = nullptr;
   float2* d_centers = nullptr;
   ag_saddle* d_raw = nullptr;
   uint8_t* d_raw_valid = nullptr;
-  ag_tag* d_tags = nullptr;
-  // pinned result staging
-  ag_tag* h_tags = nullptr;
-  int* h_ntags = nullptr;
-  uint32_t* h_status = nullptr;
   // taps
   int* d_label_fallback = nullptr;  // K3: frames the run-based kernel handed to the pixel-list kernel
   uint32_t* d_pixlist = nullptr;   // K3: compact list of mask pixels / runs, [frames][pix_cap]
@@ -129,14 +122,11 @@ struct ag_detector {
   ag_params params{};
   std::mutex mu;
   std::string err;
-  Slot slot[kSlots];
+  Slot dense;  // dense + sparse buffers of the batch pipelines
   Slot big;  // one-frame slot with grown capacities: frames that overflowed max_clusters / max_saddles are re-run here
   BoardSlot bslot[kBoardSlots];
   int slot_rr = 0;            // next board slot of the device-batch pipeline (rotates across calls)
   cudaStream_t up_stream = nullptr;  // host-frame path: uploads, ahead of the kernels
-  long dense_streams = 1;   // device-batch path: 2 = alternate chunks between two dense streams / buffer sets (measured: no gain)
-  int dense_rr = 0;
-  cudaEvent_t ev_call = nullptr;
   // host-buffer path: chunks whose results still sit in a board slot's pinned staging, with the
   // output arrays of the ag_detect_batch call they belong to (calls may overlap: "host_async")
   struct HostPend {
@@ -153,7 +143,7 @@ struct ag_detector {
   bool host_async = false;      // ag_detect_batch returns without collecting its results
   bool host_truncated = false;  // a collected frame had more tags than its call's cap_per_frame
   bool host_unresolved = false;  // a collected frame overflowed a capacity that could not be grown
-  bool device_path_busy = false;  // device-batch work may still be in flight on slot 0 / the board slots
+  bool device_path_busy = false;  // device-batch work may still be in flight on the dense slot / the board slots
   bool device_async = false;  // ag_detect_batch_device returns without ordering the results on the
                               // caller's stream; ag_detect_batch_device_wait does that
   uint64_t launches = 0;
@@ -179,7 +169,6 @@ struct ag_detector {
   long board_batch_frames = 148;  // automatic mode: launches with at least this many frames use 2 warps per frame
   long label_variant = 0;  // K3: 0 = run-based in shared memory, 1 = pixel list with per-pixel parents
   long board_saddle_tier = -1;  // -1 automatic, 0 = 512, 1 = 1024, 2 = 4096 saddles on chip in the board kernel
-  bool label_list = true;  // K3 over a compact pixel list (0 = word-oriented version only)
   bool board_timing = false;  // per-frame timing taps of the board kernel (ag_test_board_times)
   bool board_fast = true;  // four-lane group scoring of candidate boards (0 = general path only)
   long board_priority = 0;  // priority of the board-search streams: 0 = least (= default streams), 1 = greatest
@@ -210,8 +199,8 @@ namespace {
     }                                                                                        \
   } while (0)
 
-// Host-buffer entry points and taps share slot 0 with the device-batch pipeline: wait until the
-// latter has drained before touching the buffers.
+// Host-buffer entry points and the standalone operators share the dense slot with the device-batch
+// pipeline: wait until the latter has drained before touching the buffers.
 int quiesce_device_path(ag_detector* det, bool host_too = true);
 
 int fail(ag_detector* det, int code, const char* msg) {
@@ -245,6 +234,11 @@ int make_geom(ag_detector* det, int w, int h, size_t row_stride, size_t frame_st
   g->frame_stride = frame_stride;
   g->format = format;
   return AG_OK;
+}
+
+// Bytes from a frame's first pixel to its last: the padding after the last row is not the frame's.
+size_t frame_bytes(const FrameGeom& g) {
+  return g.row_stride * (size_t)(g.h - 1) + (size_t)g.w * bytes_per_px(g.format);
 }
 
 // Per-frame capacities in force for a call: the options when set, else sized from the image area
@@ -380,16 +374,19 @@ void free_board_slot(BoardSlot& B) {
   B = BoardSlot();
 }
 
-// Make sure a slot can hold `frames` frames of geometry g with `cap_tags` tags per frame.
-// `own_board` = the slot's own board-search side is needed too (host path, taps).
-int ensure_slot(ag_detector* det, Slot& S, const FrameGeom& g, int frames, int cap_tags,
-                bool need_input, bool own_board = true, bool need_parent = false) {
+// Make sure a slot can hold `frames` frames of geometry g.  `own_board` = the slot's own
+// board-search side is needed too, with host staging for `frames` frames of g.frame_stride bytes
+// and every tag of the family per frame (the one-frame slot).
+int ensure_slot(ag_detector* det, Slot& S, const FrameGeom& g, int frames, bool own_board = true,
+                bool need_parent = false) {
   int rc;
   if (!S.stream) {
     AG_CUDA(det, cudaStreamCreateWithFlags(&S.stream, cudaStreamNonBlocking));
     AG_CUDA(det, cudaEventCreateWithFlags(&S.done, cudaEventDisableTiming));
   }
-  if (own_board && (rc = ensure_board_slot(det, S.bb, frames, true))) return rc;
+  if (own_board && ((rc = ensure_board_slot(det, S.bb, frames, true)) ||
+                    (rc = ensure_host_stage(det, S.bb, (size_t)frames * g.frame_stride, frames, det->fam.n_codes))))
+    return rc;
   const bool grow_frames = frames > S.cap_frames;
   const int F = std::max(frames, S.cap_frames);
   const size_t px = std::max((size_t)g.n_px, S.cap_px);
@@ -414,54 +411,28 @@ int ensure_slot(ag_detector* det, Slot& S, const FrameGeom& g, int frames, int c
   if (grow_frames || ncl != S.cap_clusters || nsd != S.cap_saddles) {
     AG_CUDA(det, cudaStreamSynchronize(S.stream));
     if ((rc = regrow(det, &S.d_min, (size_t)F))) return rc;
-    if ((rc = regrow(det, &S.d_status, (size_t)F))) return rc;
     if ((rc = regrow(det, &S.d_ncl, (size_t)F))) return rc;
-    if ((rc = regrow(det, &S.d_ntags, (size_t)F))) return rc;
     if ((rc = regrow(det, &S.d_label_fallback, (size_t)F))) return rc;
     if ((rc = regrow(det, &S.d_acc, (size_t)F * ncl * 3))) return rc;
     if ((rc = regrow(det, &S.d_centers, (size_t)F * ncl))) return rc;
     if ((rc = regrow(det, &S.d_raw, (size_t)F * ncl))) return rc;
     if ((rc = regrow(det, &S.d_raw_valid, (size_t)F * ncl))) return rc;
-    if (S.h_ntags) cudaFreeHost(S.h_ntags);
-    if (S.h_status) cudaFreeHost(S.h_status);
-    AG_CUDA(det, cudaMallocHost((void**)&S.h_ntags, sizeof(int) * F));
-    AG_CUDA(det, cudaMallocHost((void**)&S.h_status, sizeof(uint32_t) * F));
     S.cap_clusters = ncl;
     S.cap_saddles = nsd;
-  }
-  if (grow_frames || cap_tags > S.cap_tags) {
-    AG_CUDA(det, cudaStreamSynchronize(S.stream));
-    const int ct = std::max(cap_tags, S.cap_tags);
-    if ((rc = regrow(det, &S.d_tags, (size_t)F * ct))) return rc;
-    if (S.h_tags) cudaFreeHost(S.h_tags);
-    AG_CUDA(det, cudaMallocHost((void**)&S.h_tags, sizeof(ag_tag) * (size_t)F * ct));
-    S.cap_tags = ct;
   }
   if (need_parent && !S.d_parent) {
     AG_CUDA(det, cudaStreamSynchronize(S.stream));
     if ((rc = regrow(det, &S.d_parent, (size_t)F * px))) return rc;
-  }
-  if (need_input) {
-    const size_t in_bytes = (size_t)F * g.frame_stride;
-    if (in_bytes > S.cap_in_bytes) {
-      AG_CUDA(det, cudaStreamSynchronize(S.stream));
-      if ((rc = regrow(det, &S.d_in, in_bytes))) return rc;
-      S.cap_in_bytes = in_bytes;
-    }
   }
   S.cap_frames = F;
   return AG_OK;
 }
 
 void free_slot(Slot& S) {
-  cudaFree(S.d_in); cudaFree(S.d_blur); cudaFree(S.d_resp); cudaFree(S.d_min); cudaFree(S.d_mask);
-  cudaFree(S.d_status); cudaFree(S.d_parent); cudaFree(S.d_acc); cudaFree(S.d_ncl);
-  cudaFree(S.d_ntags); cudaFree(S.d_centers); cudaFree(S.d_raw);
-  cudaFree(S.d_raw_valid); cudaFree(S.d_tags); cudaFree(S.d_pixlist); cudaFree(S.d_label_fallback);
+  cudaFree(S.d_blur); cudaFree(S.d_resp); cudaFree(S.d_min); cudaFree(S.d_mask);
+  cudaFree(S.d_parent); cudaFree(S.d_acc); cudaFree(S.d_ncl); cudaFree(S.d_centers); cudaFree(S.d_raw);
+  cudaFree(S.d_raw_valid); cudaFree(S.d_pixlist); cudaFree(S.d_label_fallback);
   free_board_slot(S.bb);
-  if (S.h_tags) cudaFreeHost(S.h_tags);
-  if (S.h_ntags) cudaFreeHost(S.h_ntags);
-  if (S.h_status) cudaFreeHost(S.h_status);
   if (S.done) cudaEventDestroy(S.done);
   if (S.stream) cudaStreamDestroy(S.stream);
   S = Slot();
@@ -560,8 +531,7 @@ int run_sparse(ag_detector* det, Slot& S, BoardSlot& B, const FrameGeom& g, int 
   // buffer as scratch (K2 has consumed it; nothing downstream reads it)
   int* parent = S.d_parent ? S.d_parent : reinterpret_cast<int*>(S.d_resp);
   det->launches += launch_label_clusters(S.d_mask, g, n, parent, S.cap_clusters, S.d_acc,
-                                         S.d_centers, S.d_ncl, d_status,
-                                         det->label_list ? S.d_pixlist : nullptr, S.pix_cap, variant,
+                                         S.d_centers, S.d_ncl, d_status, S.d_pixlist, S.pix_cap, variant,
                                          S.d_label_fallback, s);
   prof_mark(det, 2, s);
   det->launches += launch_refine_filter(S.d_blur, g, n, S.d_centers, S.d_ncl, S.cap_clusters, S.d_raw,
@@ -615,24 +585,81 @@ int run_boards(ag_detector* det, BoardSlot& S, const uint8_t* d_frames, const Fr
   return AG_OK;
 }
 
-int run_chunk(ag_detector* det, Slot& S, const uint8_t* d_frames, const FrameGeom& g, int n,
-              ag_tag* d_tags, int cap, int* d_ntags, uint32_t* d_status, bool taps,
-              cudaStream_t s) {
-  int rc;
-  if ((rc = run_dense(det, S, d_frames, g, n, true, s))) return rc;
-  // taps: the labels tap reads the per-pixel parent array, which only the pixel-list kernel writes;
-  // run it first, then the regular (run-based) labelling, whose centres the pipeline continues with
-  if (taps && det->label_variant == 0 && (rc = run_sparse(det, S, S.bb, g, n, d_status, s, true))) return rc;
-  if ((rc = run_sparse(det, S, S.bb, g, n, d_status, s))) return rc;
-  return run_boards(det, S.bb, d_frames, g, n, d_tags, cap, d_ntags, d_status, taps, s);
+constexpr uint32_t kGrowable = AG_FRAME_CLUSTER_OVERFLOW | AG_FRAME_SADDLE_OVERFLOW;
+
+// What run_one_frame runs after K1-K4: K6, nothing (the refined saddles are the result), or K6
+// keeping every intermediate for the stage taps.
+enum class FrameRun { kTags, kSaddles, kTaps };
+
+// One frame through the pipeline on the detector's one-frame slot (det->big), synchronously.  The
+// slot has its own stream and buffers, so chunks of streaming calls may be in flight meanwhile.
+// upload(d_in, stream) enqueues the copy of the frame into the slot's staged input; K1-K4 read it
+// as geometry g, K6 samples the tag bits from geometry gb at d_in + bits_offset.
+// A frame that overflows max_clusters / max_saddles is run again with what it overflowed grown
+// (clusters x16 up to 2^22, saddles to 16384; the reference has no limits) until it fits or the
+// capacities are at those limits.  first_status != 0 (the frame overflowed in a batch chunk) grows
+// them before the first run; if none can grow, that status and 0 results come back without a run.
+// The stage taps run once, at the call's capacities.
+// Out: *count = tags found (refined saddles for kSaddles) and *status = the frame's status bits;
+// the tags are in big.bb.h_tags, the refined saddles in big.bb.d_refined.
+template <typename Upload>
+int run_one_frame(ag_detector* det, const FrameGeom& g, const FrameGeom& gb, size_t bits_offset, Upload upload,
+                  FrameRun what, uint32_t first_status, int* count, uint32_t* status) {
+  struct RestoreCaps {  // the call's capacities come back on every exit
+    ag_detector* det;
+    int clusters, saddles;
+    ~RestoreCaps() {
+      det->cur_clusters = clusters;
+      det->cur_saddles = saddles;
+    }
+  } restore{det, det->cur_clusters, det->cur_saddles};
+  det->tap_valid = false;  // the taps read the buffers about to be overwritten
+  Slot& S = det->big;
+  BoardSlot& B = S.bb;
+  const bool taps = what == FrameRun::kTaps;
+  uint32_t st = first_status;
+  int cnt = 0, rc;
+  for (bool ran = false;; ran = true) {
+    if (ran || st) {
+      bool grew = false;
+      if ((st & AG_FRAME_CLUSTER_OVERFLOW) && det->cur_clusters < (1 << 22)) {
+        det->cur_clusters = (int)std::min<long>((long)det->cur_clusters * 16, 1l << 22);
+        grew = true;
+      }
+      if ((st & AG_FRAME_SADDLE_OVERFLOW) && det->cur_saddles < 16384) {
+        det->cur_saddles = 16384;
+        grew = true;
+      }
+      if (taps || !grew) break;
+    }
+    if ((rc = ensure_slot(det, S, g, 1, true, taps))) return rc;
+    const cudaStream_t s = S.stream;
+    AG_CUDA(det, upload(B.d_in, s));
+    if ((rc = run_dense(det, S, B.d_in, g, 1, true, s))) return rc;
+    // taps: the labels tap reads the per-pixel parent array, which only the pixel-list kernel writes;
+    // run it first, then the regular (run-based) labelling, whose centres the pipeline continues with
+    if (taps && det->label_variant == 0 && (rc = run_sparse(det, S, B, g, 1, B.d_status, s, true))) return rc;
+    if ((rc = run_sparse(det, S, B, g, 1, B.d_status, s))) return rc;
+    if (what == FrameRun::kSaddles) {
+      AG_CUDA(det, cudaMemcpyAsync(B.h_ntags, B.d_nref, sizeof(int), cudaMemcpyDeviceToHost, s));
+    } else {  // (K6 reports 0 tags for a frame whose saddle list K3 / K4 flagged as truncated)
+      if ((rc = run_boards(det, B, B.d_in + bits_offset, gb, 1, B.d_tags, B.hs_tags, B.d_ntags, B.d_status, taps, s)))
+        return rc;
+      AG_CUDA(det, cudaMemcpyAsync(B.h_ntags, B.d_ntags, sizeof(int), cudaMemcpyDeviceToHost, s));
+      AG_CUDA(det, cudaMemcpyAsync(B.h_tags, B.d_tags, sizeof(ag_tag) * B.hs_tags, cudaMemcpyDeviceToHost, s));
+    }
+    AG_CUDA(det, cudaMemcpyAsync(B.h_status, B.d_status, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    AG_CUDA(det, cudaStreamSynchronize(s));
+    cnt = B.h_ntags[0];
+    st = B.h_status[0];
+  }
+  *count = cnt;
+  *status = st;
+  return AG_OK;
 }
 
 void copy_out_b(const BoardSlot& B, int n, int cap, ag_tag* out, int* n_per_frame, uint32_t* frame_status,
                 int frame0, bool* truncated);
-int rerun_frame_grown(ag_detector* det, const uint8_t* host_px, const FrameGeom& g, uint32_t first_status,
-                      ag_tag* out, int cap, int* n_out, uint32_t* status_out);
-
-constexpr uint32_t kGrowable = AG_FRAME_CLUSTER_OVERFLOW | AG_FRAME_SADDLE_OVERFLOW;
 
 // Host-buffer path: wait for the chunk staged in board slot bi and hand its results to the output
 // arrays of the call that submitted it.  A frame that overflowed max_clusters / max_saddles was
@@ -649,14 +676,25 @@ int collect_host_slot(ag_detector* det, int bi) {
   for (int i = 0; i < P.n; ++i) {
     const uint32_t st = B.h_status[i];
     if (st & kGrowable) {
+      FrameGeom g = P.g;
+      g.frame_stride = g.row_stride * (size_t)g.h;
+      const uint8_t* src = P.src + (size_t)i * P.g.frame_stride;
+      auto upload = [&](uint8_t* d_in, cudaStream_t s) {
+        return cudaMemcpyAsync(d_in, src, frame_bytes(g), cudaMemcpyHostToDevice, s);
+      };
       int cnt = 0;
       uint32_t st2 = 0;
-      int rc = rerun_frame_grown(det, P.src + (size_t)i * P.g.frame_stride, P.g, st,
-                                 P.out + (size_t)(P.f0 + i) * P.cap, P.cap, &cnt, &st2);
+      int rc = run_one_frame(det, g, g, 0, upload, FrameRun::kTags, st, &cnt, &st2);
       if (rc) return rc;
+      const BoardSlot& R = det->big.bb;
+      memcpy(P.out + (size_t)(P.f0 + i) * P.cap, R.h_tags,
+             sizeof(ag_tag) * (size_t)std::min(std::min(cnt, P.cap), R.hs_tags));
+      if (cnt > P.cap) {
+        st2 |= AG_FRAME_TAG_OVERFLOW;
+        det->host_truncated = true;
+      }
       P.n_per_frame[P.f0 + i] = cnt;
       if (P.status) P.status[P.f0 + i] = st2;
-      if (cnt > P.cap) det->host_truncated = true;
       if (st2 & (kGrowable | AG_FRAME_BOARD_OVERFLOW)) det->host_unresolved = true;
     } else if (st & AG_FRAME_BOARD_OVERFLOW) {
       det->host_unresolved = true;
@@ -682,9 +720,7 @@ int quiesce_device_path(ag_detector* det, bool host_too) {
     if (rc) return rc;
   }
   if (!det->device_path_busy) return AG_OK;
-  for (auto& D : det->slot)
-    if (D.done) AG_CUDA(det, cudaEventSynchronize(D.done));
-  det->dense_rr = 0;
+  if (det->dense.done) AG_CUDA(det, cudaEventSynchronize(det->dense.done));
   for (auto& B : det->bslot)
     if (B.pending) {
       AG_CUDA(det, cudaEventSynchronize(B.ev_boards));
@@ -740,61 +776,6 @@ void copy_out_b(const BoardSlot& B, int n, int cap, ag_tag* out, int* n_per_fram
     memcpy(out + (size_t)(frame0 + i) * cap, B.h_tags + (size_t)i * B.hs_tags, sizeof(ag_tag) * m);
     if (frame_status) frame_status[frame0 + i] = B.h_status[i];
   }
-}
-
-// One frame through the whole pipeline on the detector's one-frame slot, with the capacities the
-// frame overflowed grown until it fits (clusters x16 up to 2^22, saddles up to 16384).  Synchronous;
-// uses its own stream and buffers, so chunks of streaming calls may be in flight meanwhile.
-int rerun_frame_grown(ag_detector* det, const uint8_t* host_px, const FrameGeom& g_in, uint32_t first_status,
-                      ag_tag* out, int cap, int* n_out, uint32_t* status_out) {
-  FrameGeom g = g_in;
-  g.frame_stride = g.row_stride * (size_t)g.h;
-  const int save_cl = det->cur_clusters, save_sd = det->cur_saddles;
-  int ncl = save_cl, nsd = save_sd, rc = AG_OK;
-  uint32_t st = first_status;
-  Slot& S = det->big;
-  for (;;) {
-    bool grew = false;
-    if ((st & AG_FRAME_CLUSTER_OVERFLOW) && ncl < (1 << 22)) { ncl = (int)std::min<long>((long)ncl * 16, 1l << 22); grew = true; }
-    if ((st & AG_FRAME_SADDLE_OVERFLOW) && nsd < 16384) { nsd = 16384; grew = true; }
-    if (!grew) break;  // already at the limits: the flags stay set and the caller reports them
-    det->cur_clusters = ncl;
-    det->cur_saddles = nsd;
-    if (!(rc = ensure_slot(det, S, g, 1, det->fam.n_codes, true))) {
-      const size_t bytes = g.row_stride * (size_t)(g.h - 1) + (size_t)g.w * bytes_per_px(g.format);
-      cudaStream_t s = S.stream;
-      // front end first: the board search only runs once the frame fits
-      if (cudaMemcpyAsync(S.d_in, host_px, bytes, cudaMemcpyHostToDevice, s) != cudaSuccess) rc = AG_ERR_CUDA;
-      if (!rc) rc = run_dense(det, S, S.d_in, g, 1, true, s);
-      if (!rc) rc = run_sparse(det, S, S.bb, g, 1, S.d_status, s);
-      if (!rc && (cudaMemcpyAsync(S.h_status, S.d_status, sizeof(uint32_t), cudaMemcpyDeviceToHost, s) != cudaSuccess ||
-                  cudaStreamSynchronize(s) != cudaSuccess))
-        rc = AG_ERR_CUDA;
-      if (!rc && !(S.h_status[0] & kGrowable)) {
-        rc = run_boards(det, S.bb, S.d_in, g, 1, S.d_tags, S.cap_tags, S.d_ntags, S.d_status, false, s);
-        if (!rc && (cudaMemcpyAsync(S.h_ntags, S.d_ntags, sizeof(int), cudaMemcpyDeviceToHost, s) != cudaSuccess ||
-                    cudaMemcpyAsync(S.h_status, S.d_status, sizeof(uint32_t), cudaMemcpyDeviceToHost, s) != cudaSuccess ||
-                    cudaMemcpyAsync(S.h_tags, S.d_tags, sizeof(ag_tag) * (size_t)S.cap_tags, cudaMemcpyDeviceToHost, s) !=
-                        cudaSuccess ||
-                    cudaStreamSynchronize(s) != cudaSuccess))
-          rc = AG_ERR_CUDA;
-      } else if (!rc) {
-        S.h_ntags[0] = 0;  // still too large: no board search on a truncated saddle list
-      }
-      if (rc == AG_ERR_CUDA && det->err.empty()) det->err = "re-run of an overflowed frame failed";
-    }
-    det->cur_clusters = save_cl;
-    det->cur_saddles = save_sd;
-    if (rc) return rc;
-    st = S.h_status[0];
-    const int cnt = S.h_ntags[0];
-    *n_out = cnt;
-    memcpy(out, S.h_tags, sizeof(ag_tag) * (size_t)std::min(std::min(cnt, cap), S.cap_tags));
-    if (cnt > cap) st |= AG_FRAME_TAG_OVERFLOW;
-    if (!(st & kGrowable)) break;
-  }
-  *status_out = st;
-  return AG_OK;
 }
 
 // What a synchronous host call / a wait reports after its chunks were collected.
@@ -907,11 +888,10 @@ void ag_destroy(ag_detector* det) {
   if (!det) return;
   cudaSetDevice(det->device);
   cudaDeviceSynchronize();
-  for (auto& S : det->slot) free_slot(S);
+  free_slot(det->dense);
   free_slot(det->big);
   for (auto& B : det->bslot) free_board_slot(B);
   if (det->up_stream) cudaStreamDestroy(det->up_stream);
-  if (det->ev_call) cudaEventDestroy(det->ev_call);
   for (auto e : det->ev_pool) cudaEventDestroy(e);
   cudaFree(det->d_codes);
   cudaFree(det->d_f32_a); cudaFree(det->d_f32_b); cudaFree(det->d_f32_c); cudaFree(det->d_taps);
@@ -954,9 +934,6 @@ int ag_set_option(ag_detector* det, const char* key, long value) {
   } else if (!strcmp(key, "board_batch_frames")) {
     if (value < 1) return fail(det, AG_ERR_INVALID, "board_batch_frames must be positive");
     det->board_batch_frames = value;
-  } else if (!strcmp(key, "dense_streams")) {
-    if (value < 1 || value > 2) return fail(det, AG_ERR_INVALID, "dense_streams must be 1 or 2");
-    det->dense_streams = value;
 #ifdef AG_EXPERIMENTS  // occupancy experiments only (tools/build_variant.sh); not in the shipped library
   } else if (!strcmp(key, "board_smem_pad")) {
     ag::g_board_smem_pad = (int)value;
@@ -967,8 +944,6 @@ int ag_set_option(ag_detector* det, const char* key, long value) {
   } else if (!strcmp(key, "board_saddle_tier")) {
     if (value < -1 || value > 2) return fail(det, AG_ERR_INVALID, "board_saddle_tier must be -1, 0 (512), 1 (1024) or 2 (4096)");
     det->board_saddle_tier = value;
-  } else if (!strcmp(key, "label_list")) {
-    det->label_list = value != 0;
   } else if (!strcmp(key, "board_timing")) {
     det->board_timing = value != 0;
   } else if (!strcmp(key, "board_fast")) {
@@ -1034,35 +1009,22 @@ int ag_detect_batch_device(ag_detector* det, const void* d_frames, size_t frame_
   if ((rc = collect_host(det, det->host_seq))) return rc;
   set_caps(det, g);
   const int chunk = chunk_limit(det, g, std::min<long>(det->chunk_frames, std::max(n_frames, 1)));
-  // One set of dense buffers (slot 0: K1-K4 of consecutive chunks are serial on stream s anyway),
+  // One set of dense buffers (K1-K4 of consecutive chunks are serial on stream s anyway),
   // kBoardSlots board-search sides: chunk i's K6 runs on its board slot's own stream, so the
   // searches of up to kBoardSlots chunks (of this call and of earlier calls) overlap each other
   // and the front end of the following chunks.  A board slot is reused only after its kernel has
   // finished (K4 of the new chunk writes the slot's saddle list).
-  // With dense_streams = 2 a second set of dense buffers and a second (internal) stream take every
-  // other chunk, so the latency-bound K3 / K4 of one chunk overlap the issue-bound K1 of the next.
-  const int n_dense = det->dense_streams >= 2 ? 2 : 1;
-  for (int i = 0; i < n_dense; ++i)
-    if ((rc = ensure_slot(det, det->slot[i], g, chunk, 1, false, false))) return rc;
-  cudaStream_t s0 = stream ? (cudaStream_t)stream : det->slot[0].stream;
-  cudaStream_t s1 = det->slot[n_dense - 1].stream;
+  Slot& D = det->dense;
+  if ((rc = ensure_slot(det, D, g, chunk, false))) return rc;
+  cudaStream_t s = stream ? (cudaStream_t)stream : D.stream;
   // all board slots are sized up front: an allocation (which synchronises the device) must not
   // happen in the middle of a streaming sequence of calls
   for (auto& B : det->bslot)
     if ((rc = ensure_board_slot(det, B, chunk, false))) return rc;
   // the dense buffers are shared by every device-batch call: order this call after the front end
   // of the previous one even if the caller switched streams
-  if (det->device_path_busy) AG_CUDA(det, cudaStreamWaitEvent(s0, det->slot[0].done, 0));
-  if (n_dense == 2) {  // the internal stream starts after the caller's earlier work (the frames)
-    if (!det->ev_call) AG_CUDA(det, cudaEventCreateWithFlags(&det->ev_call, cudaEventDisableTiming));
-    AG_CUDA(det, cudaEventRecord(det->ev_call, s0));
-    AG_CUDA(det, cudaStreamWaitEvent(s1, det->ev_call, 0));
-  }
+  if (det->device_path_busy) AG_CUDA(det, cudaStreamWaitEvent(s, D.done, 0));
   for (int f0 = 0; f0 < n_frames; f0 += chunk) {
-    const int which = n_dense == 2 ? det->dense_rr : 0;
-    if (n_dense == 2) det->dense_rr ^= 1;
-    Slot& D = det->slot[which];
-    cudaStream_t s = which ? s1 : s0;
     BoardSlot& B = det->bslot[det->slot_rr];
     det->slot_rr = (det->slot_rr + 1) % kBoardSlots;
     if ((rc = ensure_board_slot(det, B, chunk, false))) return rc;
@@ -1080,15 +1042,13 @@ int ag_detect_batch_device(ag_detector* det, const void* d_frames, size_t frame_
     AG_CUDA(det, cudaEventRecord(B.ev_boards, B.bstream));
     B.pending = true;
   }
-  AG_CUDA(det, cudaEventRecord(det->slot[0].done, s0));
-  if (n_dense == 2) AG_CUDA(det, cudaEventRecord(det->slot[1].done, s1));
+  AG_CUDA(det, cudaEventRecord(D.done, s));
   det->device_path_busy = true;
   // results become visible in the caller's stream order (unless the caller asked to do that
-  // itself with ag_detect_batch_device_wait, which lets consecutive calls overlap); every chunk's
-  // board kernel follows its front end, so waiting for the board kernels covers both dense streams
+  // itself with ag_detect_batch_device_wait, which lets consecutive calls overlap)
   if (!det->device_async)
     for (auto& B : det->bslot)
-      if (B.pending) AG_CUDA(det, cudaStreamWaitEvent(s0, B.ev_boards, 0));
+      if (B.pending) AG_CUDA(det, cudaStreamWaitEvent(s, B.ev_boards, 0));
   return AG_OK;
 }
 
@@ -1116,17 +1076,17 @@ int ag_dense_batch_device(ag_detector* det, const void* d_frames, size_t frame_s
   if (rc) return rc;
   if ((uintptr_t)d_frames % channel_align(format))
     return fail(det, AG_ERR_INVALID, "device frames must start at a multiple of the format's channel word");
-  Slot& S = det->slot[0];
+  Slot& S = det->dense;
   set_caps(det, g);
   const int chunk = chunk_limit(det, g, std::min<long>(det->chunk_frames, std::max(n_frames, 1)));
-  if ((rc = ensure_slot(det, S, g, chunk, 1, false, false))) return rc;
+  if ((rc = ensure_slot(det, S, g, chunk, false))) return rc;
   cudaStream_t s = stream ? (cudaStream_t)stream : S.stream;
   for (int f0 = 0; f0 < n_frames; f0 += chunk) {
     const int n = std::min(chunk, n_frames - f0);
     const uint8_t* in = (const uint8_t*)d_frames + (size_t)f0 * g.frame_stride;
     if ((rc = run_dense(det, S, in, g, n, true, s))) return rc;
   }
-  // later calls on this handle (any stream) order themselves after this one through slot 0's event
+  // later calls on this handle (any stream) order themselves after this one through the dense slot's event
   AG_CUDA(det, cudaEventRecord(S.done, s));
   det->device_path_busy = true;
   return AG_OK;
@@ -1158,8 +1118,8 @@ static int detect_batch_host(ag_detector* det, const void* frames, size_t frame_
   // input of a chunk stays in its board slot until K6 (which samples the tag bits) is done.
   const int chunk = chunk_limit(
       det, g, std::min<long>(std::min<long>(det->chunk_frames, host_chunk_for(det->host_chunk_frames, format)), n_frames));
-  Slot& D = det->slot[0];
-  if ((rc = ensure_slot(det, D, g, chunk, 1, false, false))) return rc;
+  Slot& D = det->dense;
+  if ((rc = ensure_slot(det, D, g, chunk, false))) return rc;
   if (!det->up_stream) AG_CUDA(det, cudaStreamCreateWithFlags(&det->up_stream, cudaStreamNonBlocking));
   cudaStream_t s = D.stream, up = det->up_stream;
   const size_t chunk_bytes = (size_t)chunk * g.frame_stride;
@@ -1187,8 +1147,7 @@ static int detect_batch_host(ag_detector* det, const void* frames, size_t frame_
     if ((rc = ensure_host_stage(det, B, chunk_bytes, chunk, cap_per_frame))) return rc;
     const int n = n_this;
     const uint8_t* src = (const uint8_t*)frames + (size_t)f0 * g.frame_stride;
-    const size_t bytes = (size_t)(n - 1) * g.frame_stride + g.row_stride * (size_t)(g.h - 1) +
-                         (size_t)g.w * bytes_per_px(g.format);
+    const size_t bytes = (size_t)(n - 1) * g.frame_stride + frame_bytes(g);
     const uint8_t* up_src = src;
     if (pageable) {  // (the slot's previous upload is long done: its chunk has been collected)
       if (chunk_bytes > B.cap_h_in) {
@@ -1286,7 +1245,6 @@ int ag_detect_planes(ag_detector* det, const float* luma32f, size_t f32_row_stri
     return fail(det, AG_ERR_INVALID, "bad row stride");
   std::lock_guard<std::mutex> lk(det->mu);
   AG_CUDA(det, cudaSetDevice(det->device));
-  det->tap_valid = false;
   const size_t px = (size_t)width * height;
   FrameGeom gf;  // the f32 plane, packed
   gf.w = width; gf.h = height; gf.wpr = (width + 31) / 32; gf.n_words = gf.wpr * height; gf.n_px = width * height;
@@ -1297,58 +1255,20 @@ int ag_detect_planes(ag_detector* det, const float* luma32f, size_t f32_row_stri
   g8.row_stride = (size_t)width;
   g8.format = AG_L8;
   set_caps(det, gf);
-  Slot& S = det->big;
-  const int save_cl = det->cur_clusters, save_sd = det->cur_saddles;
-  int rc = AG_OK, cnt = 0;
+  auto upload = [&](uint8_t* d_in, cudaStream_t s) {
+    const cudaError_t e = cudaMemcpy2DAsync(d_in, gf.row_stride, luma32f, f32_row_stride, gf.row_stride, height,
+                                            cudaMemcpyHostToDevice, s);
+    return e != cudaSuccess ? e
+                            : cudaMemcpy2DAsync(d_in + 4 * px, g8.row_stride, luma8, u8_row_stride, g8.row_stride,
+                                                height, cudaMemcpyHostToDevice, s);
+  };
+  int cnt = 0;
   uint32_t st = 0;
-  for (;;) {
-    if (!(rc = ensure_slot(det, S, gf, 1, det->fam.n_codes, true))) {
-      cudaStream_t s = S.stream;
-      uint8_t* d_u8 = S.d_in + 4 * px;
-      if (cudaMemcpy2DAsync(S.d_in, gf.row_stride, luma32f, f32_row_stride, gf.row_stride, height, cudaMemcpyHostToDevice, s) !=
-              cudaSuccess ||
-          cudaMemcpy2DAsync(d_u8, g8.row_stride, luma8, u8_row_stride, g8.row_stride, height, cudaMemcpyHostToDevice, s) !=
-              cudaSuccess)
-        rc = AG_ERR_CUDA;
-      if (!rc) rc = run_dense(det, S, S.d_in, gf, 1, true, s);
-      if (!rc) rc = run_sparse(det, S, S.bb, gf, 1, S.d_status, s);
-      if (!rc && (cudaMemcpyAsync(S.h_status, S.d_status, sizeof(uint32_t), cudaMemcpyDeviceToHost, s) != cudaSuccess ||
-                  cudaStreamSynchronize(s) != cudaSuccess))
-        rc = AG_ERR_CUDA;
-      if (!rc && !(S.h_status[0] & kGrowable)) {
-        rc = run_boards(det, S.bb, d_u8, g8, 1, S.d_tags, S.cap_tags, S.d_ntags, S.d_status, false, s);
-        if (!rc && (cudaMemcpyAsync(S.h_ntags, S.d_ntags, sizeof(int), cudaMemcpyDeviceToHost, s) != cudaSuccess ||
-                    cudaMemcpyAsync(S.h_status, S.d_status, sizeof(uint32_t), cudaMemcpyDeviceToHost, s) != cudaSuccess ||
-                    cudaMemcpyAsync(S.h_tags, S.d_tags, sizeof(ag_tag) * (size_t)S.cap_tags, cudaMemcpyDeviceToHost, s) !=
-                        cudaSuccess ||
-                    cudaStreamSynchronize(s) != cudaSuccess))
-          rc = AG_ERR_CUDA;
-      } else if (!rc) {
-        S.h_ntags[0] = 0;
-      }
-    }
-    if (rc) break;
-    st = S.h_status[0];
-    cnt = S.h_ntags[0];
-    bool grew = false;
-    if ((st & AG_FRAME_CLUSTER_OVERFLOW) && det->cur_clusters < (1 << 22)) {
-      det->cur_clusters = (int)std::min<long>((long)det->cur_clusters * 16, 1l << 22);
-      grew = true;
-    }
-    if ((st & AG_FRAME_SADDLE_OVERFLOW) && det->cur_saddles < 16384) {
-      det->cur_saddles = 16384;
-      grew = true;
-    }
-    if (!grew) break;
-  }
-  det->cur_clusters = save_cl;
-  det->cur_saddles = save_sd;
-  if (rc) {
-    if (det->err.empty()) det->err = "ag_detect_planes failed";
-    return rc;
-  }
+  const int rc = run_one_frame(det, gf, g8, 4 * px, upload, FrameRun::kTags, 0, &cnt, &st);
+  if (rc) return rc;
+  const BoardSlot& B = det->big.bb;
   *n = cnt;
-  memcpy(out, S.h_tags, sizeof(ag_tag) * (size_t)std::min(std::min(cnt, cap), S.cap_tags));
+  memcpy(out, B.h_tags, sizeof(ag_tag) * (size_t)std::min(std::min(cnt, cap), B.hs_tags));
   if (st & (kGrowable | AG_FRAME_BOARD_OVERFLOW))
     return fail(det, AG_ERR_CAPACITY, "frame exceeds the detector's limits (clusters > 2^22, saddles > 16384 or a board wider than the lattice)");
   return cnt > cap ? fail(det, AG_ERR_CAPACITY, "cap too small") : AG_OK;
@@ -1366,13 +1286,12 @@ int ag_stage_run(ag_detector* det, const void* pixels, int width, int height, si
   int rc = make_geom(det, width, height, row_stride, 0, format, &g);
   if (rc) return rc;
   set_caps(det, g);
-  Slot& S = det->big;  // the one-frame slot: independent of the batch pipelines
-  if ((rc = ensure_slot(det, S, g, 1, det->fam.n_codes, true, true, true))) return rc;
-  const size_t bytes = g.row_stride * (size_t)(g.h - 1) + (size_t)g.w * bytes_per_px(g.format);
-  AG_CUDA(det, cudaMemcpyAsync(S.d_in, pixels, bytes, cudaMemcpyHostToDevice, S.stream));
-  if ((rc = run_chunk(det, S, S.d_in, g, 1, S.d_tags, S.cap_tags, S.d_ntags, S.d_status, true, S.stream)))
-    return rc;
-  AG_CUDA(det, cudaStreamSynchronize(S.stream));
+  auto upload = [&](uint8_t* d_in, cudaStream_t s) {
+    return cudaMemcpyAsync(d_in, pixels, frame_bytes(g), cudaMemcpyHostToDevice, s);
+  };
+  int cnt = 0;
+  uint32_t st = 0;
+  if ((rc = run_one_frame(det, g, g, 0, upload, FrameRun::kTaps, 0, &cnt, &st))) return rc;
   det->tap_geom = g;
   det->tap_valid = true;
   return AG_OK;
@@ -1476,10 +1395,10 @@ int ag_stage_board_quads(ag_detector* det, int32_t* quads_out, int cap, int* n) 
 int ag_stage_tags(ag_detector* det, ag_tag* out, int cap, int* n) {
   AG_TAP_PROLOGUE();
   int cnt = 0;
-  AG_CUDA(det, cudaMemcpy(&cnt, S.d_ntags, sizeof(int), cudaMemcpyDeviceToHost));
+  AG_CUDA(det, cudaMemcpy(&cnt, S.bb.d_ntags, sizeof(int), cudaMemcpyDeviceToHost));
   *n = cnt;
-  int m = std::min(std::min(cnt, cap), S.cap_tags);
-  if (m > 0) AG_CUDA(det, cudaMemcpy(out, S.d_tags, sizeof(ag_tag) * m, cudaMemcpyDeviceToHost));
+  int m = std::min(std::min(cnt, cap), S.bb.hs_tags);
+  if (m > 0) AG_CUDA(det, cudaMemcpy(out, S.bb.d_tags, sizeof(ag_tag) * m, cudaMemcpyDeviceToHost));
   return AG_OK;
 }
 
@@ -1489,51 +1408,19 @@ int ag_refined_saddle_points(ag_detector* det, const void* pixels, int width, in
   if (!pixels || !out || !n) return fail(det, AG_ERR_INVALID, "null pointer");
   std::lock_guard<std::mutex> lk(det->mu);
   AG_CUDA(det, cudaSetDevice(det->device));
-  det->tap_valid = false;
   FrameGeom g;
   int rc = make_geom(det, width, height, row_stride, 0, format, &g);
   if (rc) return rc;
   set_caps(det, g);
-  Slot& S = det->big;  // the one-frame slot: independent of the batch pipelines
-  const int save_cl = det->cur_clusters, save_sd = det->cur_saddles;
-  const size_t bytes = g.row_stride * (size_t)(g.h - 1) + (size_t)g.w * bytes_per_px(g.format);
+  auto upload = [&](uint8_t* d_in, cudaStream_t s) {
+    return cudaMemcpyAsync(d_in, pixels, frame_bytes(g), cudaMemcpyHostToDevice, s);
+  };
   int cnt = 0;
   uint32_t st = 0;
-  // a frame that overflows the capacities is run again with grown ones (the reference has no limits)
-  for (;;) {
-    if (!(rc = ensure_slot(det, S, g, 1, det->fam.n_codes, true))) {
-      if (cudaMemcpyAsync(S.d_in, pixels, bytes, cudaMemcpyHostToDevice, S.stream) != cudaSuccess) rc = AG_ERR_CUDA;
-      if (!rc) rc = run_dense(det, S, S.d_in, g, 1, true, S.stream);
-      if (!rc) rc = run_sparse(det, S, S.bb, g, 1, S.d_status, S.stream);
-      if (!rc && (cudaMemcpyAsync(S.h_ntags, S.bb.d_nref, sizeof(int), cudaMemcpyDeviceToHost, S.stream) != cudaSuccess ||
-                  cudaMemcpyAsync(S.h_status, S.d_status, sizeof(uint32_t), cudaMemcpyDeviceToHost, S.stream) !=
-                      cudaSuccess ||
-                  cudaStreamSynchronize(S.stream) != cudaSuccess))
-        rc = AG_ERR_CUDA;
-    }
-    if (rc) break;
-    cnt = S.h_ntags[0];
-    st = S.h_status[0];
-    bool grew = false;
-    if ((st & AG_FRAME_CLUSTER_OVERFLOW) && det->cur_clusters < (1 << 22)) {
-      det->cur_clusters = (int)std::min<long>((long)det->cur_clusters * 16, 1l << 22);
-      grew = true;
-    }
-    if ((st & AG_FRAME_SADDLE_OVERFLOW) && det->cur_saddles < 16384) {
-      det->cur_saddles = 16384;
-      grew = true;
-    }
-    if (!grew) break;
-  }
-  det->cur_clusters = save_cl;
-  det->cur_saddles = save_sd;
-  if (rc) {
-    if (det->err.empty()) det->err = "refined_saddle_points failed";
-    return rc;
-  }
+  if ((rc = run_one_frame(det, g, g, 0, upload, FrameRun::kSaddles, 0, &cnt, &st))) return rc;
   *n = cnt;
   int m = std::min(cnt, cap);
-  if (m > 0) AG_CUDA(det, cudaMemcpy(out, S.bb.d_refined, sizeof(ag_saddle) * m, cudaMemcpyDeviceToHost));
+  if (m > 0) AG_CUDA(det, cudaMemcpy(out, det->big.bb.d_refined, sizeof(ag_saddle) * m, cudaMemcpyDeviceToHost));
   if (st & kGrowable) return fail(det, AG_ERR_CAPACITY, "frame exceeds the detector's limits (clusters > 2^22 or saddles > 16384)");
   return cnt > cap ? fail(det, AG_ERR_CAPACITY, "saddle capacity too small") : AG_OK;
 }
@@ -1581,7 +1468,7 @@ int ag_gaussian_blur_f32(ag_detector* det, const float* img, int width, int heig
   const size_t n = (size_t)width * height;
   int rc = ensure_f32(det, n);
   if (rc) return rc;
-  Slot& S = det->slot[0];
+  Slot& S = det->dense;
   if (!S.stream) {
     AG_CUDA(det, cudaStreamCreateWithFlags(&S.stream, cudaStreamNonBlocking));
     AG_CUDA(det, cudaEventCreateWithFlags(&S.done, cudaEventDisableTiming));
@@ -1629,7 +1516,7 @@ int ag_hessian_response(ag_detector* det, const float* img, int width, int heigh
   const size_t n = (size_t)width * height;
   int rc = ensure_f32(det, n);
   if (rc) return rc;
-  Slot& S = det->slot[0];
+  Slot& S = det->dense;
   if (!S.stream) {
     AG_CUDA(det, cudaStreamCreateWithFlags(&S.stream, cudaStreamNonBlocking));
     AG_CUDA(det, cudaEventCreateWithFlags(&S.done, cudaEventDisableTiming));
@@ -1733,23 +1620,23 @@ AG_API int ag_test_boards_from_saddles(ag_detector* det, const ag_saddle* saddle
   set_caps(det, g);
   if (n > det->cur_saddles) return fail(det, AG_ERR_INVALID, "more saddles than max_saddles");
   Slot& S = det->big;
-  if ((rc = ensure_slot(det, S, g, 1, det->fam.n_codes, true))) return rc;
-  const size_t bytes = g.row_stride * (size_t)(g.h - 1) + (size_t)g.w * bytes_per_px(g.format);
+  BoardSlot& B = S.bb;
+  if ((rc = ensure_slot(det, S, g, 1))) return rc;
   cudaStream_t s = S.stream;
-  AG_CUDA(det, cudaMemcpyAsync(S.d_in, pixels, bytes, cudaMemcpyHostToDevice, s));
-  if (n > 0) AG_CUDA(det, cudaMemcpyAsync(S.bb.d_refined, saddles, sizeof(ag_saddle) * n, cudaMemcpyHostToDevice, s));
-  AG_CUDA(det, cudaMemcpyAsync(S.bb.d_nref, &n, sizeof(int), cudaMemcpyHostToDevice, s));
-  AG_CUDA(det, cudaMemsetAsync(S.d_status, 0, sizeof(uint32_t), s));
-  if ((rc = run_boards(det, S.bb, S.d_in, g, 1, S.d_tags, S.cap_tags, S.d_ntags, S.d_status, true, s))) return rc;
+  AG_CUDA(det, cudaMemcpyAsync(B.d_in, pixels, frame_bytes(g), cudaMemcpyHostToDevice, s));
+  if (n > 0) AG_CUDA(det, cudaMemcpyAsync(B.d_refined, saddles, sizeof(ag_saddle) * n, cudaMemcpyHostToDevice, s));
+  AG_CUDA(det, cudaMemcpyAsync(B.d_nref, &n, sizeof(int), cudaMemcpyHostToDevice, s));
+  AG_CUDA(det, cudaMemsetAsync(B.d_status, 0, sizeof(uint32_t), s));
+  if ((rc = run_boards(det, B, B.d_in, g, 1, B.d_tags, B.hs_tags, B.d_ntags, B.d_status, true, s))) return rc;
   int nq = 0, nt = 0;
-  AG_CUDA(det, cudaMemcpyAsync(&nq, S.bb.d_tap_nquads, sizeof(int), cudaMemcpyDeviceToHost, s));
-  AG_CUDA(det, cudaMemcpyAsync(&nt, S.d_ntags, sizeof(int), cudaMemcpyDeviceToHost, s));
+  AG_CUDA(det, cudaMemcpyAsync(&nq, B.d_tap_nquads, sizeof(int), cudaMemcpyDeviceToHost, s));
+  AG_CUDA(det, cudaMemcpyAsync(&nt, B.d_ntags, sizeof(int), cudaMemcpyDeviceToHost, s));
   AG_CUDA(det, cudaStreamSynchronize(s));
   *n_quads = nq;
   *n_tags = nt;
-  const int mq = std::min(std::min(nq, quad_cap), S.bb.layout[0].max_quads), mt = std::min(std::min(nt, tag_cap), S.cap_tags);
-  if (mq > 0) AG_CUDA(det, cudaMemcpy(quads_out, S.bb.d_tap_quads, sizeof(int32_t) * 4 * mq, cudaMemcpyDeviceToHost));
-  if (mt > 0) AG_CUDA(det, cudaMemcpy(tags_out, S.d_tags, sizeof(ag_tag) * mt, cudaMemcpyDeviceToHost));
+  const int mq = std::min(std::min(nq, quad_cap), B.layout[0].max_quads), mt = std::min(std::min(nt, tag_cap), B.hs_tags);
+  if (mq > 0) AG_CUDA(det, cudaMemcpy(quads_out, B.d_tap_quads, sizeof(int32_t) * 4 * mq, cudaMemcpyDeviceToHost));
+  if (mt > 0) AG_CUDA(det, cudaMemcpy(tags_out, B.d_tags, sizeof(ag_tag) * mt, cudaMemcpyDeviceToHost));
   return AG_OK;
 }
 
