@@ -135,7 +135,8 @@ def lib():
         L.ag_test_board_layout.argtypes = [ci, ci, ci, ci, ci, ci, vp]
         L.ag_test_board_decode_room.argtypes = [ci, ci, ci, vp]
         L.ag_test_render_pose.argtypes = [vp, vp, ci, ci, ci, ci, vp, ci, C.c_uint64]
-        L.ag_test_boards_from_saddles.argtypes = [vp, vp, ci, vp, ci, ci, sz, ci, vp, ci, vp, vp, ci, vp]
+        L.ag_test_boards_from_saddles.argtypes = [vp, vp, sz, vp, ci, vp, sz, ci, ci, sz, ci, vp, ci, vp, vp, ci,
+                                                  vp, vp]
         L.ag_test_float_luma.argtypes = [vp, vp, C.c_longlong, ci, vp, vp]
         L.ag_test_host_chunk.argtypes = [C.c_longlong, ci, vp]
         _lib = L
@@ -383,15 +384,39 @@ class TagDetector:
     def _boards_from_saddles(self, saddles, img):
         """Test hook: board search + decode on a given saddle list (N x 5 float32: x, y, k, theta, phi).
         Returns (quads of the first best board [M x 4 int32], {id: corners})."""
-        sd = np.ascontiguousarray(saddles, np.float32).reshape(-1, 5)
-        img = np.ascontiguousarray(img)
-        fmt, w, h, st = image_format(img)
-        quads = np.zeros((4096, 4), np.int32)
-        tags = np.zeros(1024, TAG_DTYPE)
-        nq, nt = C.c_int(0), C.c_int(0)
-        self._check(lib().ag_test_boards_from_saddles(self._h, _p(sd), len(sd), _p(img), w, h, st, fmt, _p(quads), 4096,
-                                                      C.byref(nq), _p(tags), 1024, C.byref(nt)))
-        return quads[:nq.value].copy(), _tags_to_dict(tags[:nt.value])
+        quads, rec, n_tags, _ = self._boards_from_saddle_batch([saddles], np.asarray(img)[None])
+        return quads[0], _tags_to_dict(rec[0, :n_tags[0]])
+
+    def _boards_from_saddle_batch(self, saddle_lists, frames, tag_cap=1024):
+        """Test hook: board search + decode of frames[f] (N x H x W[...] with the saddle list
+        saddle_lists[f] (N_f x 5 float32) each, all in ONE run of the board kernel's launches, which the
+        handle's board options pick as in the pipeline.  Returns (quads of the first best board per
+        frame [list of M_f x 4 int32], tag records [frames x tag_cap TAG_DTYPE], tag counts [frames],
+        status bits [frames]).  A count of -1 means that no launch took the frame; records past the
+        count are all-ones bytes unless the kernel wrote them."""
+        lists = [np.ascontiguousarray(s, np.float32).reshape(-1, 5) for s in saddle_lists]
+        frames = np.ascontiguousarray(frames)
+        n = len(lists)
+        if n != frames.shape[0] or n == 0:
+            raise ValueError("one saddle list per frame, at least one frame")
+        fmt, w, h, st = image_format(frames[0])
+        counts = np.array([len(s) for s in lists], np.int32)
+        stride = max(1, int(counts.max()))
+        packed = np.zeros((n, stride, 5), np.float32)
+        for f, s in enumerate(lists):
+            packed[f, :len(s)] = s
+        rec = np.zeros((n, tag_cap), TAG_DTYPE)
+        n_quads, n_tags, status = np.zeros(n, np.int32), np.zeros(n, np.int32), np.zeros(n, np.uint32)
+        quad_cap = stride // 4 + 2  # the board kernel's own bound on the quads of a list
+        while True:
+            quads = np.zeros((n, quad_cap, 4), np.int32)
+            self._check(lib().ag_test_boards_from_saddles(
+                self._h, _p(packed), stride, _p(counts), n, _p(frames), frames.strides[0], w, h, st, fmt, _p(quads),
+                quad_cap, _p(n_quads), _p(rec), tag_cap, _p(n_tags), _p(status)))
+            if n_quads.max() <= quad_cap:
+                break
+            quad_cap = int(n_quads.max())
+        return [quads[f, :max(0, n_quads[f])].copy() for f in range(n)], rec, n_tags, status
 
     def _render_pose(self, d_frame_ptr, width, height, cols, rows, hinv, noise=False, seed=0):
         """Test hook: one frame of the device renderer under a given image -> page homography."""

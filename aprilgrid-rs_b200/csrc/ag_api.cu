@@ -1603,40 +1603,69 @@ AG_API int ag_test_render_pose(ag_detector* det, void* d_frame, int width, int h
   return AG_OK;
 }
 
-// Test hook (not in the public header): the board search + decoding (K6) on a GIVEN saddle list
-// (n x {x, y, k, theta, phi}, host) over a host image -- so that tests can put saddles exactly on
-// the gates of init_quads / is_valid_quad / the theta histogram.  Returns the quads of the first
-// best board (the tap) and the tags.
-AG_API int ag_test_boards_from_saddles(ag_detector* det, const ag_saddle* saddles, int n, const void* pixels,
+// Test hook (not in the public header): the board search + decoding (K6) on GIVEN saddle lists over
+// host frames -- so that tests can put saddles exactly on the gates of init_quads / is_valid_quad /
+// the theta histogram, and frames exactly on the saddle counts where the launches of a batch and the
+// on-chip tiers part.  Frame f has n_saddles[f] saddles at saddles + f * saddle_stride (records of
+// {x, y, k, theta, phi}) and its pixels at pixels + f * frame_stride (0 = packed).  All n_frames go
+// through ONE run_boards, so the handle's board options pick the launches as in the pipeline.
+// Out, per frame: the quads of the first best board (quads_out + f * quad_cap * 4, n_quads[f] of
+// them), tag_cap tag records (tags_out + f * tag_cap, n_tags[f] of them valid) and the status bits.
+// Counts start at -1 and records at all-ones bytes: a frame that no launch took comes back so.
+AG_API int ag_test_boards_from_saddles(ag_detector* det, const ag_saddle* saddles, size_t saddle_stride,
+                                       const int* n_saddles, int n_frames, const void* pixels, size_t frame_stride,
                                        int width, int height, size_t row_stride, int format, int32_t* quads_out,
-                                       int quad_cap, int* n_quads, ag_tag* tags_out, int tag_cap, int* n_tags) {
-  if (!det || !saddles || !pixels || !quads_out || !n_quads || !tags_out || !n_tags || n < 0) return AG_ERR_INVALID;
+                                       int quad_cap, int* n_quads, ag_tag* tags_out, int tag_cap, int* n_tags,
+                                       uint32_t* status) {
+  if (!det || !saddles || !n_saddles || n_frames < 1 || !pixels || !quads_out || quad_cap < 0 || !n_quads ||
+      !tags_out || tag_cap < 0 || !n_tags || !status)
+    return AG_ERR_INVALID;
   std::lock_guard<std::mutex> lk(det->mu);
   AG_CUDA(det, cudaSetDevice(det->device));
-  det->tap_valid = false;
+  det->tap_valid = false;  // the taps read the one-frame slot's board side
   FrameGeom g;
-  int rc = make_geom(det, width, height, row_stride, 0, format, &g);
+  int rc = make_geom(det, width, height, row_stride, frame_stride, format, &g);
   if (rc) return rc;
   set_caps(det, g);
-  if (n > det->cur_saddles) return fail(det, AG_ERR_INVALID, "more saddles than max_saddles");
-  Slot& S = det->big;
-  BoardSlot& B = S.bb;
-  if ((rc = ensure_slot(det, S, g, 1))) return rc;
-  cudaStream_t s = S.stream;
-  AG_CUDA(det, cudaMemcpyAsync(B.d_in, pixels, frame_bytes(g), cudaMemcpyHostToDevice, s));
-  if (n > 0) AG_CUDA(det, cudaMemcpyAsync(B.d_refined, saddles, sizeof(ag_saddle) * n, cudaMemcpyHostToDevice, s));
-  AG_CUDA(det, cudaMemcpyAsync(B.d_nref, &n, sizeof(int), cudaMemcpyHostToDevice, s));
-  AG_CUDA(det, cudaMemsetAsync(B.d_status, 0, sizeof(uint32_t), s));
-  if ((rc = run_boards(det, B, B.d_in, g, 1, B.d_tags, B.hs_tags, B.d_ntags, B.d_status, true, s))) return rc;
-  int nq = 0, nt = 0;
-  AG_CUDA(det, cudaMemcpyAsync(&nq, B.d_tap_nquads, sizeof(int), cudaMemcpyDeviceToHost, s));
-  AG_CUDA(det, cudaMemcpyAsync(&nt, B.d_ntags, sizeof(int), cudaMemcpyDeviceToHost, s));
+  int max_n = 0;
+  for (int f = 0; f < n_frames; ++f) {
+    if (n_saddles[f] < 0) return fail(det, AG_ERR_INVALID, "negative saddle count");
+    max_n = std::max(max_n, n_saddles[f]);
+  }
+  if (max_n > det->cur_saddles) return fail(det, AG_ERR_INVALID, "more saddles than max_saddles");
+  if ((size_t)max_n > saddle_stride) return fail(det, AG_ERR_INVALID, "saddle_stride smaller than a list");
+  // the board side of the one-frame slot only: its dense buffers are not needed
+  BoardSlot& B = det->big.bb;
+  if ((rc = ensure_board_slot(det, B, n_frames, true)) ||
+      (rc = ensure_host_stage(det, B, (size_t)n_frames * g.frame_stride, n_frames, det->fam.n_codes)))
+    return rc;
+  const cudaStream_t s = B.bstream;
+  const int cap = B.hs_tags, mq = B.layout[0].max_quads;
+  AG_CUDA(det, cudaMemcpyAsync(B.d_in, pixels, g.frame_stride * (size_t)(n_frames - 1) + frame_bytes(g),
+                               cudaMemcpyHostToDevice, s));
+  if (max_n > 0)
+    AG_CUDA(det, cudaMemcpy2DAsync(B.d_refined, sizeof(ag_saddle) * (size_t)B.cap_saddles, saddles,
+                                   sizeof(ag_saddle) * saddle_stride,
+                                   sizeof(ag_saddle) * (size_t)max_n, n_frames, cudaMemcpyHostToDevice, s));
+  AG_CUDA(det, cudaMemcpyAsync(B.d_nref, n_saddles, sizeof(int) * n_frames, cudaMemcpyHostToDevice, s));
+  AG_CUDA(det, cudaMemsetAsync(B.d_status, 0, sizeof(uint32_t) * n_frames, s));
+  AG_CUDA(det, cudaMemsetAsync(B.d_ntags, 0xff, sizeof(int) * n_frames, s));
+  AG_CUDA(det, cudaMemsetAsync(B.d_tags, 0xff, sizeof(ag_tag) * (size_t)cap * n_frames, s));
+  AG_CUDA(det, cudaMemsetAsync(B.d_tap_nquads, 0xff, sizeof(int) * n_frames, s));
+  AG_CUDA(det, cudaMemsetAsync(B.d_tap_quads, 0xff, sizeof(int32_t) * 4 * (size_t)mq * n_frames, s));
+  if ((rc = run_boards(det, B, B.d_in, g, n_frames, B.d_tags, cap, B.d_ntags, B.d_status, true, s))) return rc;
+  AG_CUDA(det, cudaMemcpyAsync(n_quads, B.d_tap_nquads, sizeof(int) * n_frames, cudaMemcpyDeviceToHost, s));
+  AG_CUDA(det, cudaMemcpyAsync(n_tags, B.d_ntags, sizeof(int) * n_frames, cudaMemcpyDeviceToHost, s));
+  AG_CUDA(det, cudaMemcpyAsync(status, B.d_status, sizeof(uint32_t) * n_frames, cudaMemcpyDeviceToHost, s));
+  const int kq = std::min(quad_cap, mq), kt = std::min(tag_cap, cap);
+  if (kq > 0)
+    AG_CUDA(det, cudaMemcpy2DAsync(quads_out, sizeof(int32_t) * 4 * (size_t)quad_cap, B.d_tap_quads,
+                                   sizeof(int32_t) * 4 * (size_t)mq, sizeof(int32_t) * 4 * (size_t)kq, n_frames,
+                                   cudaMemcpyDeviceToHost, s));
+  if (kt > 0)
+    AG_CUDA(det, cudaMemcpy2DAsync(tags_out, sizeof(ag_tag) * (size_t)tag_cap, B.d_tags, sizeof(ag_tag) * (size_t)cap,
+                                   sizeof(ag_tag) * (size_t)kt, n_frames, cudaMemcpyDeviceToHost, s));
   AG_CUDA(det, cudaStreamSynchronize(s));
-  *n_quads = nq;
-  *n_tags = nt;
-  const int mq = std::min(std::min(nq, quad_cap), B.layout[0].max_quads), mt = std::min(std::min(nt, tag_cap), B.hs_tags);
-  if (mq > 0) AG_CUDA(det, cudaMemcpy(quads_out, B.d_tap_quads, sizeof(int32_t) * 4 * mq, cudaMemcpyDeviceToHost));
-  if (mt > 0) AG_CUDA(det, cudaMemcpy(tags_out, B.d_tags, sizeof(ag_tag) * mt, cudaMemcpyDeviceToHost));
   return AG_OK;
 }
 

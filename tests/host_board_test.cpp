@@ -33,11 +33,12 @@ extern "C" void agb_reset_keys() { for (auto& a : g_keys) for (auto& b : a) b.cl
 extern "C" {
 
 // saddles: n x {x, y, k, theta, phi}.  Returns number of tags written (ascending id).
+// smem_saddles: the on-chip saddle tier of the device launch being mirrored (320, 512, 1024 or 4096).
 int hb_detect_from_saddles(const float* saddles, int n, const uint8_t* img, int w, int h,
                            size_t row_stride, int format, const uint64_t* codes, int n_codes,
                            int edge, int border, int hamming, int max_boards, int max_saddles,
                            agb::TagRec* out, int cap, int32_t* tap_quads, int* tap_n, int tap_cap,
-                           uint32_t* status, int use_grid, int lattice) {
+                           uint32_t* status, int use_grid, int lattice, int smem_saddles) {
   using namespace agb;
   if (n > max_saddles) return -1;
   const int N = max_saddles, Q = N / 4 + 2;
@@ -69,15 +70,17 @@ int hb_detect_from_saddles(const float* saddles, int n, const uint8_t* img, int 
   F.ctl = ctl; F.w_score = ctl + 8;
   F.warp = 0; F.n_warps = 1;
   F.lat = lattice; F.lat_off = lattice / 2;
-  // bucket grid (the device kernel sizes it the same way); use_grid = 0 tests the exhaustive scan
+  // bucket grid, sized as the device kernel's general path sizes it: 1408 buckets (8192 in the 4096
+  // tier), items for the tier's saddles -- or for max_saddles when the list is larger than the tier
+  // and lives in global memory; use_grid = 0 tests the exhaustive scan
   int bucket = 32;
-  const int grid_cap = 1408;
+  const int grid_cap = smem_saddles == 4096 ? 8192 : 1408;
   while (((w + bucket - 1) / bucket) * ((h + bucket - 1) / bucket) > grid_cap) bucket *= 2;
   std::vector<uint16_t> gstart(grid_cap + 1), gitem(N);
   if (use_grid) {
     F.g_start = gstart.data(); F.g_item = gitem.data();
     F.g_nx = (w + bucket - 1) / bucket; F.g_ny = (h + bucket - 1) / bucket;
-    F.g_cap_cells = grid_cap; F.g_cap_items = 512;  // as on the device
+    F.g_cap_cells = grid_cap; F.g_cap_items = n <= smem_saddles ? smem_saddles : max_saddles;
     F.g_inv = 1.0f / (float)bucket;
   }
   F.stack = stack.data(); F.seeds = seeds.data(); F.nn_idx = nn.data(); F.same = same.data();

@@ -22,7 +22,7 @@ def hb():
 
 
 def host_detect(hb, pkg, oracle, img, saddles=None, family=None, max_boards=2, max_saddles=2048,
-                use_grid=1, lattice=64):
+                use_grid=1, lattice=64, smem_saddles=512):
     family = pkg.TagFamily.T36H11 if family is None else family  # T16H5 is 0
     fam = pkg.family_info(family)
     if saddles is None:
@@ -38,7 +38,7 @@ def host_detect(hb, pkg, oracle, img, saddles=None, family=None, max_boards=2, m
         s.ctypes.data_as(vp), len(s), img.ctypes.data_as(vp), w, h, C.c_size_t(st), fmt,
         codes.ctypes.data_as(vp), len(codes), fam["edge"], fam["border"], fam["hamming"], max_boards,
         max_saddles, out.ctypes.data_as(vp), 1024, quads.ctypes.data_as(vp), C.byref(tapn), 1024,
-        C.byref(status), use_grid, lattice)
+        C.byref(status), use_grid, lattice, smem_saddles)
     assert n >= 0
     return ({int(t["id"]): t["xy"].reshape(4, 2).copy() for t in out[:n]}, quads[:tapn.value],
             status.value, s)
@@ -79,7 +79,8 @@ def test_bucket_grid_and_exhaustive_search_agree(hb, pkg, oracle, images):
 
 
 def test_more_saddles_than_the_on_chip_grid_holds(hb, pkg, oracle):
-    """> 512 saddles: the bucket grid is skipped (exhaustive search), result unchanged."""
+    """> 512 saddles with the 512 tier: the bucket grid's items live in the frame's workspace, as on
+    the device; result unchanged."""
     img = synth.render_board_numpy(1600, 1200, cols=12, rows=9, seed=4, tag_px=70.0)
     fe = oracle.front_end(img, want_labels=False)
     assert len(fe["refined"]) > 512
@@ -88,6 +89,26 @@ def test_more_saddles_than_the_on_chip_grid_holds(hb, pkg, oracle):
     assert sorted(got) == sorted(want) and len(want) >= 100
     for k in want:
         assert np.array_equal(got[k], want[k])
+
+
+@pytest.mark.parametrize("key", ["1408x1024", "1409x1024"])
+def test_bucket_grid_edge_lists_identical_to_oracle(hb, pkg, oracle, key):
+    """The exact-size saddle lists of the GPU suite's bucket-grid edge (1408 x 1024: 32 px buckets,
+    1409 x 1024: 64 px) through the general path as each launch of the 512 tier runs it (320 and 512
+    saddles on chip; a list beyond them keeps its grid items in the frame's workspace), and with the
+    exhaustive scan."""
+    from test_gpu_board_edges import CANVASES, canvas, exact_case
+    img = canvas(key, oracle)
+    for n in CANVASES[key][3]:
+        s, want_q, want_t = exact_case(key, n, oracle)
+        for smem, use_grid in ((320, 1), (512, 1), (512, 0)):
+            got, quads, status, _ = host_detect(hb, pkg, oracle, img, saddles=s, use_grid=use_grid,
+                                                smem_saddles=smem)
+            what = (key, n, smem, use_grid)
+            assert status == 0 and want_q is not None and np.array_equal(quads, want_q), what
+            assert sorted(got) == sorted(want_t) and len(want_t) >= 10, what
+            for k in want_t:
+                assert np.array_equal(got[k], want_t[k]), what
 
 
 def test_small_lattice_same_result_and_overflow_flag(hb, pkg, oracle, images):

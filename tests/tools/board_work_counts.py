@@ -44,7 +44,7 @@ for i in range(n):
     r = hb.hb_detect_from_saddles(s.ctypes.data_as(vp), len(s), img.ctypes.data_as(vp), 1280, 1024,
                                   C.c_size_t(1280), 0, codes.ctypes.data_as(vp), len(codes), fam["edge"],
                                   fam["border"], fam["hamming"], 2, 2048, out.ctypes.data_as(vp), 1024,
-                                  None, None, 0, C.byref(st), 1, 64)
+                                  None, None, 0, C.byref(st), 1, 64, 512)
     t_total += time.perf_counter() - t0
     c = np.array([cnt[k] for k in range(32)], np.int64)
     tot += c

@@ -39,7 +39,7 @@ for i in range(n):
     hb.hb_detect_from_saddles(s.ctypes.data_as(vp), len(s), img.ctypes.data_as(vp), 1280, 1024,
                               C.c_size_t(1280), 0, codes.ctypes.data_as(vp), len(codes), fam["edge"],
                               fam["border"], fam["hamming"], 2, 2048, out.ctypes.data_as(vp), 1024,
-                              None, None, 0, C.byref(st), 1, 64)
+                              None, None, 0, C.byref(st), 1, 64, 512)
     q = np.zeros((400000, 7), np.float32)
     m = hb.agb_get_queries(q.ctypes.data_as(vp), len(q))
     q = q[:m]
