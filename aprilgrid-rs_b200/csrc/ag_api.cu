@@ -41,12 +41,14 @@ bool family_info(int family, FamilyInfo* f) {  // src/detector.rs:369-405
 // creation errors have no handle to live in: one message per calling thread
 thread_local std::string g_create_error;
 
-// Pipeline.  The dense + sparse front end (K1-K4) of chunk i+1 runs on one stream while the
-// latency-bound board searches of chunks i, i-1, ... run on their board slots' own streams, side
-// by side.  The dense buffers of ONE slot are reused chunk after chunk (K1-K4 of consecutive
-// chunks are serial on that stream anyway); only the light board-search side is multi-buffered,
-// so the board searches of up to kBoardSlots chunks overlap each other and the front end of later
-// chunks, which hides the long tail of the slowest frames of a chunk.
+// Pipeline.  The dense front end (K1-K2) of a chunk runs on the dense stream, its sparse stages
+// (K3-K4) on the detector's sparse stream, and the latency-bound board searches of earlier chunks
+// on their board slots' own streams, side by side.  The dense buffers come in a ring of
+// kDenseSets sets used by chunks in turn, so K1 of chunk i+1 runs while K3-K4 of chunk i still
+// read chunk i's set; the light board-search side is multi-buffered further, so the board
+// searches of up to kBoardSlots chunks overlap each other and the front end of later chunks,
+// which hides the long tail of the slowest frames of a chunk.
+constexpr int kDenseSets = 2;
 constexpr int kBoardSlots = 8;
 #ifndef AG_BIG_TIER_WARPS
 #define AG_BIG_TIER_WARPS 2
@@ -96,11 +98,15 @@ struct BoardSlot {
 // Dense and sparse buffers of one chunk (K1-K4).
 struct Slot {
   cudaStream_t stream = nullptr;
+  // the last work on the buffers is done: K3-K4 of the set's latest chunk (ring of the batch
+  // pipelines), K2 (ag_dense_batch_device)
   cudaEvent_t done = nullptr;
+  cudaEvent_t ev_dense = nullptr;  // ring: K1-K2 of the set's latest chunk done (the sparse stream waits on it)
   BoardSlot bb;  // the slot's own board-search side and host staging (one-frame slot only)
+  // capacities in elements (frames x per-frame stride), except cap_frames
   int cap_frames = 0;
-  size_t cap_px = 0, cap_words = 0;
-  int cap_clusters = 0, cap_saddles = 0;
+  size_t cap_px = 0, cap_words = 0, cap_list = 0, cap_cl = 0;
+  int cap_clusters = 0;  // clusters per frame of the current call (stride of the cluster buffers)
   float *d_blur = nullptr, *d_resp = nullptr;
   uint32_t *d_min = nullptr, *d_mask = nullptr;
   int *d_parent = nullptr, *d_acc = nullptr, *d_ncl = nullptr;
@@ -110,7 +116,7 @@ struct Slot {
   // taps
   int* d_label_fallback = nullptr;  // K3: frames the run-based kernel handed to the pixel-list kernel
   uint32_t* d_pixlist = nullptr;   // K3: compact list of mask pixels / runs, [frames][pix_cap]
-  int pix_cap = 0;
+  int pix_cap = 0;  // list entries per frame of the current call
 };
 
 }  // namespace
@@ -122,7 +128,11 @@ struct ag_detector {
   ag_params params{};
   std::mutex mu;
   std::string err;
-  Slot dense;  // dense + sparse buffers of the batch pipelines
+  // dense + sparse buffers of the batch pipelines, used by chunks in turn; dense[0]'s stream is the
+  // detector's own dense stream (host-frame path, standalone operators, calls without a stream)
+  Slot dense[kDenseSets];
+  int dense_rr = 0;                      // next set of the ring (rotates across calls and both pipelines)
+  cudaStream_t sparse_stream = nullptr;  // K3-K4 of the batch pipelines
   Slot big;  // one-frame slot with grown capacities: frames that overflowed max_clusters / max_saddles are re-run here
   BoardSlot bslot[kBoardSlots];
   int slot_rr = 0;            // next board slot of the device-batch pipeline (rotates across calls)
@@ -143,7 +153,7 @@ struct ag_detector {
   bool host_async = false;      // ag_detect_batch returns without collecting its results
   bool host_truncated = false;  // a collected frame had more tags than its call's cap_per_frame
   bool host_unresolved = false;  // a collected frame overflowed a capacity that could not be grown
-  bool device_path_busy = false;  // device-batch work may still be in flight on the dense slot / the board slots
+  bool device_path_busy = false;  // device-batch work may still be in flight on the dense sets / the board slots
   bool device_async = false;  // ag_detect_batch_device returns without ordering the results on the
                               // caller's stream; ag_detect_batch_device_wait does that
   uint64_t launches = 0;
@@ -259,7 +269,9 @@ long host_chunk_for(long host_chunk_frames, int format) {
   return bpp > 8 ? std::max<long>(1, host_chunk_frames * 8 / bpp) : host_chunk_frames;
 }
 // Frames per pipeline chunk: the option, bounded so that the dense buffers of a chunk (blur +
-// response, 8 bytes per pixel) stay below 24 GB whatever the image size.
+// response, 8 bytes per pixel) stay below 24 GB whatever the image size.  The bound is per set:
+// the pipelines keep kDenseSets = 2 sets, about 8.6 bytes per pixel each with mask and pixel list,
+// so chunks of 1024 frames of 1280 x 1024 take 2 x 11.6 GB = 23.2 GB of dense buffers.
 int chunk_limit(const ag_detector* det, const FrameGeom& g, long want) {
   const long by_mem = std::max<long>(1, (long)((24ull << 30) / ((unsigned long long)g.n_px * 8ull)));
   return (int)std::max<long>(1, std::min<long>(want, by_mem));
@@ -384,47 +396,56 @@ int ensure_slot(ag_detector* det, Slot& S, const FrameGeom& g, int frames, bool 
     AG_CUDA(det, cudaStreamCreateWithFlags(&S.stream, cudaStreamNonBlocking));
     AG_CUDA(det, cudaEventCreateWithFlags(&S.done, cudaEventDisableTiming));
   }
+  // (the standalone operators create the first set's stream and event without this one)
+  if (!S.ev_dense) AG_CUDA(det, cudaEventCreateWithFlags(&S.ev_dense, cudaEventDisableTiming));
   if (own_board && ((rc = ensure_board_slot(det, S.bb, frames, true)) ||
                     (rc = ensure_host_stage(det, S.bb, (size_t)frames * g.frame_stride, frames, det->fam.n_codes))))
     return rc;
-  const bool grow_frames = frames > S.cap_frames;
-  const int F = std::max(frames, S.cap_frames);
-  const size_t px = std::max((size_t)g.n_px, S.cap_px);
-  const size_t words = std::max((size_t)g.n_words, S.cap_words);
-  if (grow_frames || px > S.cap_px || words > S.cap_words) {
-    // make sure nothing is in flight on the buffers we are about to free
+  // Per-frame strides follow this call's geometry; each buffer grows to the most elements (frames x
+  // stride) a call has needed, not to the most frames times the largest image: a set that served
+  // chunks of 1024 small frames and then 256 4K frames holds 256 x 4K pixels, not 1024 x 4K.
+  // The saddle mask is 1-4 % full; a list of 1/8 of the pixels covers every real image, fuller
+  // masks (noise) take the word-oriented labelling path.
+  const int pix_cap = (int)std::min<size_t>(std::max<size_t>((size_t)g.n_px / 8, 32768), (size_t)1 << 20);
+  const size_t px = (size_t)frames * g.n_px, words = (size_t)frames * g.n_words, list = (size_t)frames * pix_cap;
+  if (px > S.cap_px || words > S.cap_words || list > S.cap_list) {
+    // make sure nothing is in flight on the buffers we are about to free (the pipelines' chunks
+    // run on the caller's and the sparse stream: their last work on the set is S.done)
     AG_CUDA(det, cudaStreamSynchronize(S.stream));
-    if ((rc = regrow(det, &S.d_blur, (size_t)F * px))) return rc;
-    if ((rc = regrow(det, &S.d_resp, (size_t)F * px))) return rc;
+    AG_CUDA(det, cudaEventSynchronize(S.done));
+    S.cap_px = std::max(px, S.cap_px);
+    S.cap_words = std::max(words, S.cap_words);
+    S.cap_list = std::max(list, S.cap_list);
+    if ((rc = regrow(det, &S.d_blur, S.cap_px))) return rc;
+    if ((rc = regrow(det, &S.d_resp, S.cap_px))) return rc;
     // per-pixel union-find parents: only the labels tap needs them kept; the labelling kernels
     // that want per-pixel scratch otherwise use the response buffer, which is dead after K2
     if (S.d_parent) { AG_CUDA(det, cudaFree(S.d_parent)); S.d_parent = nullptr; }
-    if ((rc = regrow(det, &S.d_mask, (size_t)F * words))) return rc;
-    // the saddle mask is 1-4 % full; a list of 1/8 of the pixels covers every real image, fuller
-    // masks (noise) take the word-oriented labelling path
-    S.pix_cap = (int)std::min<size_t>(std::max<size_t>(px / 8, 32768), (size_t)1 << 20);
-    if ((rc = regrow(det, &S.d_pixlist, (size_t)F * S.pix_cap))) return rc;
-    S.cap_px = px;
-    S.cap_words = words;
+    if ((rc = regrow(det, &S.d_mask, S.cap_words))) return rc;
+    if ((rc = regrow(det, &S.d_pixlist, S.cap_list))) return rc;
   }
-  const int ncl = det->cur_clusters, nsd = det->cur_saddles;
-  if (grow_frames || ncl != S.cap_clusters || nsd != S.cap_saddles) {
+  S.pix_cap = pix_cap;
+  const int ncl = det->cur_clusters;
+  const size_t cl = (size_t)frames * ncl;
+  if (frames > S.cap_frames || cl > S.cap_cl) {
     AG_CUDA(det, cudaStreamSynchronize(S.stream));
-    if ((rc = regrow(det, &S.d_min, (size_t)F))) return rc;
-    if ((rc = regrow(det, &S.d_ncl, (size_t)F))) return rc;
-    if ((rc = regrow(det, &S.d_label_fallback, (size_t)F))) return rc;
-    if ((rc = regrow(det, &S.d_acc, (size_t)F * ncl * 3))) return rc;
-    if ((rc = regrow(det, &S.d_centers, (size_t)F * ncl))) return rc;
-    if ((rc = regrow(det, &S.d_raw, (size_t)F * ncl))) return rc;
-    if ((rc = regrow(det, &S.d_raw_valid, (size_t)F * ncl))) return rc;
-    S.cap_clusters = ncl;
-    S.cap_saddles = nsd;
+    AG_CUDA(det, cudaEventSynchronize(S.done));
+    S.cap_frames = std::max(frames, S.cap_frames);
+    S.cap_cl = std::max(cl, S.cap_cl);
+    if ((rc = regrow(det, &S.d_min, (size_t)S.cap_frames))) return rc;
+    if ((rc = regrow(det, &S.d_ncl, (size_t)S.cap_frames))) return rc;
+    if ((rc = regrow(det, &S.d_label_fallback, (size_t)S.cap_frames))) return rc;
+    if ((rc = regrow(det, &S.d_acc, S.cap_cl * 3))) return rc;
+    if ((rc = regrow(det, &S.d_centers, S.cap_cl))) return rc;
+    if ((rc = regrow(det, &S.d_raw, S.cap_cl))) return rc;
+    if ((rc = regrow(det, &S.d_raw_valid, S.cap_cl))) return rc;
   }
+  S.cap_clusters = ncl;
   if (need_parent && !S.d_parent) {
     AG_CUDA(det, cudaStreamSynchronize(S.stream));
-    if ((rc = regrow(det, &S.d_parent, (size_t)F * px))) return rc;
+    AG_CUDA(det, cudaEventSynchronize(S.done));
+    if ((rc = regrow(det, &S.d_parent, S.cap_px))) return rc;
   }
-  S.cap_frames = F;
   return AG_OK;
 }
 
@@ -434,6 +455,7 @@ void free_slot(Slot& S) {
   cudaFree(S.d_raw_valid); cudaFree(S.d_pixlist); cudaFree(S.d_label_fallback);
   free_board_slot(S.bb);
   if (S.done) cudaEventDestroy(S.done);
+  if (S.ev_dense) cudaEventDestroy(S.ev_dense);
   if (S.stream) cudaStreamDestroy(S.stream);
   S = Slot();
 }
@@ -540,6 +562,38 @@ int run_sparse(ag_detector* det, Slot& S, BoardSlot& B, const FrameGeom& g, int 
                                         B.d_nref, d_status, s);
   prof_mark(det, 3, s);
   AG_CUDA(det, cudaGetLastError());
+  return AG_OK;
+}
+
+// Both sets of the pipelines' dense ring, for chunks of `frames` frames, and the sparse stream.
+int ensure_ring(ag_detector* det, const FrameGeom& g, int frames) {
+  int rc;
+  for (auto& D : det->dense)
+    if ((rc = ensure_slot(det, D, g, frames, false))) return rc;
+  if (!det->sparse_stream) AG_CUDA(det, cudaStreamCreateWithFlags(&det->sparse_stream, cudaStreamNonBlocking));
+  return AG_OK;
+}
+
+// Front end of one pipeline chunk into the next set of the dense ring: K1-K2 on the dense stream
+// s, then K3-K4 on the sparse stream into board slot B; B.ev_front marks the refined saddles
+// ready.  The set is reused only after the sparse stages of its previous chunk (which read its
+// blur and use its response buffer as scratch), and B only after its previous board search (K4
+// writes B's saddle list).  Ordering through the set's events also holds when consecutive calls
+// come on different streams.
+int run_front(ag_detector* det, BoardSlot& B, const uint8_t* d_frames, const FrameGeom& g, int n,
+              uint32_t* d_status, cudaStream_t s) {
+  int rc;
+  Slot& D = det->dense[det->dense_rr];
+  det->dense_rr = (det->dense_rr + 1) % kDenseSets;
+  const cudaStream_t sp = det->sparse_stream;
+  AG_CUDA(det, cudaStreamWaitEvent(s, D.done, 0));
+  if ((rc = run_dense(det, D, d_frames, g, n, true, s))) return rc;
+  AG_CUDA(det, cudaEventRecord(D.ev_dense, s));
+  AG_CUDA(det, cudaStreamWaitEvent(sp, D.ev_dense, 0));
+  if (B.pending) AG_CUDA(det, cudaStreamWaitEvent(sp, B.ev_boards, 0));
+  if ((rc = run_sparse(det, D, B, g, n, d_status, sp))) return rc;
+  AG_CUDA(det, cudaEventRecord(D.done, sp));
+  AG_CUDA(det, cudaEventRecord(B.ev_front, sp));
   return AG_OK;
 }
 
@@ -720,7 +774,8 @@ int quiesce_device_path(ag_detector* det, bool host_too) {
     if (rc) return rc;
   }
   if (!det->device_path_busy) return AG_OK;
-  if (det->dense.done) AG_CUDA(det, cudaEventSynchronize(det->dense.done));
+  for (auto& D : det->dense)
+    if (D.done) AG_CUDA(det, cudaEventSynchronize(D.done));
   for (auto& B : det->bslot)
     if (B.pending) {
       AG_CUDA(det, cudaEventSynchronize(B.ev_boards));
@@ -888,7 +943,8 @@ void ag_destroy(ag_detector* det) {
   if (!det) return;
   cudaSetDevice(det->device);
   cudaDeviceSynchronize();
-  free_slot(det->dense);
+  for (auto& D : det->dense) free_slot(D);
+  if (det->sparse_stream) cudaStreamDestroy(det->sparse_stream);
   free_slot(det->big);
   for (auto& B : det->bslot) free_board_slot(B);
   if (det->up_stream) cudaStreamDestroy(det->up_stream);
@@ -1009,21 +1065,16 @@ int ag_detect_batch_device(ag_detector* det, const void* d_frames, size_t frame_
   if ((rc = collect_host(det, det->host_seq))) return rc;
   set_caps(det, g);
   const int chunk = chunk_limit(det, g, std::min<long>(det->chunk_frames, std::max(n_frames, 1)));
-  // One set of dense buffers (K1-K4 of consecutive chunks are serial on stream s anyway),
+  // The ring of dense sets (K1-K2 on stream s, K3-K4 on the sparse stream, see run_front),
   // kBoardSlots board-search sides: chunk i's K6 runs on its board slot's own stream, so the
   // searches of up to kBoardSlots chunks (of this call and of earlier calls) overlap each other
-  // and the front end of the following chunks.  A board slot is reused only after its kernel has
-  // finished (K4 of the new chunk writes the slot's saddle list).
-  Slot& D = det->dense;
-  if ((rc = ensure_slot(det, D, g, chunk, false))) return rc;
-  cudaStream_t s = stream ? (cudaStream_t)stream : D.stream;
+  // and the front end of the following chunks.
+  if ((rc = ensure_ring(det, g, chunk))) return rc;
+  cudaStream_t s = stream ? (cudaStream_t)stream : det->dense[0].stream;
   // all board slots are sized up front: an allocation (which synchronises the device) must not
   // happen in the middle of a streaming sequence of calls
   for (auto& B : det->bslot)
     if ((rc = ensure_board_slot(det, B, chunk, false))) return rc;
-  // the dense buffers are shared by every device-batch call: order this call after the front end
-  // of the previous one even if the caller switched streams
-  if (det->device_path_busy) AG_CUDA(det, cudaStreamWaitEvent(s, D.done, 0));
   for (int f0 = 0; f0 < n_frames; f0 += chunk) {
     BoardSlot& B = det->bslot[det->slot_rr];
     det->slot_rr = (det->slot_rr + 1) % kBoardSlots;
@@ -1031,10 +1082,7 @@ int ag_detect_batch_device(ag_detector* det, const void* d_frames, size_t frame_
     const int n = std::min(chunk, n_frames - f0);
     const uint8_t* in = (const uint8_t*)d_frames + (size_t)f0 * g.frame_stride;
     uint32_t* st = d_frame_status ? d_frame_status + f0 : B.d_status;
-    if (B.pending) AG_CUDA(det, cudaStreamWaitEvent(s, B.ev_boards, 0));
-    if ((rc = run_dense(det, D, in, g, n, true, s))) return rc;
-    if ((rc = run_sparse(det, D, B, g, n, st, s))) return rc;
-    AG_CUDA(det, cudaEventRecord(B.ev_front, s));
+    if ((rc = run_front(det, B, in, g, n, st, s))) return rc;
     AG_CUDA(det, cudaStreamWaitEvent(B.bstream, B.ev_front, 0));
     if ((rc = run_boards(det, B, in, g, n, d_out + (size_t)f0 * cap_per_frame, cap_per_frame,
                          d_n_per_frame + f0, st, false, B.bstream)))
@@ -1042,7 +1090,6 @@ int ag_detect_batch_device(ag_detector* det, const void* d_frames, size_t frame_
     AG_CUDA(det, cudaEventRecord(B.ev_boards, B.bstream));
     B.pending = true;
   }
-  AG_CUDA(det, cudaEventRecord(D.done, s));
   det->device_path_busy = true;
   // results become visible in the caller's stream order (unless the caller asked to do that
   // itself with ag_detect_batch_device_wait, which lets consecutive calls overlap)
@@ -1076,7 +1123,7 @@ int ag_dense_batch_device(ag_detector* det, const void* d_frames, size_t frame_s
   if (rc) return rc;
   if ((uintptr_t)d_frames % channel_align(format))
     return fail(det, AG_ERR_INVALID, "device frames must start at a multiple of the format's channel word");
-  Slot& S = det->dense;
+  Slot& S = det->dense[0];
   set_caps(det, g);
   const int chunk = chunk_limit(det, g, std::min<long>(det->chunk_frames, std::max(n_frames, 1)));
   if ((rc = ensure_slot(det, S, g, chunk, false))) return rc;
@@ -1111,17 +1158,17 @@ static int detect_batch_host(ag_detector* det, const void* frames, size_t frame_
   const uint64_t seq = ++det->host_seq;
   if (n_frames == 0) return async_call ? AG_OK : host_call_verdict(det);
   set_caps(det, g);
-  // Host frames go through the same pipeline as device-resident ones: one set of dense buffers,
-  // eight board slots.  A chunk is uploaded on the upload stream (ahead of the kernels), K1-K4
-  // run on the dense stream, K6 and the download of the results on the board slot's stream, so
-  // uploads, front end, board searches and downloads of up to eight chunks overlap.  The staged
-  // input of a chunk stays in its board slot until K6 (which samples the tag bits) is done.
+  // Host frames go through the same pipeline as device-resident ones: the ring of dense sets,
+  // eight board slots.  A chunk is uploaded on the upload stream (ahead of the kernels), K1-K2
+  // run on the dense stream, K3-K4 on the sparse stream, K6 and the download of the results on
+  // the board slot's stream, so uploads, front end, board searches and downloads of up to eight
+  // chunks overlap.  The staged input of a chunk stays in its board slot until K6 (which samples
+  // the tag bits) is done.
   const int chunk = chunk_limit(
       det, g, std::min<long>(std::min<long>(det->chunk_frames, host_chunk_for(det->host_chunk_frames, format)), n_frames));
-  Slot& D = det->dense;
-  if ((rc = ensure_slot(det, D, g, chunk, false))) return rc;
+  if ((rc = ensure_ring(det, g, chunk))) return rc;
   if (!det->up_stream) AG_CUDA(det, cudaStreamCreateWithFlags(&det->up_stream, cudaStreamNonBlocking));
-  cudaStream_t s = D.stream, up = det->up_stream;
+  cudaStream_t s = det->dense[0].stream, up = det->up_stream;
   const size_t chunk_bytes = (size_t)chunk * g.frame_stride;
   const bool pageable = is_pageable(frames);
   // Chunk schedule: the pipeline fills while the first chunk uploads and drains while the last one
@@ -1163,9 +1210,7 @@ static int detect_batch_host(ag_detector* det, const void* frames, size_t frame_
     AG_CUDA(det, cudaMemcpyAsync(B.d_in, up_src, bytes, cudaMemcpyHostToDevice, up));
     AG_CUDA(det, cudaEventRecord(B.ev_up, up));
     AG_CUDA(det, cudaStreamWaitEvent(s, B.ev_up, 0));
-    if ((rc = run_dense(det, D, B.d_in, g, n, true, s))) return rc;
-    if ((rc = run_sparse(det, D, B, g, n, B.d_status, s))) return rc;
-    AG_CUDA(det, cudaEventRecord(B.ev_front, s));
+    if ((rc = run_front(det, B, B.d_in, g, n, B.d_status, s))) return rc;
     AG_CUDA(det, cudaStreamWaitEvent(B.bstream, B.ev_front, 0));
     if ((rc = run_boards(det, B, B.d_in, g, n, B.d_tags, B.hs_tags, B.d_ntags, B.d_status, false, B.bstream)))
       return rc;
@@ -1193,7 +1238,6 @@ static int detect_batch_host(ag_detector* det, const void* frames, size_t frame_
   }
   // (a later device-batch call first collects these chunks -- it blocks until they are done -- so
   // the host path needs no busy flag of its own; streaming host calls must not drain each other)
-  AG_CUDA(det, cudaEventRecord(D.done, s));
   if (async_call) return AG_OK;  // results are collected by later calls / ag_detect_batch_wait
   if ((rc = collect_host(det, seq))) return rc;
   return host_call_verdict(det);
@@ -1468,7 +1512,7 @@ int ag_gaussian_blur_f32(ag_detector* det, const float* img, int width, int heig
   const size_t n = (size_t)width * height;
   int rc = ensure_f32(det, n);
   if (rc) return rc;
-  Slot& S = det->dense;
+  Slot& S = det->dense[0];
   if (!S.stream) {
     AG_CUDA(det, cudaStreamCreateWithFlags(&S.stream, cudaStreamNonBlocking));
     AG_CUDA(det, cudaEventCreateWithFlags(&S.done, cudaEventDisableTiming));
@@ -1516,7 +1560,7 @@ int ag_hessian_response(ag_detector* det, const float* img, int width, int heigh
   const size_t n = (size_t)width * height;
   int rc = ensure_f32(det, n);
   if (rc) return rc;
-  Slot& S = det->dense;
+  Slot& S = det->dense[0];
   if (!S.stream) {
     AG_CUDA(det, cudaStreamCreateWithFlags(&S.stream, cudaStreamNonBlocking));
     AG_CUDA(det, cudaEventCreateWithFlags(&S.done, cudaEventDisableTiming));
