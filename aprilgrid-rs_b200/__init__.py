@@ -105,6 +105,8 @@ def lib():
         L.ag_detect_batch_wait.argtypes = [vp, ci]
         L.ag_dense_batch_device.argtypes = [vp, vp, sz, ci, ci, ci, sz, ci, vp]
         L.ag_refined_saddle_points.argtypes = [vp, vp, ci, ci, sz, ci, vp, ci, vp]
+        L.ag_refined_saddle_points_batch.argtypes = [vp, vp, sz, ci, ci, ci, sz, ci, vp, ci, vp, vp]
+        L.ag_refined_saddle_points_batch_device.argtypes = [vp, vp, sz, ci, ci, ci, sz, ci, vp, ci, vp, vp, vp]
         L.ag_gaussian_blur_f32.argtypes = [vp, vp, ci, ci, C.c_float, vp]
         L.ag_hessian_response.argtypes = [vp, vp, ci, ci, vp]
         L.ag_gaussian_blur_f32_device.argtypes = [vp, vp, ci, ci, ci, C.c_float, vp, vp]
@@ -130,6 +132,7 @@ def lib():
         L.ag_multi_last_error.argtypes = [vp]
         L.ag_multi_set_option.argtypes = [vp, C.c_char_p, C.c_long]
         L.ag_multi_detect_batch.argtypes = [vp, vp, sz, ci, ci, ci, sz, ci, vp, ci, vp, vp]
+        L.ag_multi_refined_saddle_points_batch.argtypes = [vp, vp, sz, ci, ci, ci, sz, ci, vp, ci, vp, vp]
         L.ag_test_unorm_tables.argtypes = [vp, vp, vp, vp, vp]
         L.ag_test_board_times.argtypes = [vp, ci, vp, ci]
         L.ag_test_board_layout.argtypes = [ci, ci, ci, ci, ci, ci, vp]
@@ -316,6 +319,37 @@ class TagDetector:
         n = C.c_int(0)
         self._check(lib().ag_refined_saddle_points(self._h, _p(img), w, h, st, fmt, _p(out), cap, C.byref(n)))
         return out[:n.value].copy()
+
+    def refined_saddle_points_batch(self, frames, cap_per_frame=2048, return_status=False):
+        """refined_saddle_points of every frame of a batch (N x H x W[...] as detect_batch) -> list of
+        structured Saddle arrays, each byte-identical to refined_saddle_points of that frame."""
+        frames = np.ascontiguousarray(frames)
+        n = frames.shape[0]
+        out = np.zeros((n, cap_per_frame), SADDLE_DTYPE)
+        cnt = np.zeros(n, np.int32)
+        status = np.zeros(n, np.uint32)
+        if n:
+            self.refined_saddle_points_batch_into(frames, out, cnt, status)
+        res = [out[i, :cnt[i]].copy() for i in range(n)]
+        return (res, status) if return_status else res
+
+    def refined_saddle_points_batch_into(self, frames, out, cnt, status=None):
+        """refined_saddle_points_batch writing into caller-provided arrays (out: N x cap SADDLE_DTYPE,
+        cnt: N int32, status: N uint32 or None); synchronous."""
+        n = frames.shape[0]
+        fmt, w, h, st = image_format(frames[0])
+        return self._check(lib().ag_refined_saddle_points_batch(self._h, _p(frames), frames.strides[0], n, w, h, st,
+                                                                fmt, _p(out), out.shape[1], _p(cnt), _p(status)))
+
+    def refined_saddle_points_batch_device(self, d_frames_ptr, n_frames, width, height, fmt, d_out_ptr, cap_per_frame,
+                                           d_counts_ptr, d_status_ptr=None, stream=None, frame_stride=0,
+                                           row_stride=0):
+        """Device-resident frames, device-resident saddles (d_out: n_frames x cap_per_frame records of
+        SADDLE_DTYPE), asynchronous on `stream` (raw pointers); as detect_batch_device."""
+        return self._check(lib().ag_refined_saddle_points_batch_device(
+            self._h, C.c_void_p(d_frames_ptr), frame_stride, n_frames, width, height, row_stride, fmt,
+            C.c_void_p(d_out_ptr), cap_per_frame, C.c_void_p(d_counts_ptr),
+            C.c_void_p(d_status_ptr) if d_status_ptr else None, C.c_void_p(stream) if stream else None))
 
     def gaussian_blur_f32(self, img, sigma=1.5):
         """image_util::gaussian_blur_f32 (image_util.rs:110-206)."""
@@ -527,6 +561,21 @@ class MultiTagDetector:
         if n:
             self.detect_batch_into(frames, out, cnt, status)
         return [_tags_to_dict(out[i, :cnt[i]]) for i in range(n)]
+
+    def refined_saddle_points_batch(self, frames, cap_per_frame=2048):
+        """TagDetector.refined_saddle_points_batch over every device; byte-identical to one device."""
+        frames = np.ascontiguousarray(frames)
+        n = frames.shape[0]
+        out = np.zeros((n, cap_per_frame), SADDLE_DTYPE)
+        cnt = np.zeros(n, np.int32)
+        status = np.zeros(n, np.uint32)
+        if n:
+            fmt, w, h, st = image_format(frames[0])
+            rc = lib().ag_multi_refined_saddle_points_batch(self._h, _p(frames), frames.strides[0], n, w, h, st, fmt,
+                                                            _p(out), cap_per_frame, _p(cnt), _p(status))
+            if rc != AG_OK:
+                raise RuntimeError("aprilgrid_b200 error %d: %s" % (rc, lib().ag_multi_last_error(self._h).decode()))
+        return [out[i, :cnt[i]].copy() for i in range(n)]
 
 
 def saddles_as_array(s):

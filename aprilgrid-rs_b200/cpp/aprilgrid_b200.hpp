@@ -7,6 +7,7 @@
 //   detect(image)            -> std::unordered_map<uint32_t, std::array<std::pair<float,float>,4>>
 //   detect_batch(frames...)  -> vector of such maps (new entry point)
 //   refined_saddle_points(image) -> std::vector<Saddle>
+//   refined_saddle_points_batch(frames...) -> vector of such lists (new entry point)
 #pragma once
 #include <array>
 #include <optional>
@@ -105,12 +106,29 @@ class TagDetector {
     int n = 0;
     check(ag_refined_saddle_points(h_, img.pixels, img.width, img.height, img.row_stride, img.format, out.data(),
                                    (int)out.size(), &n));
-    std::vector<Saddle> r(n);
-    for (int i = 0; i < n; ++i) r[i] = Saddle{{out[i].x, out[i].y}, out[i].k, out[i].theta, out[i].phi};
-    return r;
+    return to_saddles(out.data(), n);
+  }
+
+  // frames: n_frames images of one shape, frame i at base + i * frame_stride
+  std::vector<std::vector<Saddle>> refined_saddle_points_batch(const void* base, size_t frame_stride, int n_frames,
+                                                               int width, int height, size_t row_stride, int format,
+                                                               int cap_per_frame = 2048) const {
+    std::vector<ag_saddle> out((size_t)n_frames * cap_per_frame);
+    std::vector<int> cnt(n_frames);
+    check(ag_refined_saddle_points_batch(h_, base, frame_stride, n_frames, width, height, row_stride, format,
+                                         out.data(), cap_per_frame, cnt.data(), nullptr));
+    std::vector<std::vector<Saddle>> res(n_frames);
+    for (int i = 0; i < n_frames; ++i) res[i] = to_saddles(out.data() + (size_t)i * cap_per_frame, cnt[i]);
+    return res;
   }
 
   ag_detector* handle() const { return h_; }
+
+  static std::vector<Saddle> to_saddles(const ag_saddle* s, int n) {
+    std::vector<Saddle> r(n);
+    for (int i = 0; i < n; ++i) r[i] = Saddle{{s[i].x, s[i].y}, s[i].k, s[i].theta, s[i].phi};
+    return r;
+  }
 
  private:
   void check(int rc) const {
@@ -156,6 +174,20 @@ class MultiTagDetector {
         m[t[k].id] = {{{t[k].xy[0], t[k].xy[1]}, {t[k].xy[2], t[k].xy[3]}, {t[k].xy[4], t[k].xy[5]}, {t[k].xy[6], t[k].xy[7]}}};
       res[i] = std::move(m);
     }
+    return res;
+  }
+
+  std::vector<std::vector<Saddle>> refined_saddle_points_batch(const void* base, size_t frame_stride, int n_frames,
+                                                               int width, int height, size_t row_stride, int format,
+                                                               int cap_per_frame = 2048) const {
+    std::vector<ag_saddle> out((size_t)n_frames * cap_per_frame);
+    std::vector<int> cnt(n_frames);
+    if (ag_multi_refined_saddle_points_batch(m_, base, frame_stride, n_frames, width, height, row_stride, format,
+                                             out.data(), cap_per_frame, cnt.data(), nullptr) != AG_OK)
+      throw std::runtime_error(std::string("aprilgrid_b200: ") + ag_multi_last_error(m_));
+    std::vector<std::vector<Saddle>> res(n_frames);
+    for (int i = 0; i < n_frames; ++i)
+      res[i] = TagDetector::to_saddles(out.data() + (size_t)i * cap_per_frame, cnt[i]);
     return res;
   }
 

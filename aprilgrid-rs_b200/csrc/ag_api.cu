@@ -60,6 +60,10 @@ constexpr int kBigTierBatchWarps = AG_BIG_TIER_WARPS;
 constexpr int kSingleFrameWarps = AG_SINGLE_WARPS;  // warps per frame when a launch holds only a few frames
 constexpr size_t kMaxBlockSmem = 227 * 1024;       // dynamic shared memory a block may ask for on sm_100  // warps per frame of the 4096-tier batch launch
 
+// What a batch call hands back per frame: tags (detect) or the refined saddles K4 found
+// (refined_saddle_points; the board search is skipped).
+enum class ResultKind { kTags, kSaddles };
+
 // Board-search side of a chunk: what K4 hands to K6, K6's workspace, its stream and events.
 // A few hundred KB per frame, so many of these can be in flight (see kBoardSlots).
 struct BoardSlot {
@@ -90,8 +94,13 @@ struct BoardSlot {
   ag_tag* d_tags = nullptr;
   int* d_ntags = nullptr;
   ag_tag* h_tags = nullptr;
-  int* h_ntags = nullptr;
+  int* h_ntags = nullptr;  // (also the saddle counts of a saddle chunk)
   uint32_t* h_status = nullptr;
+  // saddle chunks of the host-frame path: the records in the caller's layout, per-frame stride
+  // min(cap_per_frame, cap_saddles); capacity in records
+  ag_saddle* d_sad = nullptr;
+  ag_saddle* h_sad = nullptr;
+  size_t cap_sad = 0;
   cudaEvent_t ev_up = nullptr, ev_done = nullptr;  // upload done / results on the host
 };
 
@@ -141,9 +150,12 @@ struct ag_detector {
   // output arrays of the ag_detect_batch call they belong to (calls may overlap: "host_async")
   struct HostPend {
     bool live = false;
+    ResultKind kind = ResultKind::kTags;
     int f0 = 0, n = 0, cap = 0;
+    int sad_stride = 0;  // saddle chunks: records per frame in the slot's staging
     uint64_t seq = 0;
     ag_tag* out = nullptr;
+    ag_saddle* sad_out = nullptr;
     int* n_per_frame = nullptr;
     uint32_t* status = nullptr;
     const uint8_t* src = nullptr;  // host frames of the chunk (re-run of overflowed frames)
@@ -343,8 +355,8 @@ int ensure_board_slot(ag_detector* det, BoardSlot& B, int frames, bool drain) {
 }
 
 // Host-frame staging of a board slot: `frames` frames of `in_bytes_per_chunk` bytes in total,
-// `cap_tags` result records per frame.
-int ensure_host_stage(ag_detector* det, BoardSlot& B, size_t in_bytes, int frames, int cap_tags) {
+// `cap_tags` tag records and `sad_stride` saddle records per frame.
+int ensure_host_stage(ag_detector* det, BoardSlot& B, size_t in_bytes, int frames, int cap_tags, int sad_stride = 0) {
   int rc;
   if (!B.ev_up) {
     AG_CUDA(det, cudaEventCreateWithFlags(&B.ev_up, cudaEventDisableTiming));
@@ -367,12 +379,22 @@ int ensure_host_stage(ag_detector* det, BoardSlot& B, size_t in_bytes, int frame
     B.hs_frames = F;
     B.hs_tags = ct;
   }
+  const size_t sad = (size_t)frames * sad_stride;
+  if (sad > B.cap_sad) {
+    if ((rc = regrow(det, &B.d_sad, sad))) return rc;
+    if (B.h_sad) cudaFreeHost(B.h_sad);
+    B.h_sad = nullptr;
+    B.cap_sad = 0;
+    AG_CUDA(det, cudaMallocHost((void**)&B.h_sad, sizeof(ag_saddle) * sad));
+    B.cap_sad = sad;
+  }
   return AG_OK;
 }
 
 void free_board_slot(BoardSlot& B) {
-  cudaFree(B.d_in); cudaFree(B.d_tags); cudaFree(B.d_ntags);
+  cudaFree(B.d_in); cudaFree(B.d_tags); cudaFree(B.d_ntags); cudaFree(B.d_sad);
   if (B.h_in) cudaFreeHost(B.h_in);
+  if (B.h_sad) cudaFreeHost(B.h_sad);
   if (B.h_tags) cudaFreeHost(B.h_tags);
   if (B.h_ntags) cudaFreeHost(B.h_ntags);
   if (B.h_status) cudaFreeHost(B.h_status);
@@ -639,6 +661,29 @@ int run_boards(ag_detector* det, BoardSlot& S, const uint8_t* d_frames, const Fr
   return AG_OK;
 }
 
+// Back end of a pipeline chunk on board slot B's stream, once its front end is done (B.ev_front):
+// the board search into d_out (tags), or the copy of K4's saddle lists into d_out's layout
+// (saddles; out_stride records per frame).  Either way B.ev_boards then marks B free for the next
+// chunk's K4, so slot reuse, the streaming waits and the quiesce cover both kinds alike.
+int run_back(ag_detector* det, BoardSlot& B, ResultKind kind, const uint8_t* d_frames, const FrameGeom& g, int n,
+             void* d_out, int out_stride, int cap, int* d_n, uint32_t* d_status) {
+  const cudaStream_t s = B.bstream;
+  AG_CUDA(det, cudaStreamWaitEvent(s, B.ev_front, 0));
+  if (kind == ResultKind::kTags) {
+    const int rc = run_boards(det, B, d_frames, g, n, (ag_tag*)d_out, cap, d_n, d_status, false, s);
+    if (rc) return rc;
+  } else {
+    prof_mark(det, -1, s);  // (accounted to stage 3: the copy finishes the refined saddle list)
+    det->launches += launch_saddles_out(B.d_refined, B.cap_saddles, B.d_nref, d_status, n, (ag_saddle*)d_out,
+                                        out_stride, cap, d_n, s);
+    prof_mark(det, 3, s);
+    AG_CUDA(det, cudaGetLastError());
+  }
+  AG_CUDA(det, cudaEventRecord(B.ev_boards, s));
+  B.pending = true;
+  return AG_OK;
+}
+
 constexpr uint32_t kGrowable = AG_FRAME_CLUSTER_OVERFLOW | AG_FRAME_SADDLE_OVERFLOW;
 
 // What run_one_frame runs after K1-K4: K6, nothing (the refined saddles are the result), or K6
@@ -714,6 +759,8 @@ int run_one_frame(ag_detector* det, const FrameGeom& g, const FrameGeom& gb, siz
 
 void copy_out_b(const BoardSlot& B, int n, int cap, ag_tag* out, int* n_per_frame, uint32_t* frame_status,
                 int frame0, bool* truncated);
+void copy_out_saddles(const BoardSlot& B, int n, int cap, int stride, ag_saddle* out, int* n_per_frame,
+                      uint32_t* frame_status, int frame0, bool* truncated);
 
 // Host-buffer path: wait for the chunk staged in board slot bi and hand its results to the output
 // arrays of the call that submitted it.  A frame that overflowed max_clusters / max_saddles was
@@ -724,7 +771,11 @@ int collect_host_slot(ag_detector* det, int bi) {
   if (!P.live) return AG_OK;
   BoardSlot& B = det->bslot[bi];
   AG_CUDA(det, cudaEventSynchronize(B.ev_done));
-  copy_out_b(B, P.n, P.cap, P.out, P.n_per_frame, P.status, P.f0, &det->host_truncated);
+  const bool saddles = P.kind == ResultKind::kSaddles;
+  if (saddles)
+    copy_out_saddles(B, P.n, P.cap, P.sad_stride, P.sad_out, P.n_per_frame, P.status, P.f0, &det->host_truncated);
+  else
+    copy_out_b(B, P.n, P.cap, P.out, P.n_per_frame, P.status, P.f0, &det->host_truncated);
   P.live = false;
   B.pending = false;
   for (int i = 0; i < P.n; ++i) {
@@ -738,11 +789,18 @@ int collect_host_slot(ag_detector* det, int bi) {
       };
       int cnt = 0;
       uint32_t st2 = 0;
-      int rc = run_one_frame(det, g, g, 0, upload, FrameRun::kTags, st, &cnt, &st2);
+      int rc = run_one_frame(det, g, g, 0, upload, saddles ? FrameRun::kSaddles : FrameRun::kTags, st, &cnt, &st2);
       if (rc) return rc;
       const BoardSlot& R = det->big.bb;
-      memcpy(P.out + (size_t)(P.f0 + i) * P.cap, R.h_tags,
-             sizeof(ag_tag) * (size_t)std::min(std::min(cnt, P.cap), R.hs_tags));
+      const int m = std::min(cnt, P.cap);
+      if (saddles) {
+        // (a frame still beyond the limits keeps the list it has there, as ag_refined_saddle_points gives it)
+        if (m > 0)
+          AG_CUDA(det, cudaMemcpy(P.sad_out + (size_t)(P.f0 + i) * P.cap, R.d_refined, sizeof(ag_saddle) * m,
+                                  cudaMemcpyDeviceToHost));
+      } else {
+        memcpy(P.out + (size_t)(P.f0 + i) * P.cap, R.h_tags, sizeof(ag_tag) * (size_t)std::min(m, R.hs_tags));
+      }
       if (cnt > P.cap) {
         st2 |= AG_FRAME_TAG_OVERFLOW;
         det->host_truncated = true;
@@ -829,6 +887,19 @@ void copy_out_b(const BoardSlot& B, int n, int cap, ag_tag* out, int* n_per_fram
     if (cnt > cap) *truncated = true;
     const int m = std::min(cnt, cap);
     memcpy(out + (size_t)(frame0 + i) * cap, B.h_tags + (size_t)i * B.hs_tags, sizeof(ag_tag) * m);
+    if (frame_status) frame_status[frame0 + i] = B.h_status[i];
+  }
+}
+
+// ... of a saddle chunk: counts, status bits (with AG_FRAME_TAG_OVERFLOW) and records as
+// k_saddles_out left them, `stride` records per frame.
+void copy_out_saddles(const BoardSlot& B, int n, int cap, int stride, ag_saddle* out, int* n_per_frame,
+                      uint32_t* frame_status, int frame0, bool* truncated) {
+  for (int i = 0; i < n; ++i) {
+    const int cnt = B.h_ntags[i];
+    n_per_frame[frame0 + i] = cnt;
+    if (cnt > cap) *truncated = true;
+    memcpy(out + (size_t)(frame0 + i) * cap, B.h_sad + (size_t)i * stride, sizeof(ag_saddle) * std::min(cnt, cap));
     if (frame_status) frame_status[frame0 + i] = B.h_status[i];
   }
 }
@@ -1046,10 +1117,11 @@ int ag_stage_times(ag_detector* det, double* ms_out, uint64_t* n_out, int reset)
   return AG_OK;
 }
 
-int ag_detect_batch_device(ag_detector* det, const void* d_frames, size_t frame_stride, int n_frames,
-                           int width, int height, size_t row_stride, int format, ag_tag* d_out,
-                           int cap_per_frame, int* d_n_per_frame, uint32_t* d_frame_status,
-                           void* stream) {
+// ag_detect_batch_device and ag_refined_saddle_points_batch_device: the device-batch pipeline, whose
+// chunks end in the board search (tags) or in the copy of the refined saddles (saddles, see run_back).
+static int batch_device(ag_detector* det, ResultKind kind, const void* d_frames, size_t frame_stride, int n_frames,
+                        int width, int height, size_t row_stride, int format, void* d_out, int cap_per_frame,
+                        int* d_n_per_frame, uint32_t* d_frame_status, void* stream) {
   if (!det) return AG_ERR_INVALID;
   if (!d_frames || !d_out || !d_n_per_frame || n_frames < 0 || cap_per_frame < 1)
     return fail(det, AG_ERR_INVALID, "null pointer or bad count");
@@ -1082,13 +1154,11 @@ int ag_detect_batch_device(ag_detector* det, const void* d_frames, size_t frame_
     const int n = std::min(chunk, n_frames - f0);
     const uint8_t* in = (const uint8_t*)d_frames + (size_t)f0 * g.frame_stride;
     uint32_t* st = d_frame_status ? d_frame_status + f0 : B.d_status;
-    if ((rc = run_front(det, B, in, g, n, st, s))) return rc;
-    AG_CUDA(det, cudaStreamWaitEvent(B.bstream, B.ev_front, 0));
-    if ((rc = run_boards(det, B, in, g, n, d_out + (size_t)f0 * cap_per_frame, cap_per_frame,
-                         d_n_per_frame + f0, st, false, B.bstream)))
+    const size_t rec = kind == ResultKind::kTags ? sizeof(ag_tag) : sizeof(ag_saddle);
+    if ((rc = run_front(det, B, in, g, n, st, s)) ||
+        (rc = run_back(det, B, kind, in, g, n, (uint8_t*)d_out + (size_t)f0 * cap_per_frame * rec, cap_per_frame,
+                       cap_per_frame, d_n_per_frame + f0, st)))
       return rc;
-    AG_CUDA(det, cudaEventRecord(B.ev_boards, B.bstream));
-    B.pending = true;
   }
   det->device_path_busy = true;
   // results become visible in the caller's stream order (unless the caller asked to do that
@@ -1097,6 +1167,22 @@ int ag_detect_batch_device(ag_detector* det, const void* d_frames, size_t frame_
     for (auto& B : det->bslot)
       if (B.pending) AG_CUDA(det, cudaStreamWaitEvent(s, B.ev_boards, 0));
   return AG_OK;
+}
+
+int ag_detect_batch_device(ag_detector* det, const void* d_frames, size_t frame_stride, int n_frames,
+                           int width, int height, size_t row_stride, int format, ag_tag* d_out,
+                           int cap_per_frame, int* d_n_per_frame, uint32_t* d_frame_status,
+                           void* stream) {
+  return batch_device(det, ResultKind::kTags, d_frames, frame_stride, n_frames, width, height, row_stride, format,
+                      d_out, cap_per_frame, d_n_per_frame, d_frame_status, stream);
+}
+
+int ag_refined_saddle_points_batch_device(ag_detector* det, const void* d_frames, size_t frame_stride,
+                                          int n_frames, int width, int height, size_t row_stride, int format,
+                                          ag_saddle* d_out, int cap_per_frame, int* d_n_per_frame,
+                                          uint32_t* d_frame_status, void* stream) {
+  return batch_device(det, ResultKind::kSaddles, d_frames, frame_stride, n_frames, width, height, row_stride, format,
+                      d_out, cap_per_frame, d_n_per_frame, d_frame_status, stream);
 }
 
 int ag_detect_batch_device_wait(ag_detector* det, void* stream) {
@@ -1139,10 +1225,11 @@ int ag_dense_batch_device(ag_detector* det, const void* d_frames, size_t frame_s
   return AG_OK;
 }
 
-// ag_detect_batch proper.  async_call: return once the chunks are enqueued (streaming use, option
-// host_async); otherwise the results are in the output arrays when the call returns.
-static int detect_batch_host(ag_detector* det, const void* frames, size_t frame_stride, int n_frames, int width,
-                             int height, size_t row_stride, int format, ag_tag* out, int cap_per_frame,
+// ag_detect_batch proper, and ag_refined_saddle_points_batch (kind kSaddles, out = ag_saddle records).
+// async_call: return once the chunks are enqueued (streaming use, option host_async; tags only);
+// otherwise the results are in the output arrays when the call returns.
+static int detect_batch_host(ag_detector* det, ResultKind kind, const void* frames, size_t frame_stride, int n_frames,
+                             int width, int height, size_t row_stride, int format, void* out, int cap_per_frame,
                              int* n_per_frame, uint32_t* frame_status, bool async_call) {
   if (!det) return AG_ERR_INVALID;
   if (!frames || !out || !n_per_frame || n_frames < 0 || cap_per_frame < 1)
@@ -1191,7 +1278,11 @@ static int detect_batch_host(ag_detector* det, const void* frames, size_t frame_
     // the slot's previous chunk (of this call or an earlier one): wait for its results, hand them out
     if ((rc = collect_host_slot(det, bi))) return rc;
     if ((rc = ensure_board_slot(det, B, chunk, true))) return rc;
-    if ((rc = ensure_host_stage(det, B, chunk_bytes, chunk, cap_per_frame))) return rc;
+    // saddles: an unflagged frame has at most the slot's cap_saddles, so a large cap_per_frame does
+    // not multiply the staging; a flagged frame is re-run from the host at collection
+    const bool saddles = kind == ResultKind::kSaddles;
+    const int sad_stride = saddles ? std::min(cap_per_frame, B.cap_saddles) : 0;
+    if ((rc = ensure_host_stage(det, B, chunk_bytes, chunk, saddles ? 1 : cap_per_frame, sad_stride))) return rc;
     const int n = n_this;
     const uint8_t* src = (const uint8_t*)frames + (size_t)f0 * g.frame_stride;
     const size_t bytes = (size_t)(n - 1) * g.frame_stride + frame_bytes(g);
@@ -1210,27 +1301,32 @@ static int detect_batch_host(ag_detector* det, const void* frames, size_t frame_
     AG_CUDA(det, cudaMemcpyAsync(B.d_in, up_src, bytes, cudaMemcpyHostToDevice, up));
     AG_CUDA(det, cudaEventRecord(B.ev_up, up));
     AG_CUDA(det, cudaStreamWaitEvent(s, B.ev_up, 0));
-    if ((rc = run_front(det, B, B.d_in, g, n, B.d_status, s))) return rc;
-    AG_CUDA(det, cudaStreamWaitEvent(B.bstream, B.ev_front, 0));
-    if ((rc = run_boards(det, B, B.d_in, g, n, B.d_tags, B.hs_tags, B.d_ntags, B.d_status, false, B.bstream)))
+    // (run_back records the same events the device-batch path orders itself by: a later device call
+    // or a quiesce sees this chunk's back end and front end like one of its own)
+    if ((rc = run_front(det, B, B.d_in, g, n, B.d_status, s)) ||
+        (rc = saddles ? run_back(det, B, kind, B.d_in, g, n, B.d_sad, sad_stride, cap_per_frame, B.d_ntags, B.d_status)
+                      : run_back(det, B, kind, B.d_in, g, n, B.d_tags, B.hs_tags, B.hs_tags, B.d_ntags, B.d_status)))
       return rc;
-    // the same events the device-batch path orders itself by: a later device call (or a quiesce)
-    // sees this chunk's board kernel and front end like one of its own
-    AG_CUDA(det, cudaEventRecord(B.ev_boards, B.bstream));
     AG_CUDA(det, cudaMemcpyAsync(B.h_ntags, B.d_ntags, sizeof(int) * n, cudaMemcpyDeviceToHost, B.bstream));
     AG_CUDA(det, cudaMemcpyAsync(B.h_status, B.d_status, sizeof(uint32_t) * n, cudaMemcpyDeviceToHost,
                                  B.bstream));
-    AG_CUDA(det, cudaMemcpyAsync(B.h_tags, B.d_tags, sizeof(ag_tag) * (size_t)n * B.hs_tags,
-                                 cudaMemcpyDeviceToHost, B.bstream));
+    if (saddles)
+      AG_CUDA(det, cudaMemcpyAsync(B.h_sad, B.d_sad, sizeof(ag_saddle) * (size_t)n * sad_stride,
+                                   cudaMemcpyDeviceToHost, B.bstream));
+    else
+      AG_CUDA(det, cudaMemcpyAsync(B.h_tags, B.d_tags, sizeof(ag_tag) * (size_t)n * B.hs_tags,
+                                   cudaMemcpyDeviceToHost, B.bstream));
     AG_CUDA(det, cudaEventRecord(B.ev_done, B.bstream));
-    B.pending = true;
     auto& P = det->hpend[bi];
     P.live = true;
+    P.kind = kind;
     P.f0 = f0;
     P.n = n;
     P.cap = cap_per_frame;
+    P.sad_stride = sad_stride;
     P.seq = seq;
-    P.out = out;
+    P.out = saddles ? nullptr : (ag_tag*)out;
+    P.sad_out = saddles ? (ag_saddle*)out : nullptr;
     P.n_per_frame = n_per_frame;
     P.status = frame_status;
     P.src = src;
@@ -1246,8 +1342,17 @@ static int detect_batch_host(ag_detector* det, const void* frames, size_t frame_
 int ag_detect_batch(ag_detector* det, const void* frames, size_t frame_stride, int n_frames, int width,
                     int height, size_t row_stride, int format, ag_tag* out, int cap_per_frame,
                     int* n_per_frame, uint32_t* frame_status) {
-  return detect_batch_host(det, frames, frame_stride, n_frames, width, height, row_stride, format, out,
-                           cap_per_frame, n_per_frame, frame_status, det ? det->host_async : false);
+  return detect_batch_host(det, ResultKind::kTags, frames, frame_stride, n_frames, width, height, row_stride, format,
+                           out, cap_per_frame, n_per_frame, frame_status, det ? det->host_async : false);
+}
+
+// refined_saddle_points over a batch: always synchronous (streaming saddle calls over host frames
+// are not offered), so a host_async handle's detect chunks still in flight are collected first.
+int ag_refined_saddle_points_batch(ag_detector* det, const void* frames, size_t frame_stride, int n_frames, int width,
+                                   int height, size_t row_stride, int format, ag_saddle* out, int cap_per_frame,
+                                   int* n_per_frame, uint32_t* frame_status) {
+  return detect_batch_host(det, ResultKind::kSaddles, frames, frame_stride, n_frames, width, height, row_stride,
+                           format, out, cap_per_frame, n_per_frame, frame_status, false);
 }
 
 int ag_detect_batch_wait(ag_detector* det, int keep_in_flight) {
@@ -1268,8 +1373,8 @@ int ag_detect(ag_detector* det, const void* pixels, int width, int height, size_
               int format, ag_tag* out, int cap, int* n) {
   if (!n) return det ? fail(det, AG_ERR_INVALID, "n is null") : AG_ERR_INVALID;
   int cnt = 0;
-  int rc = detect_batch_host(det, pixels, 0, 1, width, height, row_stride, format, out, cap, &cnt, nullptr,
-                             false);
+  int rc = detect_batch_host(det, ResultKind::kTags, pixels, 0, 1, width, height, row_stride, format, out, cap, &cnt,
+                             nullptr, false);
   *n = cnt;
   return rc;
 }
@@ -1892,9 +1997,12 @@ int ag_multi_set_option(ag_multi* m, const char* key, long value) {
   return AG_OK;
 }
 
-int ag_multi_detect_batch(ag_multi* m, const void* frames, size_t frame_stride, int n_frames, int width,
-                          int height, size_t row_stride, int format, ag_tag* out, int cap_per_frame,
-                          int* n_per_frame, uint32_t* frame_status) {
+// The host-buffer batch call of one kind over every device of m: the shard boundaries, one host
+// thread per device, the worst code.  Each shard runs synchronously, whatever a device's
+// "host_async" says (ag_multi has no wait entry point), as ag_detect.
+static int multi_batch_host(ag_multi* m, ResultKind kind, const void* frames, size_t frame_stride, int n_frames,
+                            int width, int height, size_t row_stride, int format, void* out, int cap_per_frame,
+                            int* n_per_frame, uint32_t* frame_status) {
   if (!m || m->dets.empty()) return AG_ERR_INVALID;
   if (!frames || !out || !n_per_frame || n_frames < 0 || cap_per_frame < 1) {
     m->err = "null pointer or bad count";
@@ -1903,6 +2011,7 @@ int ag_multi_detect_batch(ag_multi* m, const void* frames, size_t frame_stride, 
   // the strides every shard's offsets are computed with (0 = tightly packed, as in ag_detect_batch)
   const size_t rs = row_stride ? row_stride : (size_t)(width > 0 ? width : 0) * bytes_per_px(format);
   const size_t fs = frame_stride ? frame_stride : rs * (size_t)(height > 0 ? height : 0);
+  const size_t rec = kind == ResultKind::kTags ? sizeof(ag_tag) : sizeof(ag_saddle);
   const int G = (int)m->dets.size();
   std::vector<int> rcs(G, AG_OK);
   // shard boundaries: equal ranges, or -- when the devices' measured host-to-device rates differ by
@@ -1922,10 +2031,9 @@ int ag_multi_detect_batch(ag_multi* m, const void* frames, size_t frame_stride, 
   auto work = [&](int g) {
     const long long lo = bound[g], hi = bound[g + 1];
     if (hi <= lo) return;
-    // synchronous whatever a device's "host_async" says (ag_multi has no wait entry point), as ag_detect
-    rcs[g] = detect_batch_host(m->dets[g], (const uint8_t*)frames + (size_t)lo * fs, fs, (int)(hi - lo), width,
-                               height, rs, format, out + (size_t)lo * cap_per_frame, cap_per_frame, n_per_frame + lo,
-                               frame_status ? frame_status + lo : nullptr, /*async_call=*/false);
+    rcs[g] = detect_batch_host(m->dets[g], kind, (const uint8_t*)frames + (size_t)lo * fs, fs, (int)(hi - lo), width,
+                               height, rs, format, (uint8_t*)out + (size_t)lo * cap_per_frame * rec, cap_per_frame,
+                               n_per_frame + lo, frame_status ? frame_status + lo : nullptr, /*async_call=*/false);
   };
   std::vector<std::thread> th;
   for (int g = 1; g < G; ++g) th.emplace_back(work, g);
@@ -1938,6 +2046,20 @@ int ag_multi_detect_batch(ag_multi* m, const void* frames, size_t frame_stride, 
       m->err = std::string("device ") + std::to_string(m->dets[g]->device) + ": " + ag_last_error(m->dets[g]);
     }
   return worst;
+}
+
+int ag_multi_detect_batch(ag_multi* m, const void* frames, size_t frame_stride, int n_frames, int width,
+                          int height, size_t row_stride, int format, ag_tag* out, int cap_per_frame,
+                          int* n_per_frame, uint32_t* frame_status) {
+  return multi_batch_host(m, ResultKind::kTags, frames, frame_stride, n_frames, width, height, row_stride, format, out,
+                          cap_per_frame, n_per_frame, frame_status);
+}
+
+int ag_multi_refined_saddle_points_batch(ag_multi* m, const void* frames, size_t frame_stride, int n_frames,
+                                         int width, int height, size_t row_stride, int format, ag_saddle* out,
+                                         int cap_per_frame, int* n_per_frame, uint32_t* frame_status) {
+  return multi_batch_host(m, ResultKind::kSaddles, frames, frame_stride, n_frames, width, height, row_stride, format,
+                          out, cap_per_frame, n_per_frame, frame_status);
 }
 
 }  // extern "C"

@@ -55,6 +55,10 @@ int launch_refine_filter(const float* blur, const FrameGeom& g, int n_frames, co
                          const int* n_clusters, int max_clusters, ag_saddle* raw, uint8_t* raw_valid,
                          float min_angle, float max_angle, int max_saddles, ag_saddle* refined,
                          int* n_refined, uint32_t* frame_status, cudaStream_t s);
+// the saddle entry points' result: K4's lists (in_stride per frame) -> out (out_stride per frame),
+// n_out = exact count (0 if the frame's list was truncated), AG_FRAME_TAG_OVERFLOW when n > cap
+int launch_saddles_out(const ag_saddle* refined, int in_stride, const int* n_refined, uint32_t* frame_status,
+                       int n_frames, ag_saddle* out, int out_stride, int cap, int* n_out, cudaStream_t s);
 
 // ag_board.cu
 extern int g_board_smem_pad;

@@ -717,6 +717,41 @@ k_refine_filter(const float* __restrict__ blur, FrameGeom g, const float2* __res
   }
 }
 
+// Result of the saddle entry points: each frame's refined saddles (K4's list, `in_stride` records per
+// frame) in the caller's layout (`out_stride` records per frame).  One block per frame.  The count
+// is exact, or 0 for a frame whose list K3 / K4 truncated (cluster or saddle overflow); the first
+// min(n, cap) records are copied as 32-bit words, so consecutive lanes touch consecutive words
+// whatever the 20-byte record boundaries; n > cap sets AG_FRAME_TAG_OVERFLOW.  The callers give
+// out_stride >= min(n, cap): an unflagged frame has at most in_stride saddles.
+constexpr int kSaddlesOutThreads = 256;
+constexpr int kSaddleWords = (int)(sizeof(ag_saddle) / sizeof(uint32_t));
+static_assert(sizeof(ag_saddle) == 5 * sizeof(uint32_t), "ag_saddle is five 32-bit words");
+
+__global__ void __launch_bounds__(kSaddlesOutThreads)
+k_saddles_out(const ag_saddle* __restrict__ refined, int in_stride, const int* __restrict__ n_refined,
+              uint32_t* __restrict__ frame_status, ag_saddle* __restrict__ out, int out_stride, int cap,
+              int* __restrict__ n_out) {
+  const int f = blockIdx.x;
+  const uint32_t st = frame_status[f];
+  const int n = (st & (AG_FRAME_CLUSTER_OVERFLOW | AG_FRAME_SADDLE_OVERFLOW)) ? 0 : n_refined[f];
+  const int words = min(n, cap) * kSaddleWords;
+  const uint32_t* src = reinterpret_cast<const uint32_t*>(refined + (size_t)f * in_stride);
+  uint32_t* dst = reinterpret_cast<uint32_t*>(out + (size_t)f * out_stride);
+  for (int i = threadIdx.x; i < words; i += kSaddlesOutThreads) dst[i] = src[i];
+  if (threadIdx.x == 0) {
+    n_out[f] = n;
+    if (n > cap) frame_status[f] = st | AG_FRAME_TAG_OVERFLOW;
+  }
+}
+
+int launch_saddles_out(const ag_saddle* refined, int in_stride, const int* n_refined, uint32_t* frame_status,
+                       int n_frames, ag_saddle* out, int out_stride, int cap, int* n_out, cudaStream_t s) {
+  if (n_frames <= 0) return 0;
+  k_saddles_out<<<n_frames, kSaddlesOutThreads, 0, s>>>(refined, in_stride, n_refined, frame_status, out, out_stride,
+                                                         cap, n_out);
+  return 1;
+}
+
 int launch_label_clusters(const uint32_t* mask, const FrameGeom& g, int n_frames, int* parent,
                           int max_clusters, int* acc, float2* centers, int* n_clusters,
                           uint32_t* frame_status, uint32_t* pixlist, int list_cap, int variant,

@@ -118,6 +118,10 @@ mod ffi {
         pub fn ag_detect_batch_wait(det: *mut AgDetector, keep_in_flight: c_int) -> c_int;
         pub fn ag_refined_saddle_points(det: *mut AgDetector, pixels: *const c_void, width: c_int, height: c_int,
                                         row_stride: usize, format: c_int, out: *mut AgSaddle, cap: c_int, n: *mut c_int) -> c_int;
+        pub fn ag_refined_saddle_points_batch(det: *mut AgDetector, frames: *const c_void, frame_stride: usize,
+                                              n_frames: c_int, width: c_int, height: c_int, row_stride: usize,
+                                              format: c_int, out: *mut AgSaddle, cap_per_frame: c_int,
+                                              n_per_frame: *mut c_int, frame_status: *mut u32) -> c_int;
         pub fn ag_host_alloc(bytes: usize) -> *mut c_void;
         pub fn ag_host_free(p: *mut c_void);
         pub fn ag_multi_create(family: c_int, params: *const DetectorParams, devices: *const c_int, n_devices: c_int,
@@ -127,6 +131,10 @@ mod ffi {
         pub fn ag_multi_detect_batch(m: *mut AgMulti, frames: *const c_void, frame_stride: usize, n_frames: c_int,
                                      width: c_int, height: c_int, row_stride: usize, format: c_int, out: *mut AgTag,
                                      cap_per_frame: c_int, n_per_frame: *mut c_int, frame_status: *mut u32) -> c_int;
+        pub fn ag_multi_refined_saddle_points_batch(m: *mut AgMulti, frames: *const c_void, frame_stride: usize,
+                                                    n_frames: c_int, width: c_int, height: c_int, row_stride: usize,
+                                                    format: c_int, out: *mut AgSaddle, cap_per_frame: c_int,
+                                                    n_per_frame: *mut c_int, frame_status: *mut u32) -> c_int;
     }
 }
 
@@ -142,6 +150,7 @@ const AG_RGB32F: c_int = 9;
 const AG_RGBA32F: c_int = 10;
 const AG_ERR_CAPACITY: c_int = 4;
 const TAG_CAP: usize = 1024; // >= the largest family (587 codes)
+const SADDLE_CAP: usize = 16384; // the library's hard limit per frame
 
 /// Page-locked host buffer (ag_host_alloc): frames packed here upload at the PCIe rate.
 struct Pinned {
@@ -220,6 +229,17 @@ fn pixels_of(img: &DynamicImage) -> (&[u8], c_int, usize, u32, u32) {
 
 fn corners(t: &AgTag) -> [(f32, f32); 4] {
     [(t.xy[0], t.xy[1]), (t.xy[2], t.xy[3]), (t.xy[4], t.xy[5]), (t.xy[6], t.xy[7])]
+}
+
+fn saddle_lists_of(out: &[AgSaddle], counts: &[c_int], cap: usize) -> Vec<Vec<Saddle>> {
+    (0..counts.len())
+        .map(|i| {
+            out[i * cap..i * cap + (counts[i] as usize).min(cap)]
+                .iter()
+                .map(|s| Saddle { p: (s.x, s.y), k: s.k, theta: s.theta, phi: s.phi })
+                .collect()
+        })
+        .collect()
 }
 
 fn maps_of(out: &[AgTag], counts: &[c_int], cap: usize) -> Vec<HashMap<u32, [(f32, f32); 4]>> {
@@ -368,6 +388,29 @@ impl TagDetector {
         out[..n as usize].iter().map(|s| Saddle { p: (s.x, s.y), k: s.k, theta: s.theta, phi: s.phi }).collect()
     }
 
+    /// New: `refined_saddle_points` of every image of a batch of equally sized images of one pixel format.
+    pub fn refined_saddle_points_batch(&self, imgs: &[DynamicImage]) -> Vec<Vec<Saddle>> {
+        if imgs.is_empty() {
+            return Vec::new();
+        }
+        let (packed, w, h, fmt, stride) = pack(imgs);
+        let mut out = vec![AgSaddle::default(); SADDLE_CAP * imgs.len()];
+        let mut counts = vec![0 as c_int; imgs.len()];
+        let det = self.checkout();
+        let rc = unsafe {
+            ffi::ag_refined_saddle_points_batch(det, packed.ptr as *const c_void, stride * h as usize, imgs.len() as c_int,
+                                                w as c_int, h as c_int, stride, fmt, out.as_mut_ptr(), SADDLE_CAP as c_int,
+                                                counts.as_mut_ptr(), std::ptr::null_mut())
+        };
+        if rc != 0 {
+            let msg = last_error(det);
+            self.checkin(det);
+            panic!("aprilgrid_b200: ag_refined_saddle_points_batch failed ({rc}): {msg}");
+        }
+        self.checkin(det);
+        saddle_lists_of(&out, &counts, SADDLE_CAP)
+    }
+
     #[cfg(feature = "kornia")]
     pub fn detect_kornia<const N: usize>(&self, img: &kornia::image::Image<u8, N>) -> HashMap<u32, [(f32, f32); 4]> {
         let (fmt, stride) = match img.num_channels() {
@@ -479,6 +522,26 @@ impl MultiTagDetector {
             panic!("aprilgrid_b200: ag_multi_detect_batch failed ({rc}): {msg}");
         }
         maps_of(&out, &counts, TAG_CAP)
+    }
+
+    pub fn refined_saddle_points_batch(&mut self, imgs: &[DynamicImage]) -> Vec<Vec<Saddle>> {
+        if imgs.is_empty() {
+            return Vec::new();
+        }
+        let (packed, w, h, fmt, stride) = pack(imgs);
+        let mut out = vec![AgSaddle::default(); SADDLE_CAP * imgs.len()];
+        let mut counts = vec![0 as c_int; imgs.len()];
+        let rc = unsafe {
+            ffi::ag_multi_refined_saddle_points_batch(self.m, packed.ptr as *const c_void, stride * h as usize,
+                                                      imgs.len() as c_int, w as c_int, h as c_int, stride, fmt,
+                                                      out.as_mut_ptr(), SADDLE_CAP as c_int, counts.as_mut_ptr(),
+                                                      std::ptr::null_mut())
+        };
+        if rc != 0 {
+            let msg = unsafe { std::ffi::CStr::from_ptr(ffi::ag_multi_last_error(self.m)).to_string_lossy().into_owned() };
+            panic!("aprilgrid_b200: ag_multi_refined_saddle_points_batch failed ({rc}): {msg}");
+        }
+        saddle_lists_of(&out, &counts, SADDLE_CAP)
     }
 }
 

@@ -112,7 +112,7 @@ enum {
   AG_FRAME_CLUSTER_OVERFLOW = 1, /* more saddle clusters than max_clusters            */
   AG_FRAME_SADDLE_OVERFLOW = 2,  /* more refined saddles than max_saddles             */
   AG_FRAME_BOARD_OVERFLOW = 4,   /* board grew outside the internal +-31 tag lattice  */
-  AG_FRAME_TAG_OVERFLOW = 8      /* more tags than cap_per_frame                       */
+  AG_FRAME_TAG_OVERFLOW = 8      /* more results (tags; saddles on the saddle entry points) than cap_per_frame */
 };
 
 typedef struct ag_detector ag_detector;
@@ -204,6 +204,40 @@ AG_API int ag_refined_saddle_points(ag_detector* det, const void* pixels, int wi
                                     size_t row_stride, int format, ag_saddle* out, int cap,
                                     int* n);
 
+/* refined_saddle_points on n_frames host images of one shape (layout and strides as ag_detect_batch).
+ * out[i*cap_per_frame ..]: frame i's refined saddles in the reference's order, n_per_frame[i] = their
+ * exact number; frame_status may be NULL.  Always synchronous (also on a "host_async" handle).
+ * Contract of the three saddle batch entry points (this one, _device and ag_multi_):
+ *  - Frame i's list is byte-identical to what ag_refined_saddle_points returns for that frame alone.
+ *  - Host calls: a frame that overflowed max_clusters / max_saddles in its chunk is re-run alone with
+ *    grown capacities and comes back untruncated; a frame beyond the hard limits (2^22 clusters,
+ *    16384 saddles) keeps its bits (and the list ag_refined_saddle_points gives it), and the call
+ *    returns AG_ERR_CAPACITY.  The device call cannot re-run: such a frame reports n = 0 and its bits.
+ *  - n_per_frame[i] > cap_per_frame: the count stays exact, the first cap_per_frame saddles are
+ *    written, the frame's status gets AG_FRAME_TAG_OVERFLOW, and the host calls return
+ *    AG_ERR_CAPACITY (the device call reports it through the bit only).  Nothing past
+ *    min(n, cap_per_frame) records of a frame's slot is written.
+ *  - n_frames == 0: AG_OK, nothing runs.  Null pointers, cap_per_frame < 1, n_frames < 0, bad
+ *    strides or a misaligned device address: AG_ERR_INVALID, nothing runs.
+ *  - Saddle and detect calls may be interleaved freely on one handle, on any streams; neither
+ *    changes the other's results.  A host saddle call first collects the detect chunks of
+ *    "host_async" calls still in flight, as ag_detect does. */
+AG_API int ag_refined_saddle_points_batch(ag_detector* det, const void* frames, size_t frame_stride,
+                                          int n_frames, int width, int height, size_t row_stride,
+                                          int format, ag_saddle* out, int cap_per_frame,
+                                          int* n_per_frame, uint32_t* frame_status);
+
+/* Same, frames and outputs in device memory (d_out: n_frames*cap_per_frame ag_saddle,
+ * d_n_per_frame: n_frames int32, d_frame_status: n_frames uint32 or NULL), enqueued on `stream`;
+ * option "device_async" and ag_detect_batch_device_wait apply to it exactly as to
+ * ag_detect_batch_device. */
+AG_API int ag_refined_saddle_points_batch_device(ag_detector* det, const void* d_frames,
+                                                 size_t frame_stride, int n_frames, int width,
+                                                 int height, size_t row_stride, int format,
+                                                 ag_saddle* d_out, int cap_per_frame,
+                                                 int* d_n_per_frame, uint32_t* d_frame_status,
+                                                 void* stream);
+
 /* image_util::gaussian_blur_f32(img, sigma) and image_util::hessian_response(img):
  * f32 -> f32, host buffers, width*height floats each.                                   */
 AG_API int ag_gaussian_blur_f32(ag_detector* det, const float* img, int width, int height,
@@ -288,6 +322,12 @@ AG_API int ag_multi_set_option(ag_multi* m, const char* key, long value); /* app
 AG_API int ag_multi_detect_batch(ag_multi* m, const void* frames, size_t frame_stride, int n_frames,
                                  int width, int height, size_t row_stride, int format, ag_tag* out,
                                  int cap_per_frame, int* n_per_frame, uint32_t* frame_status);
+/* ag_refined_saddle_points_batch over every device of m (same sharding as ag_multi_detect_batch). */
+AG_API int ag_multi_refined_saddle_points_batch(ag_multi* m, const void* frames, size_t frame_stride,
+                                                int n_frames, int width, int height,
+                                                size_t row_stride, int format, ag_saddle* out,
+                                                int cap_per_frame, int* n_per_frame,
+                                                uint32_t* frame_status);
 
 AG_API const char* ag_version(void);
 
