@@ -57,6 +57,12 @@ class _Params(C.Structure):
                 ("max_saddle_angle", C.c_float), ("max_num_of_boards", C.c_uint8)]
 
 
+class AgFrame(C.Structure):
+    """ag_frame (include/aprilgrid_b200.h): one frame of a frame list."""
+    _fields_ = [("pixels", C.c_void_p), ("width", C.c_int), ("height", C.c_int), ("row_stride", C.c_size_t),
+                ("format", C.c_int)]
+
+
 class DetectorParams:
     """src/detector.rs:25-41"""
 
@@ -142,6 +148,13 @@ def lib():
                                                   vp, vp]
         L.ag_test_float_luma.argtypes = [vp, vp, C.c_longlong, ci, vp, vp]
         L.ag_test_host_chunk.argtypes = [C.c_longlong, ci, vp]
+        L.ag_detect_frames.argtypes = [vp, vp, ci, vp, ci, vp, vp]
+        L.ag_refined_saddle_points_frames.argtypes = [vp, vp, ci, vp, ci, vp, vp]
+        L.ag_detect_frames_device.argtypes = [vp, vp, ci, vp, ci, vp, vp, vp]
+        L.ag_refined_saddle_points_frames_device.argtypes = [vp, vp, ci, vp, ci, vp, vp, vp]
+        L.ag_multi_detect_frames.argtypes = [vp, vp, ci, vp, ci, vp, vp]
+        L.ag_multi_refined_saddle_points_frames.argtypes = [vp, vp, ci, vp, ci, vp, vp]
+        L.ag_test_frame_plan.argtypes = [vp, ci, C.c_longlong, C.c_longlong, ci, vp, ci, vp, vp, vp, vp]
         _lib = L
     return _lib
 
@@ -164,6 +177,30 @@ def image_format(img):
     raise ValueError("unsupported image: shape %s dtype %s (want HxW or HxWxN u8/u16 with N in 2..4, "
                      "or HxWxN float32 with N in 3..4)"
                      % (img.shape, img.dtype))
+
+
+def frame_list(images):
+    """(ctypes array of AgFrame, the arrays it points into) for a list of host images of any shapes and
+    formats (as image_format takes them); keep the arrays alive while the descriptors are in use."""
+    keep = []
+    descs = (AgFrame * max(len(images), 1))()
+    for i, img in enumerate(images):
+        img = np.asarray(img)
+        if img.strides[-1] != img.itemsize or (img.ndim == 3 and img.strides[1] != img.shape[2] * img.itemsize) \
+                or img.strides[0] < 0:
+            img = np.ascontiguousarray(img)
+        fmt, w, h, st = image_format(img)
+        keep.append(img)
+        descs[i] = AgFrame(img.ctypes.data, w, h, st, fmt)
+    return descs, keep
+
+
+def device_frame_list(descs):
+    """ctypes array of AgFrame from (device pointer, width, height, fmt, row_stride) tuples."""
+    arr = (AgFrame * max(len(descs), 1))()
+    for i, (ptr, w, h, fmt, rs) in enumerate(descs):
+        arr[i] = AgFrame(ptr, w, h, rs, fmt)
+    return arr
 
 
 def family_info(family):
@@ -305,6 +342,47 @@ class TagDetector:
         """With option device_async = 1: order every detect_batch_device call issued so far on `stream`
         (None = block the host thread)."""
         return self._check(lib().ag_detect_batch_device_wait(self._h, C.c_void_p(stream) if stream else None))
+
+    def detect_frames(self, images, cap_per_frame=128, return_status=False):
+        """detect on a list of host images of any sizes and pixel formats in one call; result i is
+        byte-identical to detect(images[i])."""
+        n = len(images)
+        out = np.zeros((max(n, 1), cap_per_frame), TAG_DTYPE)
+        cnt = np.zeros(max(n, 1), np.int32)
+        status = np.zeros(max(n, 1), np.uint32)
+        descs, _keep = frame_list(images)
+        self._check(lib().ag_detect_frames(self._h, descs, n, _p(out), cap_per_frame, _p(cnt), _p(status)))
+        res = [_tags_to_dict(out[i, :cnt[i]]) for i in range(n)]
+        return (res, status[:n]) if return_status else res
+
+    def refined_saddle_points_frames(self, images, cap_per_frame=2048, return_status=False):
+        """refined_saddle_points on a list of host images of any sizes and pixel formats in one call."""
+        n = len(images)
+        out = np.zeros((max(n, 1), cap_per_frame), SADDLE_DTYPE)
+        cnt = np.zeros(max(n, 1), np.int32)
+        status = np.zeros(max(n, 1), np.uint32)
+        descs, _keep = frame_list(images)
+        self._check(lib().ag_refined_saddle_points_frames(self._h, descs, n, _p(out), cap_per_frame, _p(cnt),
+                                                          _p(status)))
+        res = [out[i, :cnt[i]].copy() for i in range(n)]
+        return (res, status[:n]) if return_status else res
+
+    def detect_frames_device(self, descs, d_out_ptr, cap_per_frame, d_counts_ptr, d_status_ptr=None, stream=None):
+        """Device-resident frames given as (ptr, width, height, fmt, row_stride) tuples, device-resident
+        results indexed by list position (d_out: len(descs) x cap_per_frame TAG_DTYPE records), asynchronous
+        on `stream` as detect_batch_device."""
+        arr = device_frame_list(descs)
+        return self._check(lib().ag_detect_frames_device(
+            self._h, arr, len(descs), C.c_void_p(d_out_ptr), cap_per_frame, C.c_void_p(d_counts_ptr),
+            C.c_void_p(d_status_ptr) if d_status_ptr else None, C.c_void_p(stream) if stream else None))
+
+    def refined_saddle_points_frames_device(self, descs, d_out_ptr, cap_per_frame, d_counts_ptr, d_status_ptr=None,
+                                            stream=None):
+        """As detect_frames_device, with SADDLE_DTYPE records."""
+        arr = device_frame_list(descs)
+        return self._check(lib().ag_refined_saddle_points_frames_device(
+            self._h, arr, len(descs), C.c_void_p(d_out_ptr), cap_per_frame, C.c_void_p(d_counts_ptr),
+            C.c_void_p(d_status_ptr) if d_status_ptr else None, C.c_void_p(stream) if stream else None))
 
     def dense_batch_device(self, d_frames_ptr, n_frames, width, height, fmt, stream=None):
         return self._check(lib().ag_dense_batch_device(
@@ -489,6 +567,25 @@ def host_chunk_frames(host_chunk, fmt):
     return out.value
 
 
+def frame_plan(geoms, chunk_frames=1024, host_chunk_frames=128, host=True, rates=None, n_devices=1):
+    """Test hook (no GPU): the plan of a frame list given as (width, height, fmt, row_stride) tuples ->
+    (order, chunk bounds into order, multi-GPU index bounds for n_devices devices with the given
+    host-to-device rates)."""
+    n = len(geoms)
+    descs = (AgFrame * max(n, 1))()
+    for i, (w, h, fmt, rs) in enumerate(geoms):
+        descs[i] = AgFrame(None, w, h, rs, fmt)
+    order = np.zeros(max(n, 1), np.int32)
+    chunk0 = np.zeros(n + 1, np.int32)
+    n_chunks = C.c_int(0)
+    bounds = np.zeros(n_devices + 1, np.int64)
+    r = np.asarray(rates, np.float64) if rates is not None else None
+    if lib().ag_test_frame_plan(descs, n, chunk_frames, host_chunk_frames, 1 if host else 0, _p(r), n_devices,
+                                _p(order), _p(chunk0), C.byref(n_chunks), _p(bounds)) != AG_OK:
+        raise ValueError("bad frame list or options")
+    return order[:n].copy(), chunk0[:n_chunks.value + 1].copy(), bounds
+
+
 def pinned_empty(shape, dtype=np.uint8):
     """numpy array in page-locked host memory (ag_host_alloc); keep the returned array alive while in use
     and release it with pinned_free(arr)."""
@@ -561,6 +658,31 @@ class MultiTagDetector:
         if n:
             self.detect_batch_into(frames, out, cnt, status)
         return [_tags_to_dict(out[i, :cnt[i]]) for i in range(n)]
+
+    def _frames(self, fn, images, cap_per_frame, dtype, return_status):
+        n = len(images)
+        out = np.zeros((max(n, 1), cap_per_frame), dtype)
+        cnt = np.zeros(max(n, 1), np.int32)
+        status = np.zeros(max(n, 1), np.uint32)
+        descs, _keep = frame_list(images)
+        rc = fn(self._h, descs, n, _p(out), cap_per_frame, _p(cnt), _p(status))
+        if rc != AG_OK:
+            raise RuntimeError("aprilgrid_b200 error %d: %s" % (rc, lib().ag_multi_last_error(self._h).decode()))
+        return out, cnt, status[:n]
+
+    def detect_frames(self, images, cap_per_frame=128, return_status=False):
+        """TagDetector.detect_frames over every device (the list cut by frame bytes); byte-identical to one
+        device."""
+        out, cnt, status = self._frames(lib().ag_multi_detect_frames, images, cap_per_frame, TAG_DTYPE, return_status)
+        res = [_tags_to_dict(out[i, :cnt[i]]) for i in range(len(images))]
+        return (res, status) if return_status else res
+
+    def refined_saddle_points_frames(self, images, cap_per_frame=2048, return_status=False):
+        """TagDetector.refined_saddle_points_frames over every device; byte-identical to one device."""
+        out, cnt, status = self._frames(lib().ag_multi_refined_saddle_points_frames, images, cap_per_frame,
+                                        SADDLE_DTYPE, return_status)
+        res = [out[i, :cnt[i]].copy() for i in range(len(images))]
+        return (res, status) if return_status else res
 
     def refined_saddle_points_batch(self, frames, cap_per_frame=2048):
         """TagDetector.refined_saddle_points_batch over every device; byte-identical to one device."""

@@ -8,6 +8,8 @@
 //   detect_batch(frames...)  -> vector of such maps (new entry point)
 //   refined_saddle_points(image) -> std::vector<Saddle>
 //   refined_saddle_points_batch(frames...) -> vector of such lists (new entry point)
+//   detect_frames / refined_saddle_points_frames(vector<ImageView>) -> the same for images of mixed
+//   sizes and pixel formats (new entry points)
 #pragma once
 #include <array>
 #include <optional>
@@ -49,6 +51,14 @@ struct ImageView {
 };
 
 using TagMap = std::unordered_map<uint32_t, std::array<std::pair<float, float>, 4>>;
+
+// ag_frame descriptors of a list of images (the two structs have the same fields in the same order).
+inline std::vector<ag_frame> frame_descs(const std::vector<ImageView>& imgs) {
+  std::vector<ag_frame> d(imgs.size());
+  for (size_t i = 0; i < imgs.size(); ++i)
+    d[i] = ag_frame{imgs[i].pixels, imgs[i].width, imgs[i].height, imgs[i].row_stride, imgs[i].format};
+  return d;
+}
 
 class TagDetector {
  public:
@@ -122,6 +132,29 @@ class TagDetector {
     return res;
   }
 
+  // images of any sizes and pixel formats, one call; result i equals detect(imgs[i])
+  std::vector<TagMap> detect_frames(const std::vector<ImageView>& imgs, int cap_per_frame = 128) const {
+    const int n = (int)imgs.size();
+    std::vector<ag_tag> out((size_t)n * cap_per_frame);
+    std::vector<int> cnt(n);
+    check(ag_detect_frames(h_, frame_descs(imgs).data(), n, out.data(), cap_per_frame, cnt.data(), nullptr));
+    std::vector<TagMap> res(n);
+    for (int i = 0; i < n; ++i) res[i] = to_map(out.data() + (size_t)i * cap_per_frame, cnt[i]);
+    return res;
+  }
+
+  std::vector<std::vector<Saddle>> refined_saddle_points_frames(const std::vector<ImageView>& imgs,
+                                                                int cap_per_frame = 2048) const {
+    const int n = (int)imgs.size();
+    std::vector<ag_saddle> out((size_t)n * cap_per_frame);
+    std::vector<int> cnt(n);
+    check(ag_refined_saddle_points_frames(h_, frame_descs(imgs).data(), n, out.data(), cap_per_frame, cnt.data(),
+                                          nullptr));
+    std::vector<std::vector<Saddle>> res(n);
+    for (int i = 0; i < n; ++i) res[i] = to_saddles(out.data() + (size_t)i * cap_per_frame, cnt[i]);
+    return res;
+  }
+
   ag_detector* handle() const { return h_; }
 
   static std::vector<Saddle> to_saddles(const ag_saddle* s, int n) {
@@ -188,6 +221,37 @@ class MultiTagDetector {
     std::vector<std::vector<Saddle>> res(n_frames);
     for (int i = 0; i < n_frames; ++i)
       res[i] = TagDetector::to_saddles(out.data() + (size_t)i * cap_per_frame, cnt[i]);
+    return res;
+  }
+
+  std::vector<TagMap> detect_frames(const std::vector<ImageView>& imgs, int cap_per_frame = 128) const {
+    const int n = (int)imgs.size();
+    std::vector<ag_tag> out((size_t)n * cap_per_frame);
+    std::vector<int> cnt(n);
+    if (ag_multi_detect_frames(m_, frame_descs(imgs).data(), n, out.data(), cap_per_frame, cnt.data(), nullptr) !=
+        AG_OK)
+      throw std::runtime_error(std::string("aprilgrid_b200: ") + ag_multi_last_error(m_));
+    std::vector<TagMap> res(n);
+    for (int i = 0; i < n; ++i) {
+      TagMap m;
+      const ag_tag* t = out.data() + (size_t)i * cap_per_frame;
+      for (int k = 0; k < cnt[i] && k < cap_per_frame; ++k)
+        m[t[k].id] = {{{t[k].xy[0], t[k].xy[1]}, {t[k].xy[2], t[k].xy[3]}, {t[k].xy[4], t[k].xy[5]}, {t[k].xy[6], t[k].xy[7]}}};
+      res[i] = std::move(m);
+    }
+    return res;
+  }
+
+  std::vector<std::vector<Saddle>> refined_saddle_points_frames(const std::vector<ImageView>& imgs,
+                                                                int cap_per_frame = 2048) const {
+    const int n = (int)imgs.size();
+    std::vector<ag_saddle> out((size_t)n * cap_per_frame);
+    std::vector<int> cnt(n);
+    if (ag_multi_refined_saddle_points_frames(m_, frame_descs(imgs).data(), n, out.data(), cap_per_frame, cnt.data(),
+                                              nullptr) != AG_OK)
+      throw std::runtime_error(std::string("aprilgrid_b200: ") + ag_multi_last_error(m_));
+    std::vector<std::vector<Saddle>> res(n);
+    for (int i = 0; i < n; ++i) res[i] = TagDetector::to_saddles(out.data() + (size_t)i * cap_per_frame, cnt[i]);
     return res;
   }
 

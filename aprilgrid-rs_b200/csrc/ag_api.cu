@@ -9,9 +9,12 @@
 
 #include <algorithm>
 #include <atomic>
+#include <functional>
+#include <map>
 #include <mutex>
 #include <string>
 #include <thread>
+#include <tuple>
 #include <vector>
 
 #include "ag_codebook.h"
@@ -102,6 +105,12 @@ struct BoardSlot {
   ag_saddle* h_sad = nullptr;
   size_t cap_sad = 0;
   cudaEvent_t ev_up = nullptr, ev_done = nullptr;  // upload done / results on the host
+  // frame lists on the device (ag_detect_frames_device): the tags of the chunk's board search,
+  // chunk-local, until k_tags_out copies them to the caller's frames; capacity in records / frames
+  ag_tag* d_ltags = nullptr;
+  int* d_lntags = nullptr;
+  size_t cap_ltags = 0;
+  int cap_lframes = 0;
 };
 
 // Dense and sparse buffers of one chunk (K1-K4).
@@ -146,6 +155,11 @@ struct ag_detector {
   BoardSlot bslot[kBoardSlots];
   int slot_rr = 0;            // next board slot of the device-batch pipeline (rotates across calls)
   cudaStream_t up_stream = nullptr;  // host-frame path: uploads, ahead of the kernels
+  // device frame lists: the memory pool of the calls' address tables, the stream that frees a call's
+  // table once its chunks are done, and the event marking the end of a call's work on the caller's stream
+  cudaMemPool_t tab_pool = nullptr;
+  cudaStream_t tab_stream = nullptr;
+  cudaEvent_t ev_tab = nullptr;
   // host-buffer path: chunks whose results still sit in a board slot's pinned staging, with the
   // output arrays of the ag_detect_batch call they belong to (calls may overlap: "host_async")
   struct HostPend {
@@ -160,6 +174,10 @@ struct ag_detector {
     uint32_t* status = nullptr;
     const uint8_t* src = nullptr;  // host frames of the chunk (re-run of overflowed frames)
     FrameGeom g{};
+    // chunks of a frame list: frame i of the chunk is the caller's frame idx[i], read from descs[i]
+    // (empty for a batch chunk: frame f0 + i at src + i * g.frame_stride)
+    std::vector<int> idx;
+    std::vector<ag_frame> descs;
   } hpend[kBoardSlots];
   uint64_t host_seq = 0;        // number of ag_detect_batch calls issued
   bool host_async = false;      // ag_detect_batch returns without collecting its results
@@ -230,23 +248,21 @@ int fail(ag_detector* det, int code, const char* msg) {
   return code;
 }
 
-int make_geom(ag_detector* det, int w, int h, size_t row_stride, size_t frame_stride, int format,
-              FrameGeom* g) {
-  if (w <= 0 || h <= 0) return fail(det, AG_ERR_INVALID, "width/height must be positive");
-  if (format == kFmtF32 || bytes_per_px(format) == 0) return fail(det, AG_ERR_INVALID, "unknown pixel format");
-  if ((long long)w * h > (1ll << 30)) return fail(det, AG_ERR_INVALID, "image too large");
+// The geometry of frames of one shape; returns what is wrong with the arguments, or nullptr.
+const char* geom_error(int w, int h, size_t row_stride, size_t frame_stride, int format, FrameGeom* g) {
+  if (w <= 0 || h <= 0) return "width/height must be positive";
+  if (format == kFmtF32 || bytes_per_px(format) == 0) return "unknown pixel format";
+  if ((long long)w * h > (1ll << 30)) return "image too large";
   size_t min_row = (size_t)w * bytes_per_px(format);
   if (row_stride == 0) row_stride = min_row;
-  if (row_stride < min_row) return fail(det, AG_ERR_INVALID, "row_stride smaller than a row");
+  if (row_stride < min_row) return "row_stride smaller than a row";
   const size_t al = (size_t)channel_align(format);
-  if (row_stride % al) return fail(det, AG_ERR_INVALID, "row_stride must be a multiple of the format's channel word");
+  if (row_stride % al) return "row_stride must be a multiple of the format's channel word";
   if (frame_stride == 0) frame_stride = row_stride * h;
-  if (frame_stride < row_stride * (size_t)(h - 1) + min_row)
-    return fail(det, AG_ERR_INVALID, "frame_stride smaller than a frame");
+  if (frame_stride < row_stride * (size_t)(h - 1) + min_row) return "frame_stride smaller than a frame";
   // other frames of a misaligned stride would start misaligned: K1 and K6 read 16-bit and f32 channels
   // with loads of their size (the host path keeps the caller's frame stride in its device staging too)
-  if (frame_stride % al)
-    return fail(det, AG_ERR_INVALID, "frame_stride must be a multiple of the format's channel word");
+  if (frame_stride % al) return "frame_stride must be a multiple of the format's channel word";
   g->w = w;
   g->h = h;
   g->wpr = (w + 31) / 32;
@@ -255,7 +271,13 @@ int make_geom(ag_detector* det, int w, int h, size_t row_stride, size_t frame_st
   g->row_stride = row_stride;
   g->frame_stride = frame_stride;
   g->format = format;
-  return AG_OK;
+  return nullptr;
+}
+
+int make_geom(ag_detector* det, int w, int h, size_t row_stride, size_t frame_stride, int format,
+              FrameGeom* g) {
+  const char* e = geom_error(w, h, row_stride, frame_stride, format, g);
+  return e ? fail(det, AG_ERR_INVALID, e) : AG_OK;
 }
 
 // Bytes from a frame's first pixel to its last: the padding after the last row is not the frame's.
@@ -391,7 +413,27 @@ int ensure_host_stage(ag_detector* det, BoardSlot& B, size_t in_bytes, int frame
   return AG_OK;
 }
 
+// Tag staging of a board slot for device frame-list chunks: `tag_stride` records for each of `frames`
+// frames.  Waits for the slot's back end only when the buffers are replaced.
+int ensure_list_stage(ag_detector* det, BoardSlot& B, int frames, int tag_stride) {
+  int rc;
+  const size_t tags = (size_t)frames * tag_stride;
+  if (tags <= B.cap_ltags && frames <= B.cap_lframes) return AG_OK;
+  if (B.pending) {
+    AG_CUDA(det, cudaEventSynchronize(B.ev_boards));
+    B.pending = false;
+  }
+  const int F = std::max(frames, B.cap_lframes);
+  const size_t T = std::max(tags, B.cap_ltags);
+  if ((rc = regrow(det, &B.d_ltags, T))) return rc;
+  if ((rc = regrow(det, &B.d_lntags, (size_t)F))) return rc;
+  B.cap_ltags = T;
+  B.cap_lframes = F;
+  return AG_OK;
+}
+
 void free_board_slot(BoardSlot& B) {
+  cudaFree(B.d_ltags); cudaFree(B.d_lntags);
   cudaFree(B.d_in); cudaFree(B.d_tags); cudaFree(B.d_ntags); cudaFree(B.d_sad);
   if (B.h_in) cudaFreeHost(B.h_in);
   if (B.h_sad) cudaFreeHost(B.h_sad);
@@ -535,6 +577,35 @@ void parallel_copy(uint8_t* dst, const uint8_t* src, size_t bytes) {
   for (auto& t : th) t.join();
 }
 
+// The pageable frames of a list chunk into the slot's pinned staging: (dst, src, bytes) segments, the
+// total cut into equal byte ranges, one per thread, whatever the frame sizes.
+struct CopySeg {
+  uint8_t* dst;
+  const uint8_t* src;
+  size_t n;
+};
+void parallel_copy_segs(const std::vector<CopySeg>& segs) {
+  size_t total = 0;
+  for (const auto& c : segs) total += c.n;
+  const unsigned hw = std::thread::hardware_concurrency();
+  size_t nt = std::min<size_t>(std::max<unsigned>(hw, 1), 24);
+  nt = std::min(nt, std::max<size_t>(total >> 22, 1));  // at least 4 MB per thread
+  const size_t per = ((total + nt - 1) / nt + 4095) & ~(size_t)4095;
+  auto part = [&](size_t lo, size_t hi) {
+    size_t off = 0;
+    for (const auto& c : segs) {
+      const size_t a = std::max(lo, off), b = std::min(hi, off + c.n);
+      if (a < b) stream_copy(c.dst + (a - off), c.src + (a - off), b - a);
+      off += c.n;
+      if (off >= hi) break;
+    }
+  };
+  std::vector<std::thread> th;
+  for (size_t t = 1; t < nt && t * per < total; ++t) th.emplace_back(part, t * per, std::min(total, (t + 1) * per));
+  part(0, std::min(per, total));
+  for (auto& t : th) t.join();
+}
+
 // Stage ids for the optional timing: 0 K1 blur+hessian+min, 1 K2 threshold, 2 K3 label+centroid,
 // 3 K4 refine+filter, 4 K6 boards+decode.
 void prof_mark(ag_detector* det, int stage, cudaStream_t s) {
@@ -661,21 +732,39 @@ int run_boards(ag_detector* det, BoardSlot& S, const uint8_t* d_frames, const Fr
   return AG_OK;
 }
 
+// Where the results of a device frame-list chunk go: chunk frame f is the caller's frame d_idx[f] of
+// out (cap records per frame), n and status (may be null).
+struct ListOut {
+  const int* d_idx;
+  void* out;
+  int cap;
+  int* n;
+  uint32_t* status;
+};
+
 // Back end of a pipeline chunk on board slot B's stream, once its front end is done (B.ev_front):
 // the board search into d_out (tags), or the copy of K4's saddle lists into d_out's layout
 // (saddles; out_stride records per frame).  Either way B.ev_boards then marks B free for the next
 // chunk's K4, so slot reuse, the streaming waits and the quiesce cover both kinds alike.
+// list (device frame lists): the saddles go straight to the caller's frames (d_out, d_n are the
+// caller's arrays); the tags land chunk-locally in d_out / d_n / d_status and k_tags_out copies them.
 int run_back(ag_detector* det, BoardSlot& B, ResultKind kind, const uint8_t* d_frames, const FrameGeom& g, int n,
-             void* d_out, int out_stride, int cap, int* d_n, uint32_t* d_status) {
+             void* d_out, int out_stride, int cap, int* d_n, uint32_t* d_status, const ListOut* list = nullptr) {
   const cudaStream_t s = B.bstream;
   AG_CUDA(det, cudaStreamWaitEvent(s, B.ev_front, 0));
   if (kind == ResultKind::kTags) {
     const int rc = run_boards(det, B, d_frames, g, n, (ag_tag*)d_out, cap, d_n, d_status, false, s);
     if (rc) return rc;
+    if (list) {
+      det->launches += launch_tags_out((const ag_tag*)d_out, out_stride, d_n, d_status, n, list->d_idx,
+                                       (ag_tag*)list->out, list->cap, list->n, list->status, s);
+      AG_CUDA(det, cudaGetLastError());
+    }
   } else {
     prof_mark(det, -1, s);  // (accounted to stage 3: the copy finishes the refined saddle list)
     det->launches += launch_saddles_out(B.d_refined, B.cap_saddles, B.d_nref, d_status, n, (ag_saddle*)d_out,
-                                        out_stride, cap, d_n, s);
+                                        out_stride, cap, d_n, s, list ? list->d_idx : nullptr,
+                                        list ? list->status : nullptr);
     prof_mark(det, 3, s);
     AG_CUDA(det, cudaGetLastError());
   }
@@ -758,9 +847,9 @@ int run_one_frame(ag_detector* det, const FrameGeom& g, const FrameGeom& gb, siz
 }
 
 void copy_out_b(const BoardSlot& B, int n, int cap, ag_tag* out, int* n_per_frame, uint32_t* frame_status,
-                int frame0, bool* truncated);
+                const int* idx, int frame0, bool* truncated);
 void copy_out_saddles(const BoardSlot& B, int n, int cap, int stride, ag_saddle* out, int* n_per_frame,
-                      uint32_t* frame_status, int frame0, bool* truncated);
+                      uint32_t* frame_status, const int* idx, int frame0, bool* truncated);
 
 // Host-buffer path: wait for the chunk staged in board slot bi and hand its results to the output
 // arrays of the call that submitted it.  A frame that overflowed max_clusters / max_saddles was
@@ -772,10 +861,11 @@ int collect_host_slot(ag_detector* det, int bi) {
   BoardSlot& B = det->bslot[bi];
   AG_CUDA(det, cudaEventSynchronize(B.ev_done));
   const bool saddles = P.kind == ResultKind::kSaddles;
+  const int* idx = P.idx.empty() ? nullptr : P.idx.data();
   if (saddles)
-    copy_out_saddles(B, P.n, P.cap, P.sad_stride, P.sad_out, P.n_per_frame, P.status, P.f0, &det->host_truncated);
+    copy_out_saddles(B, P.n, P.cap, P.sad_stride, P.sad_out, P.n_per_frame, P.status, idx, P.f0, &det->host_truncated);
   else
-    copy_out_b(B, P.n, P.cap, P.out, P.n_per_frame, P.status, P.f0, &det->host_truncated);
+    copy_out_b(B, P.n, P.cap, P.out, P.n_per_frame, P.status, idx, P.f0, &det->host_truncated);
   P.live = false;
   B.pending = false;
   for (int i = 0; i < P.n; ++i) {
@@ -783,7 +873,8 @@ int collect_host_slot(ag_detector* det, int bi) {
     if (st & kGrowable) {
       FrameGeom g = P.g;
       g.frame_stride = g.row_stride * (size_t)g.h;
-      const uint8_t* src = P.src + (size_t)i * P.g.frame_stride;
+      const uint8_t* src = idx ? (const uint8_t*)P.descs[i].pixels : P.src + (size_t)i * P.g.frame_stride;
+      const int o = idx ? idx[i] : P.f0 + i;
       auto upload = [&](uint8_t* d_in, cudaStream_t s) {
         return cudaMemcpyAsync(d_in, src, frame_bytes(g), cudaMemcpyHostToDevice, s);
       };
@@ -796,17 +887,17 @@ int collect_host_slot(ag_detector* det, int bi) {
       if (saddles) {
         // (a frame still beyond the limits keeps the list it has there, as ag_refined_saddle_points gives it)
         if (m > 0)
-          AG_CUDA(det, cudaMemcpy(P.sad_out + (size_t)(P.f0 + i) * P.cap, R.d_refined, sizeof(ag_saddle) * m,
+          AG_CUDA(det, cudaMemcpy(P.sad_out + (size_t)o * P.cap, R.d_refined, sizeof(ag_saddle) * m,
                                   cudaMemcpyDeviceToHost));
       } else {
-        memcpy(P.out + (size_t)(P.f0 + i) * P.cap, R.h_tags, sizeof(ag_tag) * (size_t)std::min(m, R.hs_tags));
+        memcpy(P.out + (size_t)o * P.cap, R.h_tags, sizeof(ag_tag) * (size_t)std::min(m, R.hs_tags));
       }
       if (cnt > P.cap) {
         st2 |= AG_FRAME_TAG_OVERFLOW;
         det->host_truncated = true;
       }
-      P.n_per_frame[P.f0 + i] = cnt;
-      if (P.status) P.status[P.f0 + i] = st2;
+      P.n_per_frame[o] = cnt;
+      if (P.status) P.status[o] = st2;
       if (st2 & (kGrowable | AG_FRAME_BOARD_OVERFLOW)) det->host_unresolved = true;
     } else if (st & AG_FRAME_BOARD_OVERFLOW) {
       det->host_unresolved = true;
@@ -879,28 +970,34 @@ void rochade_tables_host(float cone[25], float pinv[150]) {
 }
 
 // Host copy-out of one chunk's results from a board slot's pinned staging.
+// Frame i of the chunk is the caller's frame idx[i] (frame lists), or frame0 + i.
 void copy_out_b(const BoardSlot& B, int n, int cap, ag_tag* out, int* n_per_frame, uint32_t* frame_status,
-                int frame0, bool* truncated) {
+                const int* idx, int frame0, bool* truncated) {
   for (int i = 0; i < n; ++i) {
+    const int o = idx ? idx[i] : frame0 + i;
     const int cnt = B.h_ntags[i];
-    n_per_frame[frame0 + i] = cnt;
+    n_per_frame[o] = cnt;
     if (cnt > cap) *truncated = true;
     const int m = std::min(cnt, cap);
-    memcpy(out + (size_t)(frame0 + i) * cap, B.h_tags + (size_t)i * B.hs_tags, sizeof(ag_tag) * m);
-    if (frame_status) frame_status[frame0 + i] = B.h_status[i];
+    memcpy(out + (size_t)o * cap, B.h_tags + (size_t)i * B.hs_tags, sizeof(ag_tag) * m);
+    // (the slot's staging may be wider than this call's cap, so the board search need not have flagged
+    // the frame; a list call reports every frame with more tags than its cap, a batch chunk what the
+    // board search flagged, as ag_detect_batch always has)
+    if (frame_status) frame_status[o] = B.h_status[i] | (idx && cnt > cap ? (uint32_t)AG_FRAME_TAG_OVERFLOW : 0u);
   }
 }
 
 // ... of a saddle chunk: counts, status bits (with AG_FRAME_TAG_OVERFLOW) and records as
 // k_saddles_out left them, `stride` records per frame.
 void copy_out_saddles(const BoardSlot& B, int n, int cap, int stride, ag_saddle* out, int* n_per_frame,
-                      uint32_t* frame_status, int frame0, bool* truncated) {
+                      uint32_t* frame_status, const int* idx, int frame0, bool* truncated) {
   for (int i = 0; i < n; ++i) {
+    const int o = idx ? idx[i] : frame0 + i;
     const int cnt = B.h_ntags[i];
-    n_per_frame[frame0 + i] = cnt;
+    n_per_frame[o] = cnt;
     if (cnt > cap) *truncated = true;
-    memcpy(out + (size_t)(frame0 + i) * cap, B.h_sad + (size_t)i * stride, sizeof(ag_saddle) * std::min(cnt, cap));
-    if (frame_status) frame_status[frame0 + i] = B.h_status[i];
+    memcpy(out + (size_t)o * cap, B.h_sad + (size_t)i * stride, sizeof(ag_saddle) * std::min(cnt, cap));
+    if (frame_status) frame_status[o] = B.h_status[i];
   }
 }
 
@@ -914,6 +1011,93 @@ int host_call_verdict(ag_detector* det) {
                 "the +-31 tag lattice): its result is truncated, see frame_status");
   if (trunc) return fail(det, AG_ERR_CAPACITY, "cap_per_frame too small for at least one frame");
   return AG_OK;
+}
+
+// ---- frame lists -----------------------------------------------------------------------------------
+// Every descriptor of a list, checked before anything runs; geo[i] = frame i's geometry (packed frame
+// stride).  device: the address must be a multiple of the channel word too.  Returns the first
+// problem found ("frame i: ..."), or an empty string.
+std::string check_frames(const ag_frame* fr, int n, bool device, std::vector<FrameGeom>* geo) {
+  geo->resize((size_t)n);
+  for (int i = 0; i < n; ++i) {
+    const char* e = fr[i].pixels ? geom_error(fr[i].width, fr[i].height, fr[i].row_stride, 0, fr[i].format, &(*geo)[i])
+                                 : "pixels is null";
+    if (!e && device && (uintptr_t)fr[i].pixels % channel_align(fr[i].format))
+      e = "device frames must start at a multiple of the format's channel word";
+    if (e) return "frame " + std::to_string(i) + ": " + e;
+  }
+  return std::string();
+}
+
+// The order a list runs in: frames grouped by (width, height, format, row stride), groups in order of
+// first appearance, list order within a group; each group cut into chunks of one geometry by the limits
+// a batch of that geometry and group size gets (chunk_frames, and for host frames host_chunk_for), all
+// through chunk_limit.  Chunk k is order[chunk0[k] .. chunk0[k + 1]).
+struct FramePlan {
+  std::vector<int> order;
+  std::vector<int> chunk0;
+};
+FramePlan plan_frames(const std::vector<FrameGeom>& geo, long chunk_frames, long host_chunk_frames, bool host) {
+  const int n = (int)geo.size();
+  std::map<std::tuple<int, int, int, size_t>, int> group_of;
+  std::vector<std::vector<int>> groups;
+  for (int i = 0; i < n; ++i) {
+    const FrameGeom& g = geo[i];
+    auto it = group_of.emplace(std::make_tuple(g.w, g.h, g.format, g.row_stride), (int)groups.size()).first;
+    if (it->second == (int)groups.size()) groups.emplace_back();
+    groups[it->second].push_back(i);
+  }
+  FramePlan p;
+  p.order.reserve(n);
+  for (const auto& grp : groups) {
+    const FrameGeom& g = geo[grp[0]];
+    const long want = host ? std::min<long>(chunk_frames, host_chunk_for(host_chunk_frames, g.format)) : chunk_frames;
+    const int chunk = chunk_limit(nullptr, g, std::min<long>(want, (long)grp.size()));
+    for (size_t k = 0; k < grp.size(); k += chunk) p.chunk0.push_back((int)(p.order.size() + k));
+    p.order.insert(p.order.end(), grp.begin(), grp.end());
+  }
+  p.chunk0.push_back(n);
+  return p;
+}
+
+// The frame of a list with the most pixels: its automatic capacities are the call's.
+const FrameGeom& largest_frame(const std::vector<FrameGeom>& geo) {
+  size_t b = 0;
+  for (size_t i = 1; i < geo.size(); ++i)
+    if (geo[i].n_px > geo[b].n_px) b = i;
+  return geo[b];
+}
+
+// Shares of the devices of a multi-GPU set: equal, or -- when the measured host-to-device rates differ
+// by more than 5 % -- in proportion to those rates.
+std::vector<double> shard_shares(const std::vector<double>& rates, int G) {
+  double lo_r = 1e300, hi_r = 0.0, sum = 0.0;
+  for (double r : rates) { lo_r = std::min(lo_r, r); hi_r = std::max(hi_r, r); sum += r; }
+  const bool weighted = (int)rates.size() == G && lo_r > 0.0 && hi_r > 1.05 * lo_r;
+  std::vector<double> share(G);
+  for (int g = 0; g < G; ++g) share[g] = weighted ? rates[g] / sum : 1.0 / G;
+  return share;
+}
+
+// Contiguous index ranges [bound[g], bound[g + 1]) of a list, one per device, of about share[g] of the
+// list's frame bytes each: a frame goes to the range its middle byte falls in.
+std::vector<long long> list_shard_bounds(const std::vector<FrameGeom>& geo, const std::vector<double>& share) {
+  const int G = (int)share.size(), n = (int)geo.size();
+  double total = 0.0;
+  for (const auto& g : geo) total += (double)frame_bytes(g);
+  std::vector<long long> bound(G + 1, 0);
+  double acc = 0.0, before = 0.0;  // bytes of the frames before frame i
+  int i = 0;
+  for (int g = 0; g < G; ++g) {
+    acc += share[g];
+    if (g + 1 == G) {
+      i = n;
+    } else {
+      while (i < n && before + 0.5 * (double)frame_bytes(geo[i]) < acc * total) before += (double)frame_bytes(geo[i++]);
+    }
+    bound[g + 1] = i;
+  }
+  return bound;
 }
 
 }  // namespace
@@ -1019,6 +1203,9 @@ void ag_destroy(ag_detector* det) {
   free_slot(det->big);
   for (auto& B : det->bslot) free_board_slot(B);
   if (det->up_stream) cudaStreamDestroy(det->up_stream);
+  if (det->tab_stream) cudaStreamDestroy(det->tab_stream);
+  if (det->tab_pool) cudaMemPoolDestroy(det->tab_pool);
+  if (det->ev_tab) cudaEventDestroy(det->ev_tab);
   for (auto e : det->ev_pool) cudaEventDestroy(e);
   cudaFree(det->d_codes);
   cudaFree(det->d_f32_a); cudaFree(det->d_f32_b); cudaFree(det->d_f32_c); cudaFree(det->d_taps);
@@ -1225,6 +1412,53 @@ int ag_dense_batch_device(ag_detector* det, const void* d_frames, size_t frame_s
   return AG_OK;
 }
 
+// The part of a host-buffer chunk after its upload was enqueued (B.ev_up), shared by both host paths:
+// K1-K6 of the chunk staged in board slot bi, the download of its results on the slot's stream, and the
+// slot's pending record, from which collect_host_slot hands them to the call's output arrays.  Frame i
+// of a batch chunk is the caller's frame f0 + i at src + i * g.frame_stride; the caller of a list chunk
+// fills the record's idx and descs afterwards.
+static int enqueue_host_chunk(ag_detector* det, int bi, ResultKind kind, const FrameGeom& g, int n, int cap_per_frame,
+                              int sad_stride, uint64_t seq, void* out, int* n_per_frame, uint32_t* frame_status,
+                              int f0, const uint8_t* src) {
+  BoardSlot& B = det->bslot[bi];
+  const cudaStream_t s = det->dense[0].stream;
+  const bool saddles = kind == ResultKind::kSaddles;
+  int rc;
+  AG_CUDA(det, cudaStreamWaitEvent(s, B.ev_up, 0));
+  // (run_back records the same events the device-batch path orders itself by: a later device call
+  // or a quiesce sees this chunk's back end and front end like one of its own)
+  if ((rc = run_front(det, B, B.d_in, g, n, B.d_status, s)) ||
+      (rc = saddles ? run_back(det, B, kind, B.d_in, g, n, B.d_sad, sad_stride, cap_per_frame, B.d_ntags, B.d_status)
+                    : run_back(det, B, kind, B.d_in, g, n, B.d_tags, B.hs_tags, B.hs_tags, B.d_ntags, B.d_status)))
+    return rc;
+  AG_CUDA(det, cudaMemcpyAsync(B.h_ntags, B.d_ntags, sizeof(int) * n, cudaMemcpyDeviceToHost, B.bstream));
+  AG_CUDA(det, cudaMemcpyAsync(B.h_status, B.d_status, sizeof(uint32_t) * n, cudaMemcpyDeviceToHost, B.bstream));
+  if (saddles)
+    AG_CUDA(det, cudaMemcpyAsync(B.h_sad, B.d_sad, sizeof(ag_saddle) * (size_t)n * sad_stride,
+                                 cudaMemcpyDeviceToHost, B.bstream));
+  else
+    AG_CUDA(det, cudaMemcpyAsync(B.h_tags, B.d_tags, sizeof(ag_tag) * (size_t)n * B.hs_tags,
+                                 cudaMemcpyDeviceToHost, B.bstream));
+  AG_CUDA(det, cudaEventRecord(B.ev_done, B.bstream));
+  auto& P = det->hpend[bi];
+  P.live = true;
+  P.kind = kind;
+  P.f0 = f0;
+  P.n = n;
+  P.cap = cap_per_frame;
+  P.sad_stride = sad_stride;
+  P.seq = seq;
+  P.out = saddles ? nullptr : (ag_tag*)out;
+  P.sad_out = saddles ? (ag_saddle*)out : nullptr;
+  P.n_per_frame = n_per_frame;
+  P.status = frame_status;
+  P.src = src;
+  P.g = g;
+  P.idx.clear();
+  P.descs.clear();
+  return AG_OK;
+}
+
 // ag_detect_batch proper, and ag_refined_saddle_points_batch (kind kSaddles, out = ag_saddle records).
 // async_call: return once the chunks are enqueued (streaming use, option host_async; tags only);
 // otherwise the results are in the output arrays when the call returns.
@@ -1255,7 +1489,7 @@ static int detect_batch_host(ag_detector* det, ResultKind kind, const void* fram
       det, g, std::min<long>(std::min<long>(det->chunk_frames, host_chunk_for(det->host_chunk_frames, format)), n_frames));
   if ((rc = ensure_ring(det, g, chunk))) return rc;
   if (!det->up_stream) AG_CUDA(det, cudaStreamCreateWithFlags(&det->up_stream, cudaStreamNonBlocking));
-  cudaStream_t s = det->dense[0].stream, up = det->up_stream;
+  const cudaStream_t up = det->up_stream;
   const size_t chunk_bytes = (size_t)chunk * g.frame_stride;
   const bool pageable = is_pageable(frames);
   // Chunk schedule: the pipeline fills while the first chunk uploads and drains while the last one
@@ -1300,37 +1534,9 @@ static int detect_batch_host(ag_detector* det, ResultKind kind, const void* fram
     }
     AG_CUDA(det, cudaMemcpyAsync(B.d_in, up_src, bytes, cudaMemcpyHostToDevice, up));
     AG_CUDA(det, cudaEventRecord(B.ev_up, up));
-    AG_CUDA(det, cudaStreamWaitEvent(s, B.ev_up, 0));
-    // (run_back records the same events the device-batch path orders itself by: a later device call
-    // or a quiesce sees this chunk's back end and front end like one of its own)
-    if ((rc = run_front(det, B, B.d_in, g, n, B.d_status, s)) ||
-        (rc = saddles ? run_back(det, B, kind, B.d_in, g, n, B.d_sad, sad_stride, cap_per_frame, B.d_ntags, B.d_status)
-                      : run_back(det, B, kind, B.d_in, g, n, B.d_tags, B.hs_tags, B.hs_tags, B.d_ntags, B.d_status)))
+    if ((rc = enqueue_host_chunk(det, bi, kind, g, n, cap_per_frame, sad_stride, seq, out, n_per_frame, frame_status,
+                                 f0, src)))
       return rc;
-    AG_CUDA(det, cudaMemcpyAsync(B.h_ntags, B.d_ntags, sizeof(int) * n, cudaMemcpyDeviceToHost, B.bstream));
-    AG_CUDA(det, cudaMemcpyAsync(B.h_status, B.d_status, sizeof(uint32_t) * n, cudaMemcpyDeviceToHost,
-                                 B.bstream));
-    if (saddles)
-      AG_CUDA(det, cudaMemcpyAsync(B.h_sad, B.d_sad, sizeof(ag_saddle) * (size_t)n * sad_stride,
-                                   cudaMemcpyDeviceToHost, B.bstream));
-    else
-      AG_CUDA(det, cudaMemcpyAsync(B.h_tags, B.d_tags, sizeof(ag_tag) * (size_t)n * B.hs_tags,
-                                   cudaMemcpyDeviceToHost, B.bstream));
-    AG_CUDA(det, cudaEventRecord(B.ev_done, B.bstream));
-    auto& P = det->hpend[bi];
-    P.live = true;
-    P.kind = kind;
-    P.f0 = f0;
-    P.n = n;
-    P.cap = cap_per_frame;
-    P.sad_stride = sad_stride;
-    P.seq = seq;
-    P.out = saddles ? nullptr : (ag_tag*)out;
-    P.sad_out = saddles ? (ag_saddle*)out : nullptr;
-    P.n_per_frame = n_per_frame;
-    P.status = frame_status;
-    P.src = src;
-    P.g = g;
   }
   // (a later device-batch call first collects these chunks -- it blocks until they are done -- so
   // the host path needs no busy flag of its own; streaming host calls must not drain each other)
@@ -1353,6 +1559,231 @@ int ag_refined_saddle_points_batch(ag_detector* det, const void* frames, size_t 
                                    int* n_per_frame, uint32_t* frame_status) {
   return detect_batch_host(det, ResultKind::kSaddles, frames, frame_stride, n_frames, width, height, row_stride,
                            format, out, cap_per_frame, n_per_frame, frame_status, false);
+}
+
+// ag_detect_frames and ag_refined_saddle_points_frames: a list of host frames through the host-buffer
+// pipeline, chunk by chunk in the order of plan_frames; each chunk's frames are staged back to back in
+// its board slot (frame stride rounded up to 16 bytes, so that the streaming K1 still applies), so
+// the kernels see an ordinary batch.  Always synchronous.
+static int frames_host(ag_detector* det, ResultKind kind, const ag_frame* frames, int n_frames, void* out,
+                       int cap_per_frame, int* n_per_frame, uint32_t* frame_status) {
+  if (!det) return AG_ERR_INVALID;
+  if (!frames || !out || !n_per_frame || n_frames < 0 || cap_per_frame < 1)
+    return fail(det, AG_ERR_INVALID, "null pointer or bad count");
+  std::lock_guard<std::mutex> lk(det->mu);
+  std::vector<FrameGeom> geo;
+  const std::string bad = check_frames(frames, n_frames, false, &geo);
+  if (!bad.empty()) return fail(det, AG_ERR_INVALID, bad.c_str());
+  AG_CUDA(det, cudaSetDevice(det->device));
+  { int qrc = quiesce_device_path(det); if (qrc) return qrc; }
+  const uint64_t seq = ++det->host_seq;
+  if (n_frames == 0) return host_call_verdict(det);
+  set_caps(det, largest_frame(geo));
+  const FramePlan plan = plan_frames(geo, det->chunk_frames, det->host_chunk_frames, true);
+  const int n_chunks = (int)plan.chunk0.size() - 1;
+  auto staged = [&](int k) {  // geometry of chunk k as staged in a board slot
+    FrameGeom g = geo[plan.order[plan.chunk0[k]]];
+    g.frame_stride = (frame_bytes(g) + 15) & ~(size_t)15;
+    return g;
+  };
+  // everything is sized before the first chunk is enqueued: an allocation synchronises the device
+  int rc, max_frames = 0;
+  size_t max_bytes = 0;
+  for (int k = 0; k < n_chunks; ++k) {
+    const FrameGeom g = staged(k);
+    const int n = plan.chunk0[k + 1] - plan.chunk0[k];
+    max_frames = std::max(max_frames, n);
+    max_bytes = std::max(max_bytes, (size_t)n * g.frame_stride);
+    if ((rc = ensure_ring(det, g, n))) return rc;
+  }
+  if (!det->up_stream) AG_CUDA(det, cudaStreamCreateWithFlags(&det->up_stream, cudaStreamNonBlocking));
+  const cudaStream_t up = det->up_stream;
+  const bool saddles = kind == ResultKind::kSaddles;
+  std::vector<CopySeg> segs;
+  for (int k = 0; k < n_chunks; ++k) {
+    const FrameGeom g = staged(k);
+    const int* ids = plan.order.data() + plan.chunk0[k];
+    const int n = plan.chunk0[k + 1] - plan.chunk0[k];
+    const int bi = det->slot_rr;
+    BoardSlot& B = det->bslot[bi];
+    det->slot_rr = (det->slot_rr + 1) % kBoardSlots;
+    if ((rc = collect_host_slot(det, bi))) return rc;
+    if ((rc = ensure_board_slot(det, B, max_frames, true))) return rc;
+    const int sad_stride = saddles ? std::min(cap_per_frame, B.cap_saddles) : 0;
+    if ((rc = ensure_host_stage(det, B, max_bytes, max_frames, saddles ? 1 : cap_per_frame, sad_stride))) return rc;
+    // (no allocation: sized above) sets the dense sets' per-frame list stride, which K3 uses, for g
+    if ((rc = ensure_ring(det, g, n))) return rc;
+    // frames in pinned memory are uploaded directly; pageable ones through the slot's pinned staging
+    // (the slot's previous upload is done: its chunk has been collected)
+    segs.clear();
+    for (int i = 0; i < n; ++i)
+      if (is_pageable(frames[ids[i]].pixels)) {
+        if (max_bytes > B.cap_h_in) {
+          if (B.h_in) cudaFreeHost(B.h_in);
+          B.h_in = nullptr;
+          B.cap_h_in = 0;
+          AG_CUDA(det, cudaMallocHost((void**)&B.h_in, max_bytes));
+          B.cap_h_in = max_bytes;
+        }
+        segs.push_back({B.h_in + (size_t)i * g.frame_stride, (const uint8_t*)frames[ids[i]].pixels, frame_bytes(g)});
+      } else {
+        AG_CUDA(det, cudaMemcpyAsync(B.d_in + (size_t)i * g.frame_stride, frames[ids[i]].pixels, frame_bytes(g),
+                                     cudaMemcpyHostToDevice, up));
+      }
+    if (!segs.empty()) {
+      parallel_copy_segs(segs);
+      if ((int)segs.size() == n) {  // one upload of the whole staged chunk
+        AG_CUDA(det, cudaMemcpyAsync(B.d_in, B.h_in, (size_t)(n - 1) * g.frame_stride + frame_bytes(g),
+                                     cudaMemcpyHostToDevice, up));
+      } else {
+        for (const auto& c : segs)
+          AG_CUDA(det, cudaMemcpyAsync(B.d_in + (c.dst - B.h_in), c.dst, c.n, cudaMemcpyHostToDevice, up));
+      }
+    }
+    AG_CUDA(det, cudaEventRecord(B.ev_up, up));
+    if ((rc = enqueue_host_chunk(det, bi, kind, g, n, cap_per_frame, sad_stride, seq, out, n_per_frame, frame_status,
+                                 0, nullptr)))
+      return rc;
+    auto& P = det->hpend[bi];
+    P.idx.assign(ids, ids + n);
+    P.descs.resize(n);
+    for (int i = 0; i < n; ++i) P.descs[i] = frames[ids[i]];
+  }
+  if ((rc = collect_host(det, seq))) return rc;
+  return host_call_verdict(det);
+}
+
+int ag_detect_frames(ag_detector* det, const ag_frame* frames, int n_frames, ag_tag* out, int cap_per_frame,
+                     int* n_per_frame, uint32_t* frame_status) {
+  return frames_host(det, ResultKind::kTags, frames, n_frames, out, cap_per_frame, n_per_frame, frame_status);
+}
+
+int ag_refined_saddle_points_frames(ag_detector* det, const ag_frame* frames, int n_frames, ag_saddle* out,
+                                    int cap_per_frame, int* n_per_frame, uint32_t* frame_status) {
+  return frames_host(det, ResultKind::kSaddles, frames, n_frames, out, cap_per_frame, n_per_frame, frame_status);
+}
+
+// ag_detect_frames_device and ag_refined_saddle_points_frames_device: the device-batch pipeline over
+// the chunks of plan_frames.  K1 and K6 find each frame through the call's address table (see
+// FrameGeom::frame_ptrs); the results reach the caller's frames through the table's list indices
+// (k_saddles_out, or the board search into the slot's tag staging and k_tags_out).
+// The table of the whole call (frame addresses, then list indices, in plan order) is uploaded once into
+// a stream-ordered allocation from pageable host memory (the copy is staged before cudaMemcpyAsync
+// returns), and freed on the detector's table stream once every chunk of the call is done: the call
+// never waits for GPU progress, and a chunk's K1 waits for nothing but what a batch chunk waits for.
+static int frames_device(ag_detector* det, ResultKind kind, const ag_frame* frames, int n_frames, void* d_out,
+                         int cap_per_frame, int* d_n_per_frame, uint32_t* d_frame_status, void* stream) {
+  if (!det) return AG_ERR_INVALID;
+  if (!frames || !d_out || !d_n_per_frame || n_frames < 0 || cap_per_frame < 1)
+    return fail(det, AG_ERR_INVALID, "null pointer or bad count");
+  std::lock_guard<std::mutex> lk(det->mu);
+  std::vector<FrameGeom> geo;
+  const std::string bad = check_frames(frames, n_frames, true, &geo);
+  if (!bad.empty()) return fail(det, AG_ERR_INVALID, bad.c_str());
+  if (n_frames == 0) return AG_OK;
+  AG_CUDA(det, cudaSetDevice(det->device));
+  int rc;
+  if ((rc = collect_host(det, det->host_seq))) return rc;
+  set_caps(det, largest_frame(geo));
+  const FramePlan plan = plan_frames(geo, det->chunk_frames, det->host_chunk_frames, false);
+  const int n_chunks = (int)plan.chunk0.size() - 1;
+  const bool tags = kind == ResultKind::kTags;
+  // tags of a frame in the slot's staging: never more than the family has codes
+  const int tag_stride = tags ? std::min(cap_per_frame, det->fam.n_codes) : 0;
+  // the dense ring and every board slot are sized before the first chunk is enqueued (an allocation
+  // synchronises the device, and a slot's capacities are those of the call: see ensure_board_slot)
+  int max_frames = 0;
+  for (int k = 0; k < n_chunks; ++k) {
+    const int n = plan.chunk0[k + 1] - plan.chunk0[k];
+    max_frames = std::max(max_frames, n);
+    if ((rc = ensure_ring(det, geo[plan.order[plan.chunk0[k]]], n))) return rc;
+  }
+  for (auto& B : det->bslot)
+    if ((rc = ensure_board_slot(det, B, max_frames, false)) || (rc = ensure_list_stage(det, B, max_frames, tag_stride)))
+      return rc;
+  const cudaStream_t s = stream ? (cudaStream_t)stream : det->dense[0].stream;
+  if (!det->tab_stream) {
+    // a pool of the handle's own: memory a call frees is reused only once that free has happened, never
+    // by making a later call's stream wait for it (which would serialise calls under "device_async")
+    cudaMemPoolProps props = {};
+    props.allocType = cudaMemAllocationTypePinned;
+    props.location.type = cudaMemLocationTypeDevice;
+    props.location.id = det->device;
+    AG_CUDA(det, cudaMemPoolCreate(&det->tab_pool, &props));
+    int no = 0;
+    uint64_t keep = 16ull << 20;
+    AG_CUDA(det, cudaMemPoolSetAttribute(det->tab_pool, cudaMemPoolReuseAllowInternalDependencies, &no));
+    AG_CUDA(det, cudaMemPoolSetAttribute(det->tab_pool, cudaMemPoolAttrReleaseThreshold, &keep));
+    AG_CUDA(det, cudaStreamCreateWithFlags(&det->tab_stream, cudaStreamNonBlocking));
+    AG_CUDA(det, cudaEventCreateWithFlags(&det->ev_tab, cudaEventDisableTiming));
+  }
+  const size_t n_all = (size_t)n_frames;
+  std::vector<uint8_t> h_tab(n_all * (sizeof(void*) + sizeof(int)));
+  const uint8_t** h_ptrs = (const uint8_t**)h_tab.data();
+  int* h_idx = (int*)(h_tab.data() + sizeof(void*) * n_all);
+  for (size_t j = 0; j < n_all; ++j) {
+    h_ptrs[j] = (const uint8_t*)frames[plan.order[j]].pixels;
+    h_idx[j] = plan.order[j];
+  }
+  uint8_t* d_tab = nullptr;
+  AG_CUDA(det, cudaMallocFromPoolAsync((void**)&d_tab, h_tab.size(), det->tab_pool, s));
+  bool used[kBoardSlots] = {};
+  // the table is freed after every chunk that may read it, also when a chunk fails to enqueue
+  struct FreeTable {
+    ag_detector* det;
+    cudaStream_t s;
+    uint8_t* d_tab;
+    const bool* used;
+    ~FreeTable() {
+      cudaEventRecord(det->ev_tab, s);
+      cudaStreamWaitEvent(det->tab_stream, det->ev_tab, 0);
+      for (int b = 0; b < kBoardSlots; ++b)
+        if (used[b]) cudaStreamWaitEvent(det->tab_stream, det->bslot[b].ev_boards, 0);
+      cudaFreeAsync(d_tab, det->tab_stream);
+    }
+  } free_table{det, s, d_tab, used};
+  AG_CUDA(det, cudaMemcpyAsync(d_tab, h_tab.data(), h_tab.size(), cudaMemcpyHostToDevice, s));
+  for (int k = 0; k < n_chunks; ++k) {
+    const int j0 = plan.chunk0[k];
+    const int n = plan.chunk0[k + 1] - j0;
+    FrameGeom g = geo[plan.order[j0]];
+    const int bi = det->slot_rr;
+    BoardSlot& B = det->bslot[bi];
+    det->slot_rr = (det->slot_rr + 1) % kBoardSlots;
+    // (no allocation: sized above) sets the dense sets' per-frame list stride, which K3 uses, for g
+    if ((rc = ensure_ring(det, g, n))) return rc;
+    uintptr_t bits = 0;  // the streaming K1 needs every frame of the chunk aligned
+    for (int i = 0; i < n; ++i) bits |= (uintptr_t)h_ptrs[j0 + i];
+    g.frame_ptrs = (const uint8_t* const*)d_tab + j0;
+    g.ptr_bits = bits;
+    const ListOut list{(const int*)(d_tab + sizeof(void*) * n_all) + j0, d_out, cap_per_frame, d_n_per_frame,
+                       d_frame_status};
+    used[bi] = true;
+    if ((rc = run_front(det, B, nullptr, g, n, B.d_status, s)) ||
+        (rc = tags ? run_back(det, B, kind, nullptr, g, n, B.d_ltags, tag_stride, tag_stride, B.d_lntags, B.d_status,
+                              &list)
+                   : run_back(det, B, kind, nullptr, g, n, d_out, cap_per_frame, cap_per_frame, d_n_per_frame,
+                              B.d_status, &list)))
+      return rc;
+  }
+  det->device_path_busy = true;
+  if (!det->device_async)
+    for (auto& B : det->bslot)
+      if (B.pending) AG_CUDA(det, cudaStreamWaitEvent(s, B.ev_boards, 0));
+  return AG_OK;
+}
+
+int ag_detect_frames_device(ag_detector* det, const ag_frame* frames, int n_frames, ag_tag* d_out, int cap_per_frame,
+                            int* d_n_per_frame, uint32_t* d_frame_status, void* stream) {
+  return frames_device(det, ResultKind::kTags, frames, n_frames, d_out, cap_per_frame, d_n_per_frame, d_frame_status,
+                       stream);
+}
+
+int ag_refined_saddle_points_frames_device(ag_detector* det, const ag_frame* frames, int n_frames, ag_saddle* d_out,
+                                           int cap_per_frame, int* d_n_per_frame, uint32_t* d_frame_status,
+                                           void* stream) {
+  return frames_device(det, ResultKind::kSaddles, frames, n_frames, d_out, cap_per_frame, d_n_per_frame,
+                       d_frame_status, stream);
 }
 
 int ag_detect_batch_wait(ag_detector* det, int keep_in_flight) {
@@ -1732,6 +2163,31 @@ AG_API int ag_test_host_chunk(long long host_chunk_frames, int format, long long
   return AG_OK;
 }
 
+// Test hook (not in the public header; needs no GPU): the plan of a frame list -- order[n] (list
+// indices in the order they run), chunk0[*n_chunks + 1] (chunk k = order[chunk0[k] .. chunk0[k + 1])) --
+// for the options chunk_frames / host_chunk_frames and the host (host != 0) or device path, and the
+// index bounds[G + 1] of the multi-GPU split for G devices with host-to-device rates `rates` (NULL =
+// equal).  Descriptor addresses are not looked at.
+AG_API int ag_test_frame_plan(const ag_frame* frames, int n, long long chunk_frames, long long host_chunk_frames,
+                              int host, const double* rates, int G, int* order, int* chunk0, int* n_chunks,
+                              long long* bounds) {
+  if (!frames || n < 0 || chunk_frames < 1 || host_chunk_frames < 1 || G < 1 || !order || !chunk0 || !n_chunks ||
+      !bounds)
+    return AG_ERR_INVALID;
+  std::vector<FrameGeom> geo((size_t)n);
+  for (int i = 0; i < n; ++i)
+    if (geom_error(frames[i].width, frames[i].height, frames[i].row_stride, 0, frames[i].format, &geo[i]))
+      return AG_ERR_INVALID;
+  const FramePlan p = plan_frames(geo, (long)chunk_frames, (long)host_chunk_frames, host != 0);
+  std::copy(p.order.begin(), p.order.end(), order);
+  std::copy(p.chunk0.begin(), p.chunk0.end(), chunk0);
+  *n_chunks = (int)p.chunk0.size() - 1;
+  const std::vector<double> r = rates ? std::vector<double>(rates, rates + G) : std::vector<double>();
+  const std::vector<long long> b = list_shard_bounds(geo, shard_shares(r, G));
+  std::copy(b.begin(), b.end(), bounds);
+  return AG_OK;
+}
+
 // Test hook (not in the public header): ONE frame of the renderer under a GIVEN pose -- hinv maps
 // image (x, y, 1) to page coordinates in tag sides (row-major 3x3, host pointer) -- with or without
 // the noise, so that tests can pin the renderer's geometry (id <-> lattice position, corner
@@ -1997,6 +2453,27 @@ int ag_multi_set_option(ag_multi* m, const char* key, long value) {
   return AG_OK;
 }
 
+// One host thread per device g running work(g) on its shard [bound[g], bound[g + 1]); the worst code.
+static int run_shards(ag_multi* m, const std::vector<long long>& bound,
+                      const std::function<int(int, long long, long long)>& work) {
+  const int G = (int)m->dets.size();
+  std::vector<int> rcs(G, AG_OK);
+  auto one = [&](int g) {
+    if (bound[g + 1] > bound[g]) rcs[g] = work(g, bound[g], bound[g + 1]);
+  };
+  std::vector<std::thread> th;
+  for (int g = 1; g < G; ++g) th.emplace_back(one, g);
+  one(0);
+  for (auto& t : th) t.join();
+  int worst = AG_OK;
+  for (int g = 0; g < G; ++g)
+    if (rcs[g] != AG_OK && (worst == AG_OK || rcs[g] != AG_ERR_CAPACITY)) {  // a hard error outranks a capacity notice
+      worst = rcs[g];
+      m->err = std::string("device ") + std::to_string(m->dets[g]->device) + ": " + ag_last_error(m->dets[g]);
+    }
+  return worst;
+}
+
 // The host-buffer batch call of one kind over every device of m: the shard boundaries, one host
 // thread per device, the worst code.  Each shard runs synchronously, whatever a device's
 // "host_async" says (ag_multi has no wait entry point), as ag_detect.
@@ -2013,39 +2490,44 @@ static int multi_batch_host(ag_multi* m, ResultKind kind, const void* frames, si
   const size_t fs = frame_stride ? frame_stride : rs * (size_t)(height > 0 ? height : 0);
   const size_t rec = kind == ResultKind::kTags ? sizeof(ag_tag) : sizeof(ag_saddle);
   const int G = (int)m->dets.size();
-  std::vector<int> rcs(G, AG_OK);
-  // shard boundaries: equal ranges, or -- when the devices' measured host-to-device rates differ by
-  // more than 5 % -- ranges in proportion to those rates
+  // shard boundaries: frame counts in proportion to the devices' shares
+  const std::vector<double> share = shard_shares(m->h2d_gbs, G);
   std::vector<long long> bound(G + 1, 0);
-  {
-    double lo_r = 1e300, hi_r = 0.0, sum = 0.0;
-    for (double r : m->h2d_gbs) { lo_r = std::min(lo_r, r); hi_r = std::max(hi_r, r); sum += r; }
-    const bool weighted = (int)m->h2d_gbs.size() == G && lo_r > 0.0 && hi_r > 1.05 * lo_r;
-    double acc = 0.0;
-    for (int g = 0; g < G; ++g) {
-      acc += weighted ? m->h2d_gbs[g] / sum : 1.0 / G;
-      bound[g + 1] = g + 1 == G ? n_frames : std::min<long long>(n_frames, (long long)llround(acc * n_frames));
-      if (bound[g + 1] < bound[g]) bound[g + 1] = bound[g];
-    }
+  double acc = 0.0;
+  for (int g = 0; g < G; ++g) {
+    acc += share[g];
+    bound[g + 1] = g + 1 == G ? n_frames : std::min<long long>(n_frames, (long long)llround(acc * n_frames));
+    if (bound[g + 1] < bound[g]) bound[g + 1] = bound[g];
   }
-  auto work = [&](int g) {
-    const long long lo = bound[g], hi = bound[g + 1];
-    if (hi <= lo) return;
-    rcs[g] = detect_batch_host(m->dets[g], kind, (const uint8_t*)frames + (size_t)lo * fs, fs, (int)(hi - lo), width,
-                               height, rs, format, (uint8_t*)out + (size_t)lo * cap_per_frame * rec, cap_per_frame,
-                               n_per_frame + lo, frame_status ? frame_status + lo : nullptr, /*async_call=*/false);
-  };
-  std::vector<std::thread> th;
-  for (int g = 1; g < G; ++g) th.emplace_back(work, g);
-  work(0);
-  for (auto& t : th) t.join();
-  int worst = AG_OK;
-  for (int g = 0; g < G; ++g)
-    if (rcs[g] != AG_OK && (worst == AG_OK || rcs[g] != AG_ERR_CAPACITY)) {  // a hard error outranks a capacity notice
-      worst = rcs[g];
-      m->err = std::string("device ") + std::to_string(m->dets[g]->device) + ": " + ag_last_error(m->dets[g]);
-    }
-  return worst;
+  return run_shards(m, bound, [&](int g, long long lo, long long hi) {
+    return detect_batch_host(m->dets[g], kind, (const uint8_t*)frames + (size_t)lo * fs, fs, (int)(hi - lo), width,
+                             height, rs, format, (uint8_t*)out + (size_t)lo * cap_per_frame * rec, cap_per_frame,
+                             n_per_frame + lo, frame_status ? frame_status + lo : nullptr, /*async_call=*/false);
+  });
+}
+
+// A frame list over every device of m: contiguous index ranges of about equal frame bytes (weighted
+// as above), each through frames_host on its device.  Every descriptor is checked first, so that a bad
+// one stops the call before any device runs.
+static int multi_frames_host(ag_multi* m, ResultKind kind, const ag_frame* frames, int n_frames, void* out,
+                             int cap_per_frame, int* n_per_frame, uint32_t* frame_status) {
+  if (!m || m->dets.empty()) return AG_ERR_INVALID;
+  if (!frames || !out || !n_per_frame || n_frames < 0 || cap_per_frame < 1) {
+    m->err = "null pointer or bad count";
+    return AG_ERR_INVALID;
+  }
+  std::vector<FrameGeom> geo;
+  const std::string bad = check_frames(frames, n_frames, false, &geo);
+  if (!bad.empty()) {
+    m->err = bad;
+    return AG_ERR_INVALID;
+  }
+  const size_t rec = kind == ResultKind::kTags ? sizeof(ag_tag) : sizeof(ag_saddle);
+  const std::vector<long long> bound = list_shard_bounds(geo, shard_shares(m->h2d_gbs, (int)m->dets.size()));
+  return run_shards(m, bound, [&](int g, long long lo, long long hi) {
+    return frames_host(m->dets[g], kind, frames + lo, (int)(hi - lo), (uint8_t*)out + (size_t)lo * cap_per_frame * rec,
+                       cap_per_frame, n_per_frame + lo, frame_status ? frame_status + lo : nullptr);
+  });
 }
 
 int ag_multi_detect_batch(ag_multi* m, const void* frames, size_t frame_stride, int n_frames, int width,
@@ -2060,6 +2542,16 @@ int ag_multi_refined_saddle_points_batch(ag_multi* m, const void* frames, size_t
                                          int cap_per_frame, int* n_per_frame, uint32_t* frame_status) {
   return multi_batch_host(m, ResultKind::kSaddles, frames, frame_stride, n_frames, width, height, row_stride, format,
                           out, cap_per_frame, n_per_frame, frame_status);
+}
+
+int ag_multi_detect_frames(ag_multi* m, const ag_frame* frames, int n_frames, ag_tag* out, int cap_per_frame,
+                           int* n_per_frame, uint32_t* frame_status) {
+  return multi_frames_host(m, ResultKind::kTags, frames, n_frames, out, cap_per_frame, n_per_frame, frame_status);
+}
+
+int ag_multi_refined_saddle_points_frames(ag_multi* m, const ag_frame* frames, int n_frames, ag_saddle* out,
+                                          int cap_per_frame, int* n_per_frame, uint32_t* frame_status) {
+  return multi_frames_host(m, ResultKind::kSaddles, frames, n_frames, out, cap_per_frame, n_per_frame, frame_status);
 }
 
 }  // extern "C"

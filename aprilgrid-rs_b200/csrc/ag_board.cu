@@ -235,7 +235,7 @@ k_boards_decode(const uint8_t* __restrict__ frames, FrameGeom g, int n_frames,
   F.samp = F.diff + 64;
   F.remove = W + L.off_remove;
   F.max_quads = L.max_quads;
-  F.img = frames + (size_t)f * g.frame_stride;
+  F.img = frame_base(frames, g, f);
   F.w = g.w;
   F.h = g.h;
   F.format = g.format;

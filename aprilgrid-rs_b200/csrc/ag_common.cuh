@@ -50,7 +50,17 @@ struct FrameGeom {
   size_t frame_stride;  // bytes between input frames
   size_t row_stride;    // bytes between input rows
   int format;           // a public AG_* pixel format, or kFmtF32
+  // frame lists (ag_detect_frames_device): device table of the chunk's frame addresses, used in place
+  // of frames + f * frame_stride when set; ptr_bits = the OR of those addresses, for the launchers'
+  // alignment checks (the table itself is not readable on the host)
+  const uint8_t* const* frame_ptrs = nullptr;
+  uintptr_t ptr_bits = 0;
 };
+
+// First byte of frame f of a chunk.
+AG_HD const uint8_t* frame_base(const uint8_t* frames, const FrameGeom& g, int f) {
+  return g.frame_ptrs ? g.frame_ptrs[f] : frames + (size_t)f * g.frame_stride;
+}
 
 // Monotone float <-> uint key so that atomicMin on the key is a float min.
 AG_HD uint32_t float_to_ordered(float f) {

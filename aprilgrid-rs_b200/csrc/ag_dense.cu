@@ -98,7 +98,7 @@ k_blur_hessian_tile(const uint8_t* __restrict__ frames, FrameGeom g, float* __re
   const int tid = threadIdx.x;
   const int x0 = blockIdx.x * T_W, y0 = blockIdx.y * T_H;
   const int f = blockIdx.z;
-  const uint8_t* frame = frames + (size_t)f * g.frame_stride;
+  const uint8_t* frame = frame_base(frames, g, f);
 
   // 1. gray conversion of the clamped (edge-replicated) input window
   for (int i = tid; i < IN_H * IN_W; i += 256) {
@@ -321,7 +321,7 @@ k_blur_hessian_stream(const uint8_t* __restrict__ frames, FrameGeom g, int chunk
   // checks that a frame's bytes fit them)
   // The lane's pointers into the frame are held in registers (opaque, or the compiler re-derives
   // them from blockIdx in every row step); a row then costs one 32x32->64 multiply-add per access.
-  const uint8_t* src = frames + (size_t)f * g.frame_stride + (size_t)cw * kBpp;
+  const uint8_t* src = frame_base(frames, g, f) + (size_t)cw * kBpp;
   asm volatile("" : "+l"(src));
   const uint32_t rs = (uint32_t)g.row_stride;
   const bool left_out = c0 < 0, right_out = c0 >= g.w;
@@ -724,7 +724,7 @@ int launch_blur_hessian(const uint8_t* frames, const FrameGeom& g, int n_frames,
   const int bpp = bytes_per_px(g.format);
   const size_t al = bpp == 1 || bpp == 3 ? 4 : (bpp == 2 || bpp == 6 ? 8 : 16);
   const bool can_stream = (g.w % 4) == 0 && g.w >= 8 && (g.row_stride % al) == 0 && (g.frame_stride % al) == 0 &&
-                          ((uintptr_t)frames % al) == 0 && variant != 1 &&
+                          (((uintptr_t)frames | g.ptr_bits) % al) == 0 && variant != 1 &&
                           (uint64_t)g.row_stride * (uint64_t)g.h < (1ull << 32);  // 32-bit offsets within a frame
   if (can_stream) {
     const int strips = (g.w + S_COLS - 1) / S_COLS;

@@ -57,8 +57,15 @@ int launch_refine_filter(const float* blur, const FrameGeom& g, int n_frames, co
                          int* n_refined, uint32_t* frame_status, cudaStream_t s);
 // the saddle entry points' result: K4's lists (in_stride per frame) -> out (out_stride per frame),
 // n_out = exact count (0 if the frame's list was truncated), AG_FRAME_TAG_OVERFLOW when n > cap
+// idx (frame lists, may be null): frame f's results go to the caller's frame idx[f], and its final status
+// bits to status_out[idx[f]] when status_out is set
 int launch_saddles_out(const ag_saddle* refined, int in_stride, const int* n_refined, uint32_t* frame_status,
-                       int n_frames, ag_saddle* out, int out_stride, int cap, int* n_out, cudaStream_t s);
+                       int n_frames, ag_saddle* out, int out_stride, int cap, int* n_out, cudaStream_t s,
+                       const int* idx = nullptr, uint32_t* status_out = nullptr);
+// frame lists: the chunk-local tags, counts and status bits of the board search (in_stride records per
+// frame) -> the caller's frame idx[f] (cap records per frame; status_out may be null)
+int launch_tags_out(const ag_tag* tags, int in_stride, const int* n_tags, const uint32_t* frame_status, int n_frames,
+                    const int* idx, ag_tag* out, int cap, int* n_out, uint32_t* status_out, cudaStream_t s);
 
 // ag_board.cu
 extern int g_board_smem_pad;

@@ -723,6 +723,8 @@ k_refine_filter(const float* __restrict__ blur, FrameGeom g, const float2* __res
 // min(n, cap) records are copied as 32-bit words, so consecutive lanes touch consecutive words
 // whatever the 20-byte record boundaries; n > cap sets AG_FRAME_TAG_OVERFLOW.  The callers give
 // out_stride >= min(n, cap): an unflagged frame has at most in_stride saddles.
+// Frame lists: frame f of the chunk is the caller's frame idx[f] (out, n_out and status_out are
+// indexed by it; status_out, if set, receives the frame's final status bits).
 constexpr int kSaddlesOutThreads = 256;
 constexpr int kSaddleWords = (int)(sizeof(ag_saddle) / sizeof(uint32_t));
 static_assert(sizeof(ag_saddle) == 5 * sizeof(uint32_t), "ag_saddle is five 32-bit words");
@@ -730,25 +732,62 @@ static_assert(sizeof(ag_saddle) == 5 * sizeof(uint32_t), "ag_saddle is five 32-b
 __global__ void __launch_bounds__(kSaddlesOutThreads)
 k_saddles_out(const ag_saddle* __restrict__ refined, int in_stride, const int* __restrict__ n_refined,
               uint32_t* __restrict__ frame_status, ag_saddle* __restrict__ out, int out_stride, int cap,
-              int* __restrict__ n_out) {
+              int* __restrict__ n_out, const int* __restrict__ idx, uint32_t* __restrict__ status_out) {
   const int f = blockIdx.x;
+  const int o = idx ? idx[f] : f;
   const uint32_t st = frame_status[f];
   const int n = (st & (AG_FRAME_CLUSTER_OVERFLOW | AG_FRAME_SADDLE_OVERFLOW)) ? 0 : n_refined[f];
   const int words = min(n, cap) * kSaddleWords;
   const uint32_t* src = reinterpret_cast<const uint32_t*>(refined + (size_t)f * in_stride);
-  uint32_t* dst = reinterpret_cast<uint32_t*>(out + (size_t)f * out_stride);
+  uint32_t* dst = reinterpret_cast<uint32_t*>(out + (size_t)o * out_stride);
   for (int i = threadIdx.x; i < words; i += kSaddlesOutThreads) dst[i] = src[i];
   if (threadIdx.x == 0) {
-    n_out[f] = n;
-    if (n > cap) frame_status[f] = st | AG_FRAME_TAG_OVERFLOW;
+    n_out[o] = n;
+    const uint32_t st_out = n > cap ? st | AG_FRAME_TAG_OVERFLOW : st;
+    if (n > cap) frame_status[f] = st_out;
+    if (status_out) status_out[o] = st_out;
   }
 }
 
 int launch_saddles_out(const ag_saddle* refined, int in_stride, const int* n_refined, uint32_t* frame_status,
-                       int n_frames, ag_saddle* out, int out_stride, int cap, int* n_out, cudaStream_t s) {
+                       int n_frames, ag_saddle* out, int out_stride, int cap, int* n_out, cudaStream_t s,
+                       const int* idx, uint32_t* status_out) {
   if (n_frames <= 0) return 0;
   k_saddles_out<<<n_frames, kSaddlesOutThreads, 0, s>>>(refined, in_stride, n_refined, frame_status, out, out_stride,
-                                                         cap, n_out);
+                                                         cap, n_out, idx, status_out);
+  return 1;
+}
+
+// The tag twin of k_saddles_out for frame lists: the board search of a chunk writes its tags, counts
+// and status bits chunk-locally (`in_stride` records per frame); this copies the count, the status
+// bits and the first min(n, cap) records of frame f to the caller's frame idx[f].  One block per frame,
+// records copied as 32-bit words.
+constexpr int kTagsOutThreads = 128;
+constexpr int kTagWords = (int)(sizeof(ag_tag) / sizeof(uint32_t));
+static_assert(sizeof(ag_tag) == 9 * sizeof(uint32_t), "ag_tag is nine 32-bit words");
+
+__global__ void __launch_bounds__(kTagsOutThreads)
+k_tags_out(const ag_tag* __restrict__ tags, int in_stride, const int* __restrict__ n_tags,
+           const uint32_t* __restrict__ frame_status, const int* __restrict__ idx, ag_tag* __restrict__ out, int cap,
+           int* __restrict__ n_out, uint32_t* __restrict__ status_out) {
+  const int f = blockIdx.x;
+  const int o = idx[f];
+  const int n = n_tags[f];
+  const int words = min(min(n, cap), in_stride) * kTagWords;
+  const uint32_t* src = reinterpret_cast<const uint32_t*>(tags + (size_t)f * in_stride);
+  uint32_t* dst = reinterpret_cast<uint32_t*>(out + (size_t)o * cap);
+  for (int i = threadIdx.x; i < words; i += kTagsOutThreads) dst[i] = src[i];
+  if (threadIdx.x == 0) {
+    n_out[o] = n;
+    if (status_out) status_out[o] = frame_status[f];
+  }
+}
+
+int launch_tags_out(const ag_tag* tags, int in_stride, const int* n_tags, const uint32_t* frame_status, int n_frames,
+                    const int* idx, ag_tag* out, int cap, int* n_out, uint32_t* status_out, cudaStream_t s) {
+  if (n_frames <= 0) return 0;
+  k_tags_out<<<n_frames, kTagsOutThreads, 0, s>>>(tags, in_stride, n_tags, frame_status, idx, out, cap, n_out,
+                                                   status_out);
   return 1;
 }
 

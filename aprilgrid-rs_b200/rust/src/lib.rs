@@ -6,7 +6,9 @@
 //!   * `detect_kornia<const N: usize>(&self, &kornia::image::Image<u8, N>)`         (:479)
 //!   * `refined_saddle_points(&self, &DynamicImage) -> Vec<Saddle>`                 (:408)
 //! plus the added `detect_batch(&self, &[DynamicImage]) -> Vec<HashMap<..>>` (one GPU) and
-//! `MultiTagDetector::detect_batch` (every GPU of the box, frames sharded image-wise).
+//! `MultiTagDetector::detect_batch` (every GPU of the box, frames sharded image-wise).  A slice of
+//! images of mixed sizes or pixel formats goes through the frame-list entry points
+//! (`ag_detect_frames`, ...), each image from its own buffer.
 //!
 //! NOT a full drop-in: the lower-level public functions the reference's `examples/develop.rs`
 //! uses (`decode_positions`, `bit_code`, `best_tag`, `rochade_refine`, `init_quads`,
@@ -91,6 +93,17 @@ struct AgTag {
     xy: [f32; 8],
 }
 
+/// `ag_frame` of include/aprilgrid_b200.h: one image of a frame list.
+#[repr(C)]
+#[derive(Clone, Copy)]
+struct AgFrame {
+    pixels: *const c_void,
+    width: c_int,
+    height: c_int,
+    row_stride: usize,
+    format: c_int,
+}
+
 mod ffi {
     use super::*;
     #[repr(C)]
@@ -122,6 +135,16 @@ mod ffi {
                                               n_frames: c_int, width: c_int, height: c_int, row_stride: usize,
                                               format: c_int, out: *mut AgSaddle, cap_per_frame: c_int,
                                               n_per_frame: *mut c_int, frame_status: *mut u32) -> c_int;
+        pub fn ag_detect_frames(det: *mut AgDetector, frames: *const AgFrame, n_frames: c_int, out: *mut AgTag,
+                                cap_per_frame: c_int, n_per_frame: *mut c_int, frame_status: *mut u32) -> c_int;
+        pub fn ag_refined_saddle_points_frames(det: *mut AgDetector, frames: *const AgFrame, n_frames: c_int,
+                                               out: *mut AgSaddle, cap_per_frame: c_int, n_per_frame: *mut c_int,
+                                               frame_status: *mut u32) -> c_int;
+        pub fn ag_multi_detect_frames(m: *mut AgMulti, frames: *const AgFrame, n_frames: c_int, out: *mut AgTag,
+                                      cap_per_frame: c_int, n_per_frame: *mut c_int, frame_status: *mut u32) -> c_int;
+        pub fn ag_multi_refined_saddle_points_frames(m: *mut AgMulti, frames: *const AgFrame, n_frames: c_int,
+                                                     out: *mut AgSaddle, cap_per_frame: c_int,
+                                                     n_per_frame: *mut c_int, frame_status: *mut u32) -> c_int;
         pub fn ag_host_alloc(bytes: usize) -> *mut c_void;
         pub fn ag_host_free(p: *mut c_void);
         pub fn ag_multi_create(family: c_int, params: *const DetectorParams, devices: *const c_int, n_devices: c_int,
@@ -248,6 +271,26 @@ fn maps_of(out: &[AgTag], counts: &[c_int], cap: usize) -> Vec<HashMap<u32, [(f3
         .collect()
 }
 
+/// Whether every image of a slice has the size and pixel format of the first.
+fn uniform(imgs: &[DynamicImage]) -> bool {
+    let (_, fmt, _, w, h) = pixels_of(&imgs[0]);
+    imgs.iter().all(|im| {
+        let (_, f, _, ww, hh) = pixels_of(im);
+        ww == w && hh == h && f == fmt
+    })
+}
+
+/// Frame-list descriptors of a slice: each image read from its own buffer (valid while `imgs` is borrowed).
+fn frames_of(imgs: &[DynamicImage]) -> Vec<AgFrame> {
+    imgs.iter()
+        .map(|im| {
+            let (bytes, fmt, stride, w, h) = pixels_of(im);
+            AgFrame { pixels: bytes.as_ptr() as *const c_void, width: w as c_int, height: h as c_int, row_stride: stride,
+                      format: fmt }
+        })
+        .collect()
+}
+
 /// Pack equally sized images of one pixel format into one pinned buffer.
 fn pack(imgs: &[DynamicImage]) -> (Pinned, u32, u32, c_int, usize) {
     let (_, fmt, stride, w, h) = pixels_of(&imgs[0]);
@@ -337,10 +380,28 @@ impl TagDetector {
         out[..n as usize].iter().map(|t| (t.id, corners(t))).collect()
     }
 
-    /// New: one call for a batch of equally sized images of one pixel format.
+    /// New: one call for a batch of images.  Equally sized images of one pixel format are packed into
+    /// one pinned buffer; a slice of mixed sizes or formats goes through `ag_detect_frames` unpacked.
     pub fn detect_batch(&self, imgs: &[DynamicImage]) -> Vec<HashMap<u32, [(f32, f32); 4]>> {
         if imgs.is_empty() {
             return Vec::new();
+        }
+        if !uniform(imgs) {
+            let frames = frames_of(imgs);
+            let mut out = vec![AgTag { id: 0, xy: [0.0; 8] }; TAG_CAP * imgs.len()];
+            let mut counts = vec![0 as c_int; imgs.len()];
+            let det = self.checkout();
+            let rc = unsafe {
+                ffi::ag_detect_frames(det, frames.as_ptr(), imgs.len() as c_int, out.as_mut_ptr(), TAG_CAP as c_int,
+                                      counts.as_mut_ptr(), std::ptr::null_mut())
+            };
+            if rc != 0 {
+                let msg = last_error(det);
+                self.checkin(det);
+                panic!("aprilgrid_b200: ag_detect_frames failed ({rc}): {msg}");
+            }
+            self.checkin(det);
+            return maps_of(&out, &counts, TAG_CAP);
         }
         let (packed, w, h, fmt, stride) = pack(imgs);
         let mut out = vec![AgTag { id: 0, xy: [0.0; 8] }; TAG_CAP * imgs.len()];
@@ -388,10 +449,27 @@ impl TagDetector {
         out[..n as usize].iter().map(|s| Saddle { p: (s.x, s.y), k: s.k, theta: s.theta, phi: s.phi }).collect()
     }
 
-    /// New: `refined_saddle_points` of every image of a batch of equally sized images of one pixel format.
+    /// New: `refined_saddle_points` of every image of a batch (mixed sizes and formats as in `detect_batch`).
     pub fn refined_saddle_points_batch(&self, imgs: &[DynamicImage]) -> Vec<Vec<Saddle>> {
         if imgs.is_empty() {
             return Vec::new();
+        }
+        if !uniform(imgs) {
+            let frames = frames_of(imgs);
+            let mut out = vec![AgSaddle::default(); SADDLE_CAP * imgs.len()];
+            let mut counts = vec![0 as c_int; imgs.len()];
+            let det = self.checkout();
+            let rc = unsafe {
+                ffi::ag_refined_saddle_points_frames(det, frames.as_ptr(), imgs.len() as c_int, out.as_mut_ptr(),
+                                                     SADDLE_CAP as c_int, counts.as_mut_ptr(), std::ptr::null_mut())
+            };
+            if rc != 0 {
+                let msg = last_error(det);
+                self.checkin(det);
+                panic!("aprilgrid_b200: ag_refined_saddle_points_frames failed ({rc}): {msg}");
+            }
+            self.checkin(det);
+            return saddle_lists_of(&out, &counts, SADDLE_CAP);
         }
         let (packed, w, h, fmt, stride) = pack(imgs);
         let mut out = vec![AgSaddle::default(); SADDLE_CAP * imgs.len()];
@@ -509,6 +587,20 @@ impl MultiTagDetector {
         if imgs.is_empty() {
             return Vec::new();
         }
+        if !uniform(imgs) {
+            let frames = frames_of(imgs);
+            let mut out = vec![AgTag { id: 0, xy: [0.0; 8] }; TAG_CAP * imgs.len()];
+            let mut counts = vec![0 as c_int; imgs.len()];
+            let rc = unsafe {
+                ffi::ag_multi_detect_frames(self.m, frames.as_ptr(), imgs.len() as c_int, out.as_mut_ptr(),
+                                            TAG_CAP as c_int, counts.as_mut_ptr(), std::ptr::null_mut())
+            };
+            if rc != 0 {
+                let msg = unsafe { std::ffi::CStr::from_ptr(ffi::ag_multi_last_error(self.m)).to_string_lossy().into_owned() };
+                panic!("aprilgrid_b200: ag_multi_detect_frames failed ({rc}): {msg}");
+            }
+            return maps_of(&out, &counts, TAG_CAP);
+        }
         let (packed, w, h, fmt, stride) = pack(imgs);
         let mut out = vec![AgTag { id: 0, xy: [0.0; 8] }; TAG_CAP * imgs.len()];
         let mut counts = vec![0 as c_int; imgs.len()];
@@ -527,6 +619,21 @@ impl MultiTagDetector {
     pub fn refined_saddle_points_batch(&mut self, imgs: &[DynamicImage]) -> Vec<Vec<Saddle>> {
         if imgs.is_empty() {
             return Vec::new();
+        }
+        if !uniform(imgs) {
+            let frames = frames_of(imgs);
+            let mut out = vec![AgSaddle::default(); SADDLE_CAP * imgs.len()];
+            let mut counts = vec![0 as c_int; imgs.len()];
+            let rc = unsafe {
+                ffi::ag_multi_refined_saddle_points_frames(self.m, frames.as_ptr(), imgs.len() as c_int,
+                                                           out.as_mut_ptr(), SADDLE_CAP as c_int, counts.as_mut_ptr(),
+                                                           std::ptr::null_mut())
+            };
+            if rc != 0 {
+                let msg = unsafe { std::ffi::CStr::from_ptr(ffi::ag_multi_last_error(self.m)).to_string_lossy().into_owned() };
+                panic!("aprilgrid_b200: ag_multi_refined_saddle_points_frames failed ({rc}): {msg}");
+            }
+            return saddle_lists_of(&out, &counts, SADDLE_CAP);
         }
         let (packed, w, h, fmt, stride) = pack(imgs);
         let mut out = vec![AgSaddle::default(); SADDLE_CAP * imgs.len()];

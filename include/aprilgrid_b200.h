@@ -238,6 +238,56 @@ AG_API int ag_refined_saddle_points_batch_device(ag_detector* det, const void* d
                                                  int* d_n_per_frame, uint32_t* d_frame_status,
                                                  void* stream);
 
+/* ---- lists of frames of mixed sizes and pixel formats ---------------------------------------
+ * One frame of a list: the fields and their order are those of the C++ mirror's ImageView. */
+typedef struct ag_frame {
+  const void* pixels; /* host or device address, as the entry point says */
+  int width, height;
+  size_t row_stride; /* bytes, 0 = packed */
+  int format;        /* AG_L8 .. AG_RGBA32F */
+} ag_frame;
+
+/* detect / refined_saddle_points on a list of n_frames frames, each with its own address, size,
+ * row stride and pixel format.  Outputs are laid out as on the _batch siblings and indexed by list
+ * position: out[i*cap_per_frame ..], n_per_frame[i], frame_status[i] (may be NULL).
+ * Contract of the six list entry points (these two, the _device pair and the ag_multi_ pair):
+ *  - Frame i's result is byte-identical to what ag_detect / ag_refined_saddle_points returns for
+ *    that frame alone; the grouping and order of the list never change a result.
+ *  - Every descriptor is checked before anything runs: null pixels, width or height <= 0, an
+ *    unknown format, a row stride shorter than a row or not a multiple of the channel word, and (on
+ *    the device calls) a device address that is not a multiple of the channel word.  One bad
+ *    descriptor, a null list, n_frames < 0 or cap_per_frame < 1: AG_ERR_INVALID, nothing runs and no
+ *    output is touched.  n_frames == 0: AG_OK.  Frames may alias each other.
+ *  - Capacities as on the _batch siblings: the host calls re-run a frame that overflowed
+ *    max_clusters / max_saddles alone with grown capacities; a frame beyond the hard limits keeps
+ *    its bits and the call returns AG_ERR_CAPACITY; the device calls report n = 0 and the bits.
+ *    n_per_frame[i] > cap_per_frame: the count stays exact, the first cap_per_frame records are
+ *    written, AG_FRAME_TAG_OVERFLOW is set (and the host calls return AG_ERR_CAPACITY).  The
+ *    per-frame capacities of a list call are those the largest frame of the list would get alone, so
+ *    the device call flags no frame that ag_detect_batch_device on that frame's shape would not.
+ *  - Frames are grouped by (width, height, format, row_stride) in order of first appearance; each
+ *    group runs in chunks of one geometry through the same pipeline as a batch, so the groups
+ *    overlap in it.  A group of one frame still costs one chunk's launches.
+ *  - List calls and the other calls may be interleaved on one handle, on any streams, without
+ *    changing each other's results.  A host list call first collects the chunks of "host_async"
+ *    calls still in flight; it is always synchronous. */
+AG_API int ag_detect_frames(ag_detector* det, const ag_frame* frames, int n_frames, ag_tag* out,
+                            int cap_per_frame, int* n_per_frame, uint32_t* frame_status);
+AG_API int ag_refined_saddle_points_frames(ag_detector* det, const ag_frame* frames, int n_frames,
+                                           ag_saddle* out, int cap_per_frame, int* n_per_frame,
+                                           uint32_t* frame_status);
+/* Same, with `pixels` of every descriptor a DEVICE address (the descriptor array itself is on the
+ * host) and DEVICE outputs (d_out: n_frames*cap_per_frame records, d_n_per_frame: n_frames int32,
+ * d_frame_status: n_frames uint32 or NULL).  Enqueued on `stream` as ag_detect_batch_device; option
+ * "device_async" and ag_detect_batch_device_wait apply to them exactly as to that call.  The frames
+ * must stay valid until the results are ordered on the stream. */
+AG_API int ag_detect_frames_device(ag_detector* det, const ag_frame* frames, int n_frames, ag_tag* d_out,
+                                   int cap_per_frame, int* d_n_per_frame, uint32_t* d_frame_status,
+                                   void* stream);
+AG_API int ag_refined_saddle_points_frames_device(ag_detector* det, const ag_frame* frames, int n_frames,
+                                                  ag_saddle* d_out, int cap_per_frame, int* d_n_per_frame,
+                                                  uint32_t* d_frame_status, void* stream);
+
 /* image_util::gaussian_blur_f32(img, sigma) and image_util::hessian_response(img):
  * f32 -> f32, host buffers, width*height floats each.                                   */
 AG_API int ag_gaussian_blur_f32(ag_detector* det, const float* img, int width, int height,
@@ -328,6 +378,14 @@ AG_API int ag_multi_refined_saddle_points_batch(ag_multi* m, const void* frames,
                                                 size_t row_stride, int format, ag_saddle* out,
                                                 int cap_per_frame, int* n_per_frame,
                                                 uint32_t* frame_status);
+/* ag_detect_frames / ag_refined_saddle_points_frames over every device of m: the list is cut into
+ * contiguous index ranges of about equal frame bytes (weighted by the devices' host-to-device rates
+ * as above); byte-identical to one device processing the list. */
+AG_API int ag_multi_detect_frames(ag_multi* m, const ag_frame* frames, int n_frames, ag_tag* out,
+                                  int cap_per_frame, int* n_per_frame, uint32_t* frame_status);
+AG_API int ag_multi_refined_saddle_points_frames(ag_multi* m, const ag_frame* frames, int n_frames,
+                                                 ag_saddle* out, int cap_per_frame, int* n_per_frame,
+                                                 uint32_t* frame_status);
 
 AG_API const char* ag_version(void);
 
